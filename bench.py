@@ -3,7 +3,7 @@
 and % of the HBM roofline, on 1..8 B200 (BASELINE.json `metric`).
 
     python bench.py --gpus N --steps K --warmup W [--workload cfg4] [--scaling weak|strong]
-                    [--launch graph|stream] [--gather fused|nccl] [--impl reference]
+                    [--launch graph|stream] [--gather fused|nccl] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic coefficient
 vectors: a single launch of the fused evaluator (funobj mode 2 + funcon mode 2
@@ -423,6 +423,28 @@ def time_small(torch, pb, ring, steps, warmup):
     return {"ms_per_step": ms, "kernel_ms": ms, "launches": laps * nset}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(torch, out, ncnln, path):
+    """What a caller of the timed path receives from one step -- f [P], g [P][nC], c [P][ncnln],
+    J [P][ncnln*S] in the device band layout, result [P][2] -- as path/<name>.npy, float64.  When
+    the batch holds more than DUMP_BYTES of them, the rows of a sorted sample of problems drawn with
+    a fixed seed are written, so two runs with the same arguments write the same problems."""
+    arrays = {"f": out["f"], "g": out["g"], "c": out["c"][:, :ncnln], "J": out["J"], "result": out["result"]}
+    arrays = {k: v for k, v in arrays.items() if v is not None}
+    P = int(out["f"].shape[0])
+    row_bytes = sum(v[0].numel() * v.element_size() for v in arrays.values())
+    n = min(P, DUMP_BYTES // row_bytes)
+    idx = None
+    if n < P:
+        rows = np.sort(np.random.default_rng(0).choice(P, n, replace=False))
+        idx = torch.from_numpy(rows).to(out["f"].device)
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), (v if idx is None else v.index_select(0, idx)).cpu().numpy())
+
+
 def d2h_ceiling(torch, device, nbytes, reps=3):
     """What the link gives: ONE plain cudaMemcpyAsync of `nbytes` from HBM into pinned host memory
     (torch's non_blocking copy_), best of `reps`; -> GB/s"""
@@ -694,7 +716,12 @@ def main():
     ap.add_argument("--gather", default=os.environ.get("NTG_BENCH_GATHER", "fused"), choices=["fused", "nccl"],
                     help="N > 1: how the 16 B/problem result table reaches every rank")
     ap.add_argument("--ref-step-seconds", type=float, default=1.0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                         f"(rank 0; a fixed sample of problems when the batch holds more than {DUMP_BYTES >> 20} MB)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(a.warmup, 3)
     _quiet_stdout()
 
@@ -765,6 +792,8 @@ def main():
     gather_checked = False
     if peers is not None:
         gather_checked = check_gather(torch, dist, peers, ring["sets"][(a.steps - 1) % ring["nset"]][1]["result"], Ptot)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(torch, ring["sets"][(a.steps - 1) % ring["nset"]][1], pb.dims.ncnln, a.dump_outputs)
 
     ms = torch.tensor([ms_graph if use_graph else rs["ms_per_step"], rs["kernel_ms"], rs["ms_per_step"]],
                       dtype=torch.float64, device="cuda")

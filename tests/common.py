@@ -46,13 +46,18 @@ def load_golden(name):
     return d
 
 
-def golden_spec(name):
+def golden_module():
+    """tests/golden/make_golden.py: the seeded inputs of every fixture"""
     import importlib.util
     p = os.path.join(GOLDEN, "make_golden.py")
     spec = importlib.util.spec_from_file_location("make_golden", p)
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
-    return mod.case_inputs(name)
+    return mod
+
+
+def golden_spec(name):
+    return golden_module().case_inputs(name)
 
 
 GOLDEN_CASES = ["cfg2_vanderpol", "cfg3_kincar", "cfg4_kincar64", "cfg5_syn6", "syn6_small", "endpoint"]

@@ -20,14 +20,6 @@ def port():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    from oracle import oracle
-    if not oracle.have_ref():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    return oracle.Oracle("ref")
-
-
-@pytest.fixture(scope="session")
 def built_libs():
     """The product libraries must exist (built in-tree by __graft_entry__.build())."""
     from ntg_b200 import build

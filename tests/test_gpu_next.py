@@ -7,7 +7,7 @@ import os
 import numpy as np
 import pytest
 
-from common import assert_bitexact, assert_close, golden_spec, load_golden
+from common import GOLDEN, assert_bitexact, assert_close, golden_module, golden_spec, load_golden
 from ntg_b200 import configs
 
 pytestmark = pytest.mark.gpu
@@ -596,30 +596,25 @@ def test_solver_edge_cases(port):
 
 
 @pytest.mark.gpu
-def test_batched_integrate_all_three_rules(ref):
-    """ntgb_integrate against the UNMODIFIED reference's IntegrateVector (src/integrator.c:16-38,
-    compiled into oracle/_ref) for FEULER / BEULER / TRAPEZOID: bit-identical sums on non-uniform times."""
+def test_batched_integrate_all_three_rules():
+    """ntgb_integrate against the UNMODIFIED reference's IntegrateVector (src/integrator.c:16-38) for
+    FEULER / BEULER / TRAPEZOID: bit-identical sums on non-uniform times (tests/golden/integrate.npz)."""
     import ctypes as C
     import torch
     from ntg_b200 import problem
     core = problem.core()
     core.ntgb_integrate.argtypes = [C.c_int, C.c_longlong, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     core.ntgb_integrate.restype = C.c_int
-    rng = np.random.default_rng(11)
-    for n in (1, 2, 17, 401):
-        t = np.sort(rng.uniform(0, 3, n))
-        f = rng.normal(size=(37, n))
+    gm = golden_module()
+    want = np.load(os.path.join(GOLDEN, "integrate.npz"))
+    rows = gm.INTEGRATE_ROWS
+    for t, f in gm.integrate_inputs():
+        n = t.size
+        assert_bitexact(t, want[f"t{n}"], "seeded inputs reproduce")
         fd, td = torch.from_numpy(f).cuda(), torch.from_numpy(t).cuda()
         for rule in (0, 1, 2):
-            out = torch.full((37,), np.nan, dtype=torch.float64, device="cuda")
-            assert core.ntgb_integrate(rule, 37, n, fd.data_ptr(), td.data_ptr(), out.data_ptr(), None) == 0
+            out = torch.full((rows,), np.nan, dtype=torch.float64, device="cuda")
+            assert core.ntgb_integrate(rule, rows, n, fd.data_ptr(), td.data_ptr(), out.data_ptr(), None) == 0
             torch.cuda.synchronize()
-            want = np.zeros(37)
-            for q in range(37):
-                I = C.c_double(0.0)
-                row = np.ascontiguousarray(f[q])
-                ref.lib.IntegrateVector(C.byref(I), row.ctypes.data_as(C.POINTER(C.c_double)),
-                                        t.ctypes.data_as(C.POINTER(C.c_double)), n, rule)
-                want[q] = I.value
-            assert_bitexact(out.cpu().numpy(), want, f"rule {rule}, n {n}")
+            assert_bitexact(out.cpu().numpy(), want[f"I{n}_rule{rule}"], f"rule {rule}, n {n}")
     assert core.ntgb_integrate(7, 1, 2, fd.data_ptr(), td.data_ptr(), out.data_ptr(), None) != 0

@@ -1,10 +1,11 @@
 """The oracle port (oracle/ntg_oracle.c) against the committed golden vectors
-generated from the UNMODIFIED reference (tests/golden/make_golden.py), and --
-where oracle/_ref is present -- against the reference itself, bit for bit."""
+generated from the UNMODIFIED reference (tests/golden/make_golden.py), bit for bit."""
+import os
+
 import numpy as np
 import pytest
 
-from common import GOLDEN_CASES, assert_bitexact, golden_spec, load_golden
+from common import GOLDEN, GOLDEN_CASES, assert_bitexact, golden_module, golden_spec, load_golden
 from ntg_b200 import configs
 
 
@@ -24,39 +25,48 @@ def test_port_matches_golden_bit_exact(port, name):
 
 
 @pytest.mark.parametrize("name", ["cfg2_vanderpol", "cfg4_kincar64", "syn6_small", "endpoint"])
-def test_port_matches_reference_bit_exact(port, ref, name):
-    spec, X = golden_spec(name)
-    rng = np.random.default_rng(11)
-    X = np.vstack([X, rng.uniform(-3, 3, (5, spec.nC))])
-    a = ref.eval(spec, X, linear=True)
+def test_port_matches_reference_bit_exact(port, name):
+    """The golden rows and five more against the reference's outputs for them (rows_<name>.npz: f, g, c;
+    band and dense Jacobians, NaN where the reference never writes, by the sha256 of their bytes); the
+    linear rows, bounds and tables against <name>.npz."""
+    gm = golden_module()
+    spec, X = gm.row_inputs(name)
+    want = np.load(os.path.join(GOLDEN, f"rows_{name}.npz"))
+    assert gm.digest(X) == str(want["X_sha256"]), "seeded inputs reproduce"
     b = port.eval(spec, X, linear=True)
-    assert a["pattern_bad"] == 0, "reference wrote outside / skipped inside the expected band"
-    for k in ("f", "g", "c", "Jband", "Jdense", "A", "bl", "bu"):
-        assert_bitexact(b[k], a[k], f"{name}.{k}")
-    Ba, offa, cola = ref.tables(spec)
+    assert b["pattern_bad"] == 0, "wrote outside / skipped inside the expected band"
+    for k in ("f", "g", "c"):
+        assert_bitexact(b[k], want[k], f"{name}.{k}")
+    g = load_golden(name)
+    assert_bitexact(b["Jband"][:g["X"].shape[0]], g["Jband"], f"{name}.Jband (golden rows)")
+    for k in ("Jband", "Jdense"):
+        assert gm.digest(b[k]) == str(want[k + "_sha256"]), f"{name}.{k}: not bit-identical to the reference"
+    for k in ("A", "bl", "bu"):
+        assert_bitexact(b[k], g[k], f"{name}.{k}")
     Bb, offb, colb = port.tables(spec)
-    for x, y in zip(Ba, Bb):
-        assert_bitexact(y, x, "tables")
-    assert_bitexact(offb, offa, "offsets")
-    assert_bitexact(colb, cola, "pattern")
+    for j, x in enumerate(Bb):
+        assert_bitexact(x, g["B"][j], "tables")
+    assert_bitexact(offb, g["off"], "offsets")
+    assert_bitexact(colb, g["col0"], "pattern")
 
 
 @pytest.mark.parametrize("mode", [0, 1, 2])
-def test_port_modes_match_reference(port, ref, mode):
-    """mode 0 values only, 1 derivatives only, 2 both (reference src/ntg.c:294-334, :354-370).
+def test_port_modes_match_reference(port, mode):
+    """mode 0 values only, 1 derivatives only, 2 both (reference src/ntg.c:294-334, :354-370), against
+    the reference's outputs in each mode (endpoint_modes.npz; mode 2 is endpoint.npz).
     The reference crashes in funcon mode 1 with trajectory constraints (writes through
     C == NULL, src/constraints.c:152-153), so mode 1 is compared on the objective only."""
+    gm = golden_module()
     spec, X = golden_spec("endpoint")
+    m = np.load(os.path.join(GOLDEN, "endpoint_modes.npz"))
+    assert gm.digest(X) == str(m["X_sha256"]), "seeded inputs reproduce"
+    e = load_golden("endpoint")
+    want = {0: {"f": m["mode0_f"], "c": m["mode0_c"]}, 1: {"g": m["mode1_g"]},
+            2: {k: e[k] for k in ("f", "c", "g", "Jband")}}[mode]
     mc = mode if mode != 1 else -1
-    a = ref.eval(spec, X, mode_obj=mode, mode_con=mc)
     b = port.eval(spec, X, mode_obj=mode, mode_con=mc)
-    if mode != 1:
-        assert_bitexact(b["f"], a["f"], "f")
-        assert_bitexact(b["c"], a["c"], "c")
-    if mode != 0:
-        assert_bitexact(b["g"], a["g"], "g")
-    if mode == 2:
-        assert_bitexact(b["Jband"], a["Jband"], "J")
+    for k, v in want.items():
+        assert_bitexact(b[k], v, k)
     full = port.eval(spec, X)
     if mode == 1:
         b1 = port.eval(spec, X, mode_obj=1, mode_con=1)
@@ -64,13 +74,19 @@ def test_port_modes_match_reference(port, ref, mode):
         assert_bitexact(b1["Jband"], full["Jband"], "mode-1 Jacobian equals mode-2 Jacobian")
 
 
-def test_reference_examples_known_answers(ref):
+def test_reference_examples_known_answers(port):
     """SURVEY.md section 8(c)(4): examples/vanderpol.c at its shipped initial guess has
-    objective bps[19]-bps[0] and a gradient summing to 10; kincar at ones(14) has zero cost."""
-    from oracle import oracle
-    ex = load_golden("example_vanderpol")
-    r = oracle.run_reference_example("vanderpol", ex["X"])
-    assert_bitexact(r["f"], ex["f"], "example fixture reproduces")
+    objective bps[19]-bps[0] and a gradient summing to 10; kincar at ones(14) has zero cost.
+    The fixtures hold what the reference's own build of the two example programs returned; the
+    port evaluates the problems they pose (20 breakpoints, no nonlinear constraints) and must
+    reproduce them bit for bit."""
+    def run(spec, ex):
+        r = port.eval(spec, ex["X"], mode_con=-1, dense=False, band=False, linear=True)
+        assert [spec.nC, spec.nclin, spec.ncnln] == list(ex["dims"])
+        for k in ("f", "g", "A", "bl", "bu"):
+            assert_bitexact(r[k], ex[k], f"example fixture reproduces: {k}")
+        return r
+    r = run(configs.vanderpol(20, constraints=False), load_golden("example_vanderpol"))
     # the survey's independent derivation (5.0000000000000036) is good to ~1e-14; the reference itself
     # returns the trapezoid sum of a constant 1 over the accumulated breakpoints
     assert abs(r["f"][0] - 5.0000000000000036) < 1e-14 and r["f"][0] == 5.000000000000001
@@ -78,9 +94,7 @@ def test_reference_examples_known_answers(ref):
                                            1.99998465327921, 2.01328105217118, -0.64058440312767,
                                            2.62731102431689], rtol=0, atol=2e-14)
     np.testing.assert_allclose(r["f"][1], 12.92863341437716, rtol=1e-14)
-    k = load_golden("example_kincar")
-    rk = oracle.run_reference_example("kincar", k["X"])
-    assert_bitexact(rk["f"], k["f"], "kincar fixture reproduces")
+    rk = run(configs.kincar(20, constraints=False), load_golden("example_kincar"))
     assert abs(rk["f"][0]) < 1e-25 and np.abs(rk["g"][0]).max() < 1e-14
 
 
