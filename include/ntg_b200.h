@@ -343,6 +343,40 @@ typedef struct ntgb_sqp_opts {
 int  ntgb_solve_sqp(ntgb_problem *pb, int P, double *C, double *f, double *viol, int *iters, int *status,
                     double *lambda, int *istate, const ntgb_sqp_opts *opts, void *stream);
 
+/*
+ * Per-problem constraint bounds: one call solves P problems that share the setup's functions and
+ * constraint rows but each have their own bounds -- e.g. a batch of MPC problems that start from
+ * different states (the initial state is a linear equality row: lowerb == upperb == x0).
+ *
+ * lowerb / upperb are DEVICE arrays [P][nb], nb = nlic+nltc+nlfc+nnlic+nnltc+nnlfc: row p is problem
+ * p's version of ntgb_setup.lowerb / upperb, compact like them (one value per trajectory constraint,
+ * expanded over the breakpoints as ntgb_get_bounds does); |b| >= 1e19 means "no bound".  NULL with
+ * nb > 0 is NTGB_EINVAL, returned before any CUDA call.  Everything else is as in ntgb_solve_eq /
+ * ntgb_solve_sqp.
+ *
+ * The SETUP's bounds decide the structure: the linear rows with lower == upper there are the equality
+ * rows that get eliminated (ntgb_solve_eq_bounds, like ntgb_solve_eq, refuses nonlinear and inequality
+ * rows).  Each problem's bounds are checked on the device, per problem; the call does not fail for
+ * them.  A problem is rejected when it has a NaN bound or lower > upper, when a row the setup
+ * eliminates has lower != upper, or when its equality right-hand sides are inconsistent (possible only
+ * if the setup's equality rows are dependent; residual > 1e-8 (1 + |b|_inf)).  A rejected problem gets
+ * status NTGB_STATUS_BAD_BOUNDS, its C is left untouched bit for bit, iters is 0, viol is NaN and its
+ * lambda / istate rows are 0; the other problems are solved as if it were absent.
+ *
+ * viol, status, lambda and istate (3 on eliminated rows, 1 / 2 on active rows) are measured against
+ * each problem's own bounds.  Not so ntgb_eval's result[p][1] (max nonlinear violation), which keeps
+ * using the setup's bounds.
+ *
+ * Cost: one extra kernel per call (k_bounds_prep, one warp per problem) and P*nC doubles of
+ * per-problem C_part read by the solver kernels instead of one shared vector.
+ */
+#define NTGB_STATUS_BAD_BOUNDS 5
+int  ntgb_solve_eq_bounds(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb,
+                          double *f, int *iters, int *status, const ntgb_solve_opts *opts, void *stream);
+int  ntgb_solve_sqp_bounds(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb,
+                           double *f, double *viol, int *iters, int *status, double *lambda, int *istate,
+                           const ntgb_sqp_opts *opts, void *stream);
+
 /* Gathered result tables for the fused multi-GPU gather (ntgb_eval_args.peer_result): alloc creates
  * this rank's table (rows x 2 doubles, zeroed) and the 64-byte CUDA IPC handle the other ranks
  * need; open maps another rank's table into this process (peer access over NVLink is enabled on

@@ -113,6 +113,7 @@ class NtgbPack(C.Structure):
 
 
 JAC_NONE, JAC_DENSE, JAC_BAND = 0, 1, 2
+STATUS_BAD_BOUNDS = 5  # NTGB_STATUS_BAD_BOUNDS: the per-problem bounds of that problem were rejected
 ROLES = ("icf", "ucf", "fcf", "nlicf", "nltcf", "nlfcf")
 
 

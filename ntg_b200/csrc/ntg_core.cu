@@ -31,6 +31,7 @@
 #include "ntg_kernel_args.h"
 #include "pgs_device.cuh"
 #include "ntg_sqp.cuh"
+#include "ntg_bounds.h"
 
 namespace {
 
@@ -132,6 +133,7 @@ struct ntgb_problem {
         bool ready = false;
         int nr = 0;
         double *N = nullptr, *Cpart = nullptr; /* device: N [nr][nC] (basis vector k contiguous), Cpart [nC] */
+        double *M = nullptr, *Ae = nullptr;    /* device: Cpart = M b, M [nC][nclin]; A row-major [nclin][nC] */
         int cap = 0;                           /* problems the per-problem scratch below holds */
         double *blob = nullptr;
         int *iblob = nullptr;
@@ -142,6 +144,7 @@ struct ntgb_problem {
         bool ready = false;
         int nr = 0, n_li = 0, m = 0;
         double *N = nullptr, *Cpart = nullptr;
+        double *M = nullptr, *Ae = nullptr; /* Cpart = M be, M [nC][me]; eliminated rows Ae [me][nC] */
         int *li_idx = nullptr;      /* [n_li] linear row of general constraint i */
         double *hl = nullptr, *hu = nullptr; /* [m] bounds: linear inequality rows, then the nonlinear rows */
         double *A = nullptr;        /* dense nclin x nC, column-major (for A_in^T mu) */
@@ -164,6 +167,8 @@ struct ntgb_problem {
     } sqp;
     /* scratch of ntgb_linesearch: trial coefficients, result table, linear violation */
     struct { size_t n = 0; double *Ct = nullptr, *res = nullptr, *lv = nullptr; } ls;
+    /* per-problem bounds of ntgb_solve_*_bounds (k_bounds_prep): Cpart [P][nC], hl / hu [P][m], be [P][me] */
+    struct { size_t n = 0; double *blob = nullptr; } bnd;
 };
 
 namespace {
@@ -344,11 +349,14 @@ __global__ void k_ls_pick(const double *res, const double *lv, const double *alp
  * Per-problem vectors are stored component-major ([k][P]) so that a warp's accesses coalesce. */
 constexpr int kSolveMaxNr = 32;
 
-__global__ void k_solve_init(int P, int nC, int nr, const double *N, const double *Cpart, double *C, double *y,
-                             double *H, int *state, int *iters, int *fails)
+__global__ void k_solve_init(int P, int nC, int nr, const double *N, const double *Cpart, int Cstride, double *C,
+                             double *y, double *H, int *state, int *iters, int *fails)
 {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= P) return;
+    /* per-problem bounds (Cstride = nC): k_bounds_prep has set state / iters, a rejected problem keeps its C */
+    if (Cstride != 0 && state[p] == NTGB_STATUS_BAD_BOUNDS) return;
+    Cpart += (size_t)p * Cstride;
     double *Cp = C + (size_t)p * nC;
     for (int k = 0; k < nr; k++) {
         double a = 0.0;
@@ -467,12 +475,13 @@ __global__ void k_solve_dir(int P, int nC, int nr, const double *N, const double
 }
 
 /* accept the line-search step (or count a failure), rebuild C from the reduced variables */
-__global__ void k_solve_update(int P, int nC, int nr, const double *N, const double *Cpart, const double *phi0,
-                               const double *alpha_best, const double *phi_best, const double *d, double *y,
-                               double *H, double *C, int *state, int *iters, int *fails, int *count)
+__global__ void k_solve_update(int P, int nC, int nr, const double *N, const double *Cpart, int Cstride,
+                               const double *phi0, const double *alpha_best, const double *phi_best, const double *d,
+                               double *y, double *H, double *C, int *state, int *iters, int *fails, int *count)
 {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= P || state[p] != 0) return;
+    Cpart += (size_t)p * Cstride;
     iters[p] += 1;
     if (!(phi_best[p] < phi0[p])) {
         /* no decrease along d: retry once from steepest descent, then give up */
@@ -495,9 +504,11 @@ __global__ void k_solve_update(int P, int nC, int nr, const double *N, const dou
 }
 
 /* Host: orthonormal null-space basis N of A (m x n, column-major) and the minimum-norm solution of
- * A*C = b, by Householder QR with column pivoting of A^T. */
+ * A*C = b, by Householder QR with column pivoting of A^T.  Mop (optional) receives the linear operator
+ * of that solution, Cpart = Mop b for any right-hand side b ([n][m] row-major; zero columns for the
+ * rows the pivoting found dependent), which the per-problem-bounds solvers apply on the device. */
 int reduce_linear(const std::vector<double> &A, int m, int n, const std::vector<double> &b, std::vector<double> &N,
-                  std::vector<double> &Cpart, int &nr)
+                  std::vector<double> &Cpart, int &nr, std::vector<double> *Mop = nullptr)
 {
     std::vector<double> M((size_t)n * std::max(m, 1)), Q((size_t)n * n, 0.0), v(n);
     std::vector<int> perm(m);
@@ -555,6 +566,20 @@ int reduce_linear(const std::vector<double> &A, int m, int n, const std::vector<
     Cpart.assign(n, 0.0);
     for (int l = 0; l < r; l++)
         for (int i = 0; i < n; i++) Cpart[i] += Q[i + (size_t)l * n] * w[l];
+    if (Mop) {
+        /* column j = the same back substitution for b = e_j */
+        Mop->assign((size_t)n * m, 0.0);
+        std::vector<double> wj(r);
+        for (int j = 0; j < m; j++) {
+            for (int i = 0; i < r; i++) {
+                double a = perm[i] == j ? 1.0 : 0.0;
+                for (int l = 0; l < i; l++) a -= M[l + (size_t)i * n] * wj[l];
+                wj[i] = a / M[i + (size_t)i * n];
+            }
+            for (int l = 0; l < r; l++)
+                for (int i = 0; i < n; i++) (*Mop)[(size_t)i * m + j] += Q[i + (size_t)l * n] * wj[l];
+        }
+    }
     double bmax = 0.0, res = 0.0;
     for (int j = 0; j < m; j++) {
         double a = -b[j];
@@ -831,9 +856,9 @@ int alm_prepare(ntgb_problem *pb)
             be[r] = pb->lin_lb[eq[r]];
             for (int c = 0; c < nC; c++) Ae[r + (size_t)c * me] = pb->A[eq[r] + (size_t)c * nclin];
         }
-        std::vector<double> N, Cpart;
+        std::vector<double> N, Cpart, Mop;
         int nr = 0;
-        if ((rc = reduce_linear(Ae, me, nC, be, N, Cpart, nr))) return rc;
+        if ((rc = reduce_linear(Ae, me, nC, be, N, Cpart, nr, &Mop))) return rc;
         al.nr = nr;
         al.hN = N;
         al.eq = eq;
@@ -843,6 +868,13 @@ int alm_prepare(ntgb_problem *pb)
         if (N.empty()) N.push_back(0.0);
         if ((rc = dev_upload(pb, &al.N, N.data(), N.size()))) return rc;
         if ((rc = dev_upload(pb, &al.Cpart, Cpart.data(), Cpart.size()))) return rc;
+        /* for per-problem right-hand sides: Cpart = M be and the rows to check the residual against */
+        std::vector<double> Aer((size_t)std::max(me, 1) * nC, 0.0);
+        for (int r = 0; r < me; r++)
+            for (int c = 0; c < nC; c++) Aer[(size_t)r * nC + c] = Ae[r + (size_t)c * me];
+        if (Mop.empty()) Mop.push_back(0.0);
+        if ((rc = dev_upload(pb, &al.M, Mop.data(), Mop.size()))) return rc;
+        if ((rc = dev_upload(pb, &al.Ae, Aer.data(), Aer.size()))) return rc;
         if (li.empty()) li.push_back(0);
         if ((rc = dev_upload(pb, &al.li_idx, li.data(), li.size()))) return rc;
         /* bounds of the general constraints: NPSOL's bl/bu behind the variables and, for the
@@ -893,7 +925,8 @@ struct SqpDesc {
     const double *N;      /* [nr][nC] */
     const double *ArN;    /* [n_li][nr] reduced gradients of the linear inequality rows */
     const int *li_idx;    /* [n_li] */
-    const double *hl, *hu; /* [m] */
+    const double *hl, *hu; /* [m] per problem, problem p's at hl + p*hstride (0: one shared set) */
+    int Cstride, hstride;  /* per-problem strides of Cpart (0 or nC) and hl / hu (0 or m) */
     double gtol, ctol, rho_pen;
 };
 
@@ -908,16 +941,21 @@ __global__ void k_sqp_init(int P, SqpDesc D, SqpArrays S, const double *Cpart, d
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= P) return;
     const int nC = D.nC, nr = D.nr;
+    /* per-problem bounds: k_bounds_prep has set state / iters; a rejected problem keeps its C */
+    const bool rejected = D.Cstride != 0 && state[p] == NTGB_STATUS_BAD_BOUNDS;
+    Cpart += (size_t)p * D.Cstride;
     double *Cp = C + (size_t)p * nC, *y = S.y + (size_t)p * nr;
-    for (int k = 0; k < nr; k++) {
-        double a = 0.0;
-        for (int e = 0; e < nC; e++) a += D.N[(size_t)k * nC + e] * (Cp[e] - Cpart[e]);
-        y[k] = a;
-    }
-    for (int e = 0; e < nC; e++) {
-        double a = Cpart[e];
-        for (int k = 0; k < nr; k++) a += D.N[(size_t)k * nC + e] * y[k];
-        Cp[e] = a;
+    if (!rejected) {
+        for (int k = 0; k < nr; k++) {
+            double a = 0.0;
+            for (int e = 0; e < nC; e++) a += D.N[(size_t)k * nC + e] * (Cp[e] - Cpart[e]);
+            y[k] = a;
+        }
+        for (int e = 0; e < nC; e++) {
+            double a = Cpart[e];
+            for (int k = 0; k < nr; k++) a += D.N[(size_t)k * nC + e] * y[k];
+            Cp[e] = a;
+        }
     }
     for (int e = 0; e < nr * nr; e++) S.B[(size_t)p * nr * nr + e] = (e / nr == e % nr) ? 1.0 : 0.0;
     for (int i = 0; i < D.m; i++) {
@@ -929,6 +967,10 @@ __global__ void k_sqp_init(int P, SqpDesc D, SqpArrays S, const double *Cpart, d
         S.flag[(size_t)p * 8 + k] = 0;
     }
     S.flag[(size_t)p * 8 + 3] = 1; /* B is the identity */
+    if (rejected) {
+        S.scal[(size_t)p * 8 + 3] = NAN; /* reported violation */
+        return;
+    }
     state[p] = 0;
     iters[p] = 0;
 }
@@ -1017,7 +1059,7 @@ __global__ void k_sqp_step(int P, ntgb_devtab T, SqpDesc D, SqpArrays S, const d
                             S.grLold + (size_t)p * nr, S.grold + (size_t)p * nr, S.d + (size_t)p * nr, S.scal + (size_t)p * 8, S.flag + (size_t)p * 8,
                             S.istate + (size_t)p * m};
     const sqp::StepOpts so{D.gtol, D.ctol, D.rho_pen};
-    sqp::sqp_step(cg, w, st, so, f[p], gr, hrow, D.hl, D.hu, Bm, Lm, vec);
+    sqp::sqp_step(cg, w, st, so, f[p], gr, hrow, D.hl + (size_t)p * D.hstride, D.hu + (size_t)p * D.hstride, Bm, Lm, vec);
     __syncthreads();
     const int status = st.flag[5];
     if (status != 0) {
@@ -1049,10 +1091,11 @@ __global__ void k_sqp_merit(int Q, int nalpha, SqpDesc D, const double *scal, co
     const int lane = threadIdx.x & 31;
     if (q >= Q) return;
     const int p = pidx != nullptr ? pidx[q / nalpha] : q / nalpha;
+    const double *hl = D.hl + (size_t)p * D.hstride, *hu = D.hu + (size_t)p * D.hstride;
     double acc = 0.0;
     for (int i = lane; i < D.m; i += 32) {
         const double h = i < D.n_li ? lin[(size_t)q * D.nclin + D.li_idx[i]] : c[(size_t)q * D.ncnln + (i - D.n_li)];
-        const double lo = D.hl[i], hi = D.hu[i];
+        const double lo = hl[i], hi = hu[i];
         double v = 0.0;
         if (lo > -sqp::kBig && lo - h > v) v = lo - h;
         if (hi < sqp::kBig && h - hi > v) v = h - hi;
@@ -1070,6 +1113,7 @@ __global__ void k_sqp_update(int P, SqpDesc D, SqpArrays S, const double *Cpart,
     if (p >= P || state[p] != 0) return;
     const int nC = D.nC, nr = D.nr;
     int *flag = S.flag + (size_t)p * 8;
+    Cpart += (size_t)p * D.Cstride;
     iters[p] += 1;
     if (!(phi_best[p] < phi0[p])) {
         if (flag[3]) {
@@ -1102,11 +1146,18 @@ __global__ void k_sqp_update(int P, SqpDesc D, SqpArrays S, const double *Cpart,
  * eliminated equality rows are the least-squares solution of Ae' le = g - A_in' l_in - J' l_nl
  * (W = (Ae Ae')^-1 Ae, host-built); gL is that right-hand side in the full space (k_alm_grad). */
 __global__ void k_sqp_outputs(int P, SqpDesc D, SqpArrays S, int me, const int *eq_idx, const double *W, const double *gL,
-                              double *lambda, int *istate)
+                              const int *state, double *lambda, int *istate)
 {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= P) return;
     const int ntot = D.nclin + D.ncnln;
+    if (state[p] == NTGB_STATUS_BAD_BOUNDS) { /* rejected by k_bounds_prep: no multipliers, no active set */
+        for (int i = 0; i < ntot; i++) {
+            if (lambda != nullptr) lambda[(size_t)p * ntot + i] = 0.0;
+            if (istate != nullptr) istate[(size_t)p * ntot + i] = 0;
+        }
+        return;
+    }
     if (lambda != nullptr) {
         double *lp = lambda + (size_t)p * ntot;
         for (int i = 0; i < D.m; i++) lp[i < D.n_li ? D.li_idx[i] : D.nclin + (i - D.n_li)] = S.lam[(size_t)p * D.m + i];
@@ -1122,6 +1173,86 @@ __global__ void k_sqp_outputs(int P, SqpDesc D, SqpArrays S, int me, const int *
         for (int r = 0; r < me; r++) ip[eq_idx[r]] = 3;
     }
 }
+
+/* ---- per-problem bounds (ntgb_solve_eq_bounds / ntgb_solve_sqp_bounds) ----------------------------- */
+struct BoundsDesc {
+    ntgb::BoundsLayout L;
+    int nC, n_li, m, me;
+    const int *li_idx;  /* [n_li] linear rows kept as general rows */
+    const int *eq_idx;  /* [me] eliminated linear rows, nullptr: row r */
+    const double *M;    /* [nC][me] Cpart = M be */
+    const double *Ae;   /* [me][nC] eliminated rows */
+};
+
+/* one warp per problem, once per call: problem p's compact bounds -> hl / hu [m] (SQP order), be [me],
+ * Cpart = M be, and the checks of ntg_bounds.h; a rejected problem gets status 5 and counts as finished */
+__global__ void k_bounds_prep(int P, BoundsDesc B, const double *lowerb, const double *upperb, double *hl, double *hu,
+                              double *be, double *Cpart, int *state, int *iters, int *count)
+{
+    const long long q = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (q >= P) return;
+    const int nb = B.L.nb();
+    const double *lo = lowerb + (size_t)q * nb, *up = upperb + (size_t)q * nb;
+    double *bep = be + (size_t)q * B.me, *Cp = Cpart + (size_t)q * B.nC;
+    unsigned bad = ntgb::bounds_expand(B.L, lo, up, B.li_idx, B.n_li, B.eq_idx, B.me, hl + (size_t)q * B.m,
+                                       hu + (size_t)q * B.m, bep, lane, 32);
+    __syncwarp();
+    for (int e = lane; e < B.nC; e += 32) Cp[e] = ntgb::bounds_cpart(B.M, B.me, bep, e);
+    __syncwarp();
+    double res = 0.0, bmax = 0.0;
+    for (int r = lane; r < B.me; r += 32) {
+        res = ntgb::bounds_max(res, fabs(ntgb::bounds_residual(B.Ae + (size_t)r * B.nC, B.nC, Cp, bep[r])));
+        bmax = fmax(bmax, fabs(bep[r]));
+    }
+    for (int d = 16; d > 0; d >>= 1) {
+        bad |= __shfl_xor_sync(0xffffffffu, bad, d);
+        res = ntgb::bounds_max(res, __shfl_xor_sync(0xffffffffu, res, d));
+        bmax = fmax(bmax, __shfl_xor_sync(0xffffffffu, bmax, d));
+    }
+    if (ntgb::bounds_inconsistent(res, bmax)) bad |= ntgb::kBoundsInconsistent;
+    if (lane == 0) {
+        state[q] = bad ? NTGB_STATUS_BAD_BOUNDS : 0;
+        iters[q] = 0;
+        if (bad) atomicAdd(count, 1);
+    }
+}
+
+/* per-problem bounds: size the scratch (grows with P, never per iteration) and run k_bounds_prep;
+ * returns problem p's Cpart / hl / hu at Cpart + p*nC, hl + p*m, hu + p*m */
+int bounds_prepare(ntgb_problem *pb, int P, const double *lowerb, const double *upperb, const BoundsDesc &B,
+                   cudaStream_t st, int *state, int *iters, int *count, double **Cpart, double **hl, double **hu)
+{
+    const size_t n = (size_t)P * ((size_t)B.nC + 2 * (size_t)B.m + (size_t)B.me);
+    if (n > pb->bnd.n) {
+        CUDA_TRY(cudaStreamSynchronize(st));
+        if (pb->bnd.blob) cudaFree(pb->bnd.blob);
+        pb->bnd.blob = nullptr;
+        pb->bnd.n = 0;
+        CUDA_TRY(cudaMalloc((void **)&pb->bnd.blob, n * sizeof(double)));
+        pb->bnd.n = n;
+    }
+    double *q = pb->bnd.blob;
+    *Cpart = q; q += (size_t)P * B.nC;
+    *hl = q;    q += (size_t)P * B.m;
+    *hu = q;    q += (size_t)P * B.m;
+    double *be = q;
+    const long long threads = (long long)P * 32;
+    CUDA_TRY(launch(k_bounds_prep, (unsigned)((threads + 127) / 128), 128, st, P, B, lowerb, upperb, *hl, *hu, be, *Cpart,
+                    state, iters, count));
+    return 0;
+}
+
+ntgb::BoundsLayout bounds_layout(const ntgb_problem *pb)
+{
+    return ntgb::BoundsLayout{pb->nlic, pb->nltc, pb->nlfc, pb->nnlic, pb->nnltc, pb->nnlfc, pb->dims.nbps};
+}
+
+int solve_eq_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f, int *iters,
+                  int *status, const ntgb_solve_opts *opts, void *stream);
+int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                   double *viol_out, int *iters, int *status, double *lambda, int *istate, const ntgb_sqp_opts *opts,
+                   void *stream);
 
 } /* namespace */
 
@@ -1181,6 +1312,7 @@ void ntgb_destroy(ntgb_problem *pb)
     if (pb->sqp.iblob) cudaFree(pb->sqp.iblob);
     if (pb->red.blob) cudaFree(pb->red.blob);
     if (pb->red.iblob) cudaFree(pb->red.iblob);
+    if (pb->bnd.blob) cudaFree(pb->bnd.blob);
     for (auto &h : pb->hs) {
         double *hsp[] = {h.C, h.f, h.g, h.c, h.J, h.Z, h.result};
         for (double *p : hsp)
@@ -2043,6 +2175,26 @@ int ntgb_solve_eq(ntgb_problem *pb, int P, double *C, double *f, int *iters, int
                   const ntgb_solve_opts *opts, void *stream)
 {
     if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_eq: null argument");
+    return solve_eq_impl(pb, P, C, nullptr, nullptr, f, iters, status, opts, stream);
+}
+
+int ntgb_solve_eq_bounds(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                         int *iters, int *status, const ntgb_solve_opts *opts, void *stream)
+{
+    if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_eq_bounds: null argument");
+    if (bounds_layout(pb).nb() > 0 && (!lowerb || !upperb))
+        return fail(NTGB_EINVAL, "ntgb_solve_eq_bounds: lowerb / upperb is NULL");
+    return solve_eq_impl(pb, P, C, lowerb, upperb, f, iters, status, opts, stream);
+}
+
+} /* extern "C" */
+
+namespace {
+
+/* ntgb_solve_eq and ntgb_solve_eq_bounds: lowerb == nullptr = the setup's bounds for every problem */
+int solve_eq_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f, int *iters,
+                  int *status, const ntgb_solve_opts *opts, void *stream)
+{
     if (P <= 0) return 0;
     const ntgb_dims &dm = pb->dims;
     if (dm.ncnln > 0) return fail(NTGB_EINVAL, "ntgb_solve_eq: problem has %d nonlinear constraints", dm.ncnln);
@@ -2062,9 +2214,9 @@ int ntgb_solve_eq(ntgb_problem *pb, int P, double *C, double *f, int *iters, int
     const int nC = dm.nC;
     int rc;
     if (!pb->red.ready) {
-        std::vector<double> N, Cpart;
+        std::vector<double> N, Cpart, Mop;
         int nr = 0;
-        if ((rc = reduce_linear(pb->A, dm.nclin, nC, pb->lin_lb, N, Cpart, nr))) return rc;
+        if ((rc = reduce_linear(pb->A, dm.nclin, nC, pb->lin_lb, N, Cpart, nr, &Mop))) return rc;
         if (nr > kSolveMaxNr)
             return fail(NTGB_ELIMIT, "ntgb_solve_eq: %d free directions after eliminating the linear constraints (limit %d)",
                         nr, kSolveMaxNr);
@@ -2072,6 +2224,12 @@ int ntgb_solve_eq(ntgb_problem *pb, int P, double *C, double *f, int *iters, int
         if (N.empty()) N.push_back(0.0);
         if ((rc = dev_upload(pb, &pb->red.N, N.data(), N.size()))) return rc;
         if ((rc = dev_upload(pb, &pb->red.Cpart, Cpart.data(), Cpart.size()))) return rc;
+        std::vector<double> Ar((size_t)std::max(dm.nclin, 1) * nC, 0.0);
+        for (int r = 0; r < dm.nclin; r++)
+            for (int c = 0; c < nC; c++) Ar[(size_t)r * nC + c] = pb->A[r + (size_t)c * dm.nclin];
+        if (Mop.empty()) Mop.push_back(0.0);
+        if ((rc = dev_upload(pb, &pb->red.M, Mop.data(), Mop.size()))) return rc;
+        if ((rc = dev_upload(pb, &pb->red.Ae, Ar.data(), Ar.size()))) return rc;
         pb->red.ready = true;
     }
     const int nr = pb->red.nr;
@@ -2106,8 +2264,18 @@ int ntgb_solve_eq(ntgb_problem *pb, int P, double *C, double *f, int *iters, int
     for (int a = 0; a < kNalpha; a++) ha[a] = std::ldexp(1.0, -a);
     CUDA_TRY(cudaMemcpyAsync(alphas, ha, sizeof ha, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
+    const double *Cpart = pb->red.Cpart;
+    int Cstride = 0;
+    if (lowerb) {
+        /* every linear row is eliminated (the refusals above): be = the expanded linear bounds */
+        BoundsDesc B{bounds_layout(pb), nC, 0, 0, dm.nclin, nullptr, nullptr, pb->red.M, pb->red.Ae};
+        double *Cp = nullptr, *hl = nullptr, *hu = nullptr;
+        if ((rc = bounds_prepare(pb, P, lowerb, upperb, B, st, state, its, count, &Cp, &hl, &hu))) return rc;
+        Cpart = Cp;
+        Cstride = nC;
+    }
     const unsigned grid = (unsigned)((P + 127) / 128);
-    CUDA_TRY(launch(k_solve_init, grid, 128, st, P, nC, nr, pb->red.N, pb->red.Cpart, C, y, H, state, its, fails));
+    CUDA_TRY(launch(k_solve_init, grid, 128, st, P, nC, nr, pb->red.N, Cpart, Cstride, C, y, H, state, its, fails));
     ntgb_eval_args a;
     memset(&a, 0, sizeof a);
     a.P = P; a.C = C; a.mode_obj = 2; a.mode_con = -1; a.f = fv; a.g = g; a.jac_layout = NTGB_JAC_NONE; a.stream = st;
@@ -2123,7 +2291,7 @@ int ntgb_solve_eq(ntgb_problem *pb, int P, double *C, double *f, int *iters, int
         }
         if ((rc = ntgb_linesearch(pb, P, C, dC, kNalpha, alphas, 0.0, o.c1, phi0, dphi0, ab, pbest, nullptr, st)))
             return rc;
-        CUDA_TRY(launch(k_solve_update, grid, 128, st, P, nC, nr, pb->red.N, pb->red.Cpart, phi0, ab, pbest, d, y, H,
+        CUDA_TRY(launch(k_solve_update, grid, 128, st, P, nC, nr, pb->red.N, Cpart, Cstride, phi0, ab, pbest, d, y, H,
                         C, state, its, fails, count));
     }
     if (f) {
@@ -2135,6 +2303,10 @@ int ntgb_solve_eq(ntgb_problem *pb, int P, double *C, double *f, int *iters, int
     CUDA_TRY(cudaStreamSynchronize(st));
     return 0;
 }
+
+} /* namespace */
+
+extern "C" {
 
 int ntgb_solve_nlp(ntgb_problem *pb, int P, double *C, double *f, double *viol_out, int *iters, int *status,
                    const ntgb_nlp_opts *opts, void *stream)
@@ -2221,7 +2393,7 @@ int ntgb_solve_nlp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
     CUDA_TRY(cudaMemcpyAsync(alphas, ha, sizeof ha, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemsetAsync(res, 0, sizeof(double) * 2 * Q, st));
     const unsigned grid = (unsigned)((P + 127) / 128);
-    CUDA_TRY(launch(k_solve_init, grid, 128, st, P, nC, nr, al.N, al.Cpart, C, y, H, state, its, fails));
+    CUDA_TRY(launch(k_solve_init, grid, 128, st, P, nC, nr, al.N, al.Cpart, 0, C, y, H, state, its, fails));
     CUDA_TRY(launch(k_alm_prep, grid, 128, st, P, m, o.rho0, lam, rho, violp, fin));
     CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
 
@@ -2289,7 +2461,7 @@ int ntgb_solve_nlp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
                                     dphi0, ab, pbest));
                 }
             }
-            CUDA_TRY(launch(k_solve_update, grid, 128, st, P, nC, nr, al.N, al.Cpart, phi0, ab, pbest, d, y, H, C, state, its,
+            CUDA_TRY(launch(k_solve_update, grid, 128, st, P, nC, nr, al.N, al.Cpart, 0, phi0, ab, pbest, d, y, H, C, state, its,
                             fails, count));
         }
         /* round finished: fresh multipliers at the point reached, then the outer update */
@@ -2314,6 +2486,28 @@ int ntgb_solve_sqp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
                    double *lambda, int *istate, const ntgb_sqp_opts *opts, void *stream)
 {
     if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_sqp: null argument");
+    return solve_sqp_impl(pb, P, C, nullptr, nullptr, f, viol_out, iters, status, lambda, istate, opts, stream);
+}
+
+int ntgb_solve_sqp_bounds(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                          double *viol_out, int *iters, int *status, double *lambda, int *istate,
+                          const ntgb_sqp_opts *opts, void *stream)
+{
+    if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_sqp_bounds: null argument");
+    if (bounds_layout(pb).nb() > 0 && (!lowerb || !upperb))
+        return fail(NTGB_EINVAL, "ntgb_solve_sqp_bounds: lowerb / upperb is NULL");
+    return solve_sqp_impl(pb, P, C, lowerb, upperb, f, viol_out, iters, status, lambda, istate, opts, stream);
+}
+
+} /* extern "C" */
+
+namespace {
+
+/* ntgb_solve_sqp and ntgb_solve_sqp_bounds: lowerb == nullptr = the setup's bounds for every problem */
+int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                   double *viol_out, int *iters, int *status, double *lambda, int *istate, const ntgb_sqp_opts *opts,
+                   void *stream)
+{
     if (P <= 0) return 0;
     const ntgb_dims &dm = pb->dims;
     ntgb_sqp_opts o{100, 1e-6, 1e-8, 1e4, 1e-4, 4};
@@ -2454,15 +2648,25 @@ int ntgb_solve_sqp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
     SqpDesc D;
     D.nC = nC; D.nr = nr; D.m = m; D.n_li = n_li; D.nclin = nclin; D.ncnln = ncnln;
     D.N = al.N; D.ArN = sq.ArN; D.li_idx = al.li_idx; D.hl = al.hl; D.hu = al.hu;
+    D.Cstride = 0; D.hstride = 0;
     D.gtol = o.gtol; D.ctol = o.ctol; D.rho_pen = o.rho_pen;
+    const double *Cpart = al.Cpart;
 
     double ha[kNalpha];
     for (int a = 0; a < kNalpha; a++) ha[a] = std::ldexp(1.0, -a);
     CUDA_TRY(cudaMemcpyAsync(alphas, ha, sizeof ha, cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemsetAsync(res, 0, sizeof(double) * 2 * Q, st));
-    const unsigned grid = (unsigned)((P + 127) / 128);
-    CUDA_TRY(launch(k_sqp_init, grid, 128, st, P, D, S, al.Cpart, C, state, its));
     CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
+    if (lowerb) {
+        BoundsDesc B{bounds_layout(pb), nC, n_li, m, sq.me, al.li_idx, sq.eq_idx, al.M, al.Ae};
+        double *Cp = nullptr, *hl = nullptr, *hu = nullptr;
+        if ((rc = bounds_prepare(pb, P, lowerb, upperb, B, st, state, its, count, &Cp, &hl, &hu))) return rc;
+        Cpart = Cp;
+        D.hl = hl; D.hu = hu;
+        D.Cstride = nC; D.hstride = m;
+    }
+    const unsigned grid = (unsigned)((P + 127) / 128);
+    CUDA_TRY(launch(k_sqp_init, grid, 128, st, P, D, S, Cpart, C, state, its));
     if (smem > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(k_sqp_step, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 
     ntgb_eval_args ea;
@@ -2522,7 +2726,7 @@ int ntgb_solve_sqp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
             CUDA_TRY(launch(k_alm_pick2, (unsigned)((n2 + 127) / 128), 128, st, res, alphas + kN1, idx, n2, kN2, o.c1, phi0, dphi0,
                             ab, pbest));
         }
-        CUDA_TRY(launch(k_sqp_update, grid, 128, st, P, D, S, al.Cpart, phi0, ab, pbest, C, state, its, count));
+        CUDA_TRY(launch(k_sqp_update, grid, 128, st, P, D, S, Cpart, phi0, ab, pbest, C, state, its, count));
     }
     if (lambda || istate) {
         /* gL = g - A_in' l_in - J' l_nl in the full space (k_alm_grad adds dh' mu: mu = -lambda) */
@@ -2530,7 +2734,7 @@ int ntgb_solve_sqp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
         CUDA_TRY(launch(k_scale_copy, (unsigned)((totm + 255) / 256), 256, st, totm, -1.0, (const double *)S.lam, mu));
         const long long tot = (long long)P * nC;
         CUDA_TRY(launch(k_alm_grad, (unsigned)((tot + 127) / 128), 128, st, P, pb->tab, nclin, n_li, al.li_idx, al.A, g, J, mu, gL));
-        CUDA_TRY(launch(k_sqp_outputs, grid, 128, st, P, D, S, sq.me, sq.eq_idx, sq.W, gL, lambda, istate));
+        CUDA_TRY(launch(k_sqp_outputs, grid, 128, st, P, D, S, sq.me, sq.eq_idx, sq.W, gL, (const int *)state, lambda, istate));
     }
     if (f) CUDA_TRY(cudaMemcpyAsync(f, fv, sizeof(double) * Pz, cudaMemcpyDeviceToDevice, st));
     if (viol_out) CUDA_TRY(cudaMemcpy2DAsync(viol_out, sizeof(double), S.scal + 3, 8 * sizeof(double), sizeof(double), Pz,
@@ -2540,6 +2744,10 @@ int ntgb_solve_sqp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
     CUDA_TRY(cudaStreamSynchronize(st));
     return 0;
 }
+
+} /* namespace */
+
+extern "C" {
 
 int ntgb_peer_table_alloc(ntgb_problem *pb, size_t rows, double **table, unsigned char handle[64])
 {

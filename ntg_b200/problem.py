@@ -56,6 +56,10 @@ def core() -> C.CDLL:
         lib.ntgb_solve_nlp.restype = C.c_int
         lib.ntgb_solve_sqp.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 9
         lib.ntgb_solve_sqp.restype = C.c_int
+        lib.ntgb_solve_eq_bounds.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 8
+        lib.ntgb_solve_eq_bounds.restype = C.c_int
+        lib.ntgb_solve_sqp_bounds.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 11
+        lib.ntgb_solve_sqp_bounds.restype = C.c_int
         lib.ntgb_peer_table_alloc.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p), C.c_char_p]
         lib.ntgb_peer_table_open.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p)]
         lib.ntgb_peer_table_close.argtypes = [C.c_void_p, C.c_void_p]
@@ -296,18 +300,39 @@ class Problem:
                                       ab.data_ptr(), pbest.data_ptr(), Cn.data_ptr(), st))
         return ab, pbest, Cn
 
-    def solve_eq(self, Cdev, max_iter=0, gtol=0.0, c1=0.0, check_every=0):
+    def _check_bounds(self, Cdev, lowerb, upperb):
+        """per-problem bounds: both or neither, float64 CUDA tensors [P][spec.nbounds] next to Cdev"""
+        import torch
+        if lowerb is None and upperb is None:
+            return False
+        shape = (Cdev.shape[0], self.spec.nbounds)
+        for name, b in (("lowerb", lowerb), ("upperb", upperb)):
+            if b is None:
+                raise ValueError(f"{name} is missing: per-problem bounds need both lowerb and upperb")
+            if not (b.is_cuda and b.dtype == torch.float64 and b.is_contiguous() and tuple(b.shape) == shape
+                    and b.device == Cdev.device):
+                raise ValueError(f"{name} must be a contiguous float64 tensor of shape {shape} on {Cdev.device}")
+        return True
+
+    def solve_eq(self, Cdev, max_iter=0, gtol=0.0, c1=0.0, check_every=0, lowerb=None, upperb=None):
         """batched reduced-space BFGS (ntgb_solve_eq); Cdev [P][nC] is overwritten with the solutions.
-        Returns f [P], iters [P], status [P] (1 converged, 2 no further decrease, 0 iteration limit)."""
+        Returns f [P], iters [P], status [P] (1 converged, 2 no further decrease, 0 iteration limit).
+        lowerb / upperb [P][spec.nbounds] (device): each problem's own bounds, in the layout of
+        spec.lowerb / upperb (ntgb_solve_eq_bounds; status 5 = that problem's bounds were rejected)."""
         import torch
         P = Cdev.shape[0]
+        per_problem = self._check_bounds(Cdev, lowerb, upperb)
         f = torch.zeros(P, dtype=torch.float64, device=Cdev.device)
         it = torch.zeros(P, dtype=torch.int32, device=Cdev.device)
         stt = torch.zeros(P, dtype=torch.int32, device=Cdev.device)
         opts = SolveOpts(int(max_iter), float(gtol), float(c1), int(check_every))
         st = torch.cuda.current_stream(Cdev.device).cuda_stream
-        _check(core().ntgb_solve_eq(self._h, P, Cdev.data_ptr(), f.data_ptr(), it.data_ptr(), stt.data_ptr(),
-                                    C.addressof(opts), st))
+        if per_problem:
+            _check(core().ntgb_solve_eq_bounds(self._h, P, Cdev.data_ptr(), lowerb.data_ptr(), upperb.data_ptr(),
+                                               f.data_ptr(), it.data_ptr(), stt.data_ptr(), C.addressof(opts), st))
+        else:
+            _check(core().ntgb_solve_eq(self._h, P, Cdev.data_ptr(), f.data_ptr(), it.data_ptr(), stt.data_ptr(),
+                                        C.addressof(opts), st))
         return f, it, stt
 
     def solve_nlp(self, Cdev, max_outer=0, max_inner=0, gtol=0.0, ctol=0.0, rho0=0.0, rho_mul=0.0, rho_max=0.0,
@@ -327,11 +352,14 @@ class Problem:
                                      stt.data_ptr(), C.addressof(opts), st))
         return f, v, it, stt
 
-    def solve_sqp(self, Cdev, max_iter=0, gtol=0.0, ctol=0.0, rho_pen=0.0, c1=0.0, check_every=0, multipliers=False):
+    def solve_sqp(self, Cdev, max_iter=0, gtol=0.0, ctol=0.0, rho_pen=0.0, c1=0.0, check_every=0, multipliers=False,
+                  lowerb=None, upperb=None):
         """batched SQP solve (ntgb_solve_sqp); Cdev [P][nC] is overwritten.  Returns f [P], violation [P],
-        iters [P], status [P] and, with multipliers=True, lambda and istate [P][nclin + ncnln] (NPSOL's order)."""
+        iters [P], status [P] and, with multipliers=True, lambda and istate [P][nclin + ncnln] (NPSOL's order).
+        lowerb / upperb [P][spec.nbounds] (device): each problem's own bounds (ntgb_solve_sqp_bounds)."""
         import torch
         P, d = Cdev.shape[0], self.dims
+        per_problem = self._check_bounds(Cdev, lowerb, upperb)
         f = torch.zeros(P, dtype=torch.float64, device=Cdev.device)
         v = torch.zeros(P, dtype=torch.float64, device=Cdev.device)
         it = torch.zeros(P, dtype=torch.int32, device=Cdev.device)
@@ -342,9 +370,14 @@ class Problem:
             ist = torch.zeros((P, d.nclin + d.ncnln), dtype=torch.int32, device=Cdev.device)
         opts = SqpOpts(int(max_iter), float(gtol), float(ctol), float(rho_pen), float(c1), int(check_every))
         st = torch.cuda.current_stream(Cdev.device).cuda_stream
-        _check(core().ntgb_solve_sqp(self._h, P, Cdev.data_ptr(), f.data_ptr(), v.data_ptr(), it.data_ptr(), stt.data_ptr(),
-                                     lam.data_ptr() if multipliers else None, ist.data_ptr() if multipliers else None,
-                                     C.addressof(opts), st))
+        lam_p, ist_p = (lam.data_ptr(), ist.data_ptr()) if multipliers else (None, None)
+        if per_problem:
+            _check(core().ntgb_solve_sqp_bounds(self._h, P, Cdev.data_ptr(), lowerb.data_ptr(), upperb.data_ptr(),
+                                                f.data_ptr(), v.data_ptr(), it.data_ptr(), stt.data_ptr(), lam_p, ist_p,
+                                                C.addressof(opts), st))
+        else:
+            _check(core().ntgb_solve_sqp(self._h, P, Cdev.data_ptr(), f.data_ptr(), v.data_ptr(), it.data_ptr(),
+                                         stt.data_ptr(), lam_p, ist_p, C.addressof(opts), st))
         return (f, v, it, stt, lam, ist) if multipliers else (f, v, it, stt)
 
     def spline_interp(self, Cdev, tdev):
