@@ -377,6 +377,44 @@ int  ntgb_solve_sqp_bounds(ntgb_problem *pb, int P, double *C, const double *low
                            double *f, double *viol, int *iters, int *status, double *lambda, int *istate,
                            const ntgb_sqp_opts *opts, void *stream);
 
+/*
+ * SQP warm start: solver state carried from one call to the next, for receding-horizon MPC (each step
+ * re-solves nearly the same problem with its initial state moved) and real-time iteration (a fixed
+ * small max_iter per control step).  The reduced space C = C_part + N y depends on the setup's linear
+ * rows, not on the bounds, so the quasi-Newton Hessian B of the reduced Lagrangian in y stays
+ * meaningful from one call to the next, with or without per-problem bounds.
+ *
+ * ntgb_sqp_warm_doubles: n, the doubles in one problem's row of warm-start state for this setup
+ * (prepares the reduced form if needed).
+ *
+ * ntgb_solve_sqp_warm: ntgb_solve_sqp (lowerb == upperb == NULL) or ntgb_solve_sqp_bounds (both
+ * non-NULL, as there) with solver state carried in warm (DEVICE, [P][n], in and out).  Exactly one of
+ * lowerb / upperb NULL, or warm NULL, is NTGB_EINVAL before any CUDA call.
+ *
+ * One row of warm:
+ *   - Rows are independent: row p belongs to problem p and nothing else.  Between calls rows may be
+ *     copied, permuted, gathered or dropped with their problems (problems joining or leaving the
+ *     fleet), and moved to another ntgb_problem created from the same setup (e.g. on another GPU).
+ *   - Content: a header (format tag, nr, m, a 64-bit digest of the reduced form), then the merit
+ *     weight nu and B as nr x nr (layout: ntg_b200/csrc/ntg_warm.h).
+ *   - A row is used only if tag, nr, m and digest all match this setup.  Any other row -- all zeros,
+ *     another setup's, garbage -- is a cold start: B = I, nu = 0, every output bit-identical to
+ *     ntgb_solve_sqp / ntgb_solve_sqp_bounds.  From a matching row a NaN, infinite or negative nu is
+ *     taken as 0 and B is read from its lower triangle; a B that is not positive definite is replaced
+ *     by I.  No content of warm makes a call fail.
+ *   - Warm start: B and nu from the row, no previous step.  If no step from it decreases the merit
+ *     function, the solver restarts once from B = I as it does mid-solve.  The QP's working set is not
+ *     warm-started; lambda / istate are outputs only.
+ *   - On return every problem's row holds its B and nu of the last iteration, for status 0 (iteration
+ *     limit), 1, 2 and 4.  Rows of problems with rejected bounds (NTGB_STATUS_BAD_BOUNDS) are left
+ *     untouched bit for bit, like their C.  A call that fails before the end leaves warm unchanged.
+ * Cost: nr^2 + 6 doubles per problem read once and written once per call.
+ */
+int  ntgb_sqp_warm_doubles(ntgb_problem *pb, size_t *n);
+int  ntgb_solve_sqp_warm(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb,
+                         double *warm, double *f, double *viol, int *iters, int *status, double *lambda,
+                         int *istate, const ntgb_sqp_opts *opts, void *stream);
+
 /* Gathered result tables for the fused multi-GPU gather (ntgb_eval_args.peer_result): alloc creates
  * this rank's table (rows x 2 doubles, zeroed) and the 64-byte CUDA IPC handle the other ranks
  * need; open maps another rank's table into this process (peer access over NVLink is enabled on

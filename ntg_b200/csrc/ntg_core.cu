@@ -32,6 +32,7 @@
 #include "pgs_device.cuh"
 #include "ntg_sqp.cuh"
 #include "ntg_bounds.h"
+#include "ntg_warm.h"
 
 namespace {
 
@@ -150,6 +151,7 @@ struct ntgb_problem {
         double *A = nullptr;        /* dense nclin x nC, column-major (for A_in^T mu) */
         std::vector<double> hN;     /* host copy of N */
         std::vector<int> eq, li;    /* linear rows: eliminated equalities / kept as general constraints */
+        uint64_t digest = 0;        /* ntg_warm.h warm_digest of this reduced form: SQP warm-start rows match it */
         size_t cap = 0, capt = 0;
         double *blob = nullptr, *tblob = nullptr;
         int *iblob = nullptr;
@@ -865,6 +867,7 @@ int alm_prepare(ntgb_problem *pb)
         al.li = li;
         al.n_li = (int)li.size();
         al.m = al.n_li + ncnln;
+        al.digest = ntgb::warm_digest(nC, nr, al.m, al.n_li, li.data(), N.data());
         if (N.empty()) N.push_back(0.0);
         if ((rc = dev_upload(pb, &al.N, N.data(), N.size()))) return rc;
         if ((rc = dev_upload(pb, &al.Cpart, Cpart.data(), Cpart.size()))) return rc;
@@ -936,7 +939,10 @@ struct SqpArrays {
     int *flag, *istate;
 };
 
-__global__ void k_sqp_init(int P, SqpDesc D, SqpArrays S, const double *Cpart, double *C, int *state, int *iters)
+/* warm (ntgb_solve_sqp_warm, nullptr otherwise): a row matching the setup (ntg_warm.h) gives B, nu and
+ * the flags "no previous step, B is not the identity"; any other row starts cold like warm == nullptr */
+__global__ void k_sqp_init(int P, SqpDesc D, SqpArrays S, const double *Cpart, double *C, int *state, int *iters,
+                           const double *warm, ntgb::WarmKey wk)
 {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= P) return;
@@ -957,7 +963,9 @@ __global__ void k_sqp_init(int P, SqpDesc D, SqpArrays S, const double *Cpart, d
             Cp[e] = a;
         }
     }
-    for (int e = 0; e < nr * nr; e++) S.B[(size_t)p * nr * nr + e] = (e / nr == e % nr) ? 1.0 : 0.0;
+    double nu;
+    const bool hot = ntgb::warm_load(warm != nullptr && !rejected ? warm + (size_t)p * ntgb::warm_doubles(nr) : nullptr, wk,
+                                     S.B + (size_t)p * nr * nr, &nu);
     for (int i = 0; i < D.m; i++) {
         S.lam[(size_t)p * D.m + i] = 0.0;
         S.istate[(size_t)p * D.m + i] = 0;
@@ -966,13 +974,25 @@ __global__ void k_sqp_init(int P, SqpDesc D, SqpArrays S, const double *Cpart, d
         S.scal[(size_t)p * 8 + k] = 0.0;
         S.flag[(size_t)p * 8 + k] = 0;
     }
-    S.flag[(size_t)p * 8 + 3] = 1; /* B is the identity */
+    S.scal[(size_t)p * 8] = nu;
+    if (!hot) S.flag[(size_t)p * 8 + 3] = 1; /* B is the identity */
     if (rejected) {
         S.scal[(size_t)p * 8 + 3] = NAN; /* reported violation */
         return;
     }
     state[p] = 0;
     iters[p] = 0;
+}
+
+/* one warp per problem after the iteration loop: B and nu of problem p's last pass into its row of warm;
+ * rows of problems rejected by k_bounds_prep are not touched */
+__global__ void k_sqp_warm_store(int P, SqpArrays S, ntgb::WarmKey wk, const int *state, double *warm)
+{
+    const long long q = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (q >= P || state[q] == NTGB_STATUS_BAD_BOUNDS) return;
+    const int nr = wk.nr;
+    ntgb::warm_encode(warm + (size_t)q * ntgb::warm_doubles(nr), wk, S.scal[(size_t)q * 8], S.B + (size_t)q * nr * nr,
+                      (int)(threadIdx.x & 31), 32);
 }
 
 /* reduced gradient, row values and reduced row gradients of problem p into shared memory, then one
@@ -1250,9 +1270,9 @@ ntgb::BoundsLayout bounds_layout(const ntgb_problem *pb)
 
 int solve_eq_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f, int *iters,
                   int *status, const ntgb_solve_opts *opts, void *stream);
-int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
-                   double *viol_out, int *iters, int *status, double *lambda, int *istate, const ntgb_sqp_opts *opts,
-                   void *stream);
+int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *warm,
+                   double *f, double *viol_out, int *iters, int *status, double *lambda, int *istate,
+                   const ntgb_sqp_opts *opts, void *stream);
 
 } /* namespace */
 
@@ -2486,7 +2506,7 @@ int ntgb_solve_sqp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
                    double *lambda, int *istate, const ntgb_sqp_opts *opts, void *stream)
 {
     if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_sqp: null argument");
-    return solve_sqp_impl(pb, P, C, nullptr, nullptr, f, viol_out, iters, status, lambda, istate, opts, stream);
+    return solve_sqp_impl(pb, P, C, nullptr, nullptr, nullptr, f, viol_out, iters, status, lambda, istate, opts, stream);
 }
 
 int ntgb_solve_sqp_bounds(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
@@ -2496,17 +2516,40 @@ int ntgb_solve_sqp_bounds(ntgb_problem *pb, int P, double *C, const double *lowe
     if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_sqp_bounds: null argument");
     if (bounds_layout(pb).nb() > 0 && (!lowerb || !upperb))
         return fail(NTGB_EINVAL, "ntgb_solve_sqp_bounds: lowerb / upperb is NULL");
-    return solve_sqp_impl(pb, P, C, lowerb, upperb, f, viol_out, iters, status, lambda, istate, opts, stream);
+    return solve_sqp_impl(pb, P, C, lowerb, upperb, nullptr, f, viol_out, iters, status, lambda, istate, opts, stream);
+}
+
+int ntgb_sqp_warm_doubles(ntgb_problem *pb, size_t *n)
+{
+    if (!pb || !n) return fail(NTGB_EINVAL, "ntgb_sqp_warm_doubles: null argument");
+    DeviceGuard dg(pb->device);
+    if (!dg.ok) return fail(NTGB_ECUDA, "cannot select device %d", pb->device);
+    int rc;
+    if ((rc = alm_prepare(pb))) return rc;
+    if (pb->alm.nr < 1) return fail(NTGB_EINVAL, "ntgb_sqp_warm_doubles: the linear equalities leave no free direction");
+    *n = ntgb::warm_doubles(pb->alm.nr);
+    return 0;
+}
+
+int ntgb_solve_sqp_warm(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *warm,
+                        double *f, double *viol_out, int *iters, int *status, double *lambda, int *istate,
+                        const ntgb_sqp_opts *opts, void *stream)
+{
+    if (!pb || !C || !warm) return fail(NTGB_EINVAL, "ntgb_solve_sqp_warm: null argument");
+    if ((lowerb == nullptr) != (upperb == nullptr))
+        return fail(NTGB_EINVAL, "ntgb_solve_sqp_warm: exactly one of lowerb / upperb is NULL");
+    return solve_sqp_impl(pb, P, C, lowerb, upperb, warm, f, viol_out, iters, status, lambda, istate, opts, stream);
 }
 
 } /* extern "C" */
 
 namespace {
 
-/* ntgb_solve_sqp and ntgb_solve_sqp_bounds: lowerb == nullptr = the setup's bounds for every problem */
-int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
-                   double *viol_out, int *iters, int *status, double *lambda, int *istate, const ntgb_sqp_opts *opts,
-                   void *stream)
+/* ntgb_solve_sqp, ntgb_solve_sqp_bounds and ntgb_solve_sqp_warm: lowerb == nullptr = the setup's bounds for
+ * every problem; warm == nullptr = cold start, no state written back */
+int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *warm,
+                   double *f, double *viol_out, int *iters, int *status, double *lambda, int *istate,
+                   const ntgb_sqp_opts *opts, void *stream)
 {
     if (P <= 0) return 0;
     const ntgb_dims &dm = pb->dims;
@@ -2666,7 +2709,8 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
         D.Cstride = nC; D.hstride = m;
     }
     const unsigned grid = (unsigned)((P + 127) / 128);
-    CUDA_TRY(launch(k_sqp_init, grid, 128, st, P, D, S, Cpart, C, state, its));
+    const ntgb::WarmKey wk{nr, m, al.digest};
+    CUDA_TRY(launch(k_sqp_init, grid, 128, st, P, D, S, Cpart, C, state, its, (const double *)warm, wk));
     if (smem > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(k_sqp_step, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 
     ntgb_eval_args ea;
@@ -2728,6 +2772,9 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
         }
         CUDA_TRY(launch(k_sqp_update, grid, 128, st, P, D, S, Cpart, phi0, ab, pbest, C, state, its, count));
     }
+    if (warm)
+        CUDA_TRY(launch(k_sqp_warm_store, (unsigned)(((long long)P * 32 + 127) / 128), 128, st, P, S, wk, (const int *)state,
+                        warm));
     if (lambda || istate) {
         /* gL = g - A_in' l_in - J' l_nl in the full space (k_alm_grad adds dh' mu: mu = -lambda) */
         const long long totm = (long long)P * mz;

@@ -60,6 +60,10 @@ def core() -> C.CDLL:
         lib.ntgb_solve_eq_bounds.restype = C.c_int
         lib.ntgb_solve_sqp_bounds.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 11
         lib.ntgb_solve_sqp_bounds.restype = C.c_int
+        lib.ntgb_sqp_warm_doubles.argtypes = [C.c_void_p, C.POINTER(C.c_size_t)]
+        lib.ntgb_sqp_warm_doubles.restype = C.c_int
+        lib.ntgb_solve_sqp_warm.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 12
+        lib.ntgb_solve_sqp_warm.restype = C.c_int
         lib.ntgb_peer_table_alloc.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p), C.c_char_p]
         lib.ntgb_peer_table_open.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p)]
         lib.ntgb_peer_table_close.argtypes = [C.c_void_p, C.c_void_p]
@@ -352,14 +356,33 @@ class Problem:
                                      stt.data_ptr(), C.addressof(opts), st))
         return f, v, it, stt
 
+    def sqp_warm_doubles(self) -> int:
+        """doubles in one problem's row of SQP warm-start state (ntgb_sqp_warm_doubles)"""
+        n = C.c_size_t(0)
+        _check(core().ntgb_sqp_warm_doubles(self._h, C.byref(n)))
+        return n.value
+
+    def sqp_warm_state(self, P: int):
+        """zeroed warm-start state for P problems, float64 [P][sqp_warm_doubles()] on this Problem's device:
+        every row starts cold; solve_sqp(..., warm=) fills it"""
+        import torch
+        return torch.zeros((P, self.sqp_warm_doubles()), dtype=torch.float64, device=torch.device("cuda", self.device))
+
     def solve_sqp(self, Cdev, max_iter=0, gtol=0.0, ctol=0.0, rho_pen=0.0, c1=0.0, check_every=0, multipliers=False,
-                  lowerb=None, upperb=None):
+                  lowerb=None, upperb=None, warm=None):
         """batched SQP solve (ntgb_solve_sqp); Cdev [P][nC] is overwritten.  Returns f [P], violation [P],
         iters [P], status [P] and, with multipliers=True, lambda and istate [P][nclin + ncnln] (NPSOL's order).
-        lowerb / upperb [P][spec.nbounds] (device): each problem's own bounds (ntgb_solve_sqp_bounds)."""
+        lowerb / upperb [P][spec.nbounds] (device): each problem's own bounds (ntgb_solve_sqp_bounds).
+        warm [P][sqp_warm_doubles()] (device, from sqp_warm_state): solver state carried from the previous
+        call and updated in place (ntgb_solve_sqp_warm)."""
         import torch
         P, d = Cdev.shape[0], self.dims
         per_problem = self._check_bounds(Cdev, lowerb, upperb)
+        if warm is not None:
+            shape = (P, self.sqp_warm_doubles())
+            if not (isinstance(warm, torch.Tensor) and warm.is_cuda and warm.dtype == torch.float64
+                    and warm.is_contiguous() and tuple(warm.shape) == shape and warm.device == Cdev.device):
+                raise ValueError(f"warm must be a contiguous float64 tensor of shape {shape} on {Cdev.device}")
         f = torch.zeros(P, dtype=torch.float64, device=Cdev.device)
         v = torch.zeros(P, dtype=torch.float64, device=Cdev.device)
         it = torch.zeros(P, dtype=torch.int32, device=Cdev.device)
@@ -371,7 +394,12 @@ class Problem:
         opts = SqpOpts(int(max_iter), float(gtol), float(ctol), float(rho_pen), float(c1), int(check_every))
         st = torch.cuda.current_stream(Cdev.device).cuda_stream
         lam_p, ist_p = (lam.data_ptr(), ist.data_ptr()) if multipliers else (None, None)
-        if per_problem:
+        if warm is not None:
+            lo_p, up_p = (lowerb.data_ptr(), upperb.data_ptr()) if per_problem else (None, None)
+            _check(core().ntgb_solve_sqp_warm(self._h, P, Cdev.data_ptr(), lo_p, up_p, warm.data_ptr(), f.data_ptr(),
+                                              v.data_ptr(), it.data_ptr(), stt.data_ptr(), lam_p, ist_p,
+                                              C.addressof(opts), st))
+        elif per_problem:
             _check(core().ntgb_solve_sqp_bounds(self._h, P, Cdev.data_ptr(), lowerb.data_ptr(), upperb.data_ptr(),
                                                 f.data_ptr(), v.data_ptr(), it.data_ptr(), stt.data_ptr(), lam_p, ist_p,
                                                 C.addressof(opts), st))
