@@ -77,6 +77,12 @@ struct DeviceGuard {
     }
 };
 
+/* device scratch of one solver, sized and carved by scratch_carve */
+struct Scratch {
+    void *p = nullptr;
+    size_t bytes = 0;
+};
+
 } /* namespace */
 
 struct ntgb_problem {
@@ -129,22 +135,12 @@ struct ntgb_problem {
         size_t lastP = 0;
     } zc;
     std::vector<double> lin_lb, lin_ub; /* expanded linear bounds, [nclin] */
-    /* reduced-space data of ntgb_solve_eq: C = C_part + N*y */
-    struct {
-        bool ready = false;
-        int nr = 0;
-        double *N = nullptr, *Cpart = nullptr; /* device: N [nr][nC] (basis vector k contiguous), Cpart [nC] */
-        double *M = nullptr, *Ae = nullptr;    /* device: Cpart = M b, M [nC][nclin]; A row-major [nclin][nC] */
-        int cap = 0;                           /* problems the per-problem scratch below holds */
-        double *blob = nullptr;
-        int *iblob = nullptr;
-    } red;
-    /* ntgb_solve_nlp: equality rows eliminated (own N / Cpart), the other linear rows kept as
-     * general constraints next to the nonlinear ones */
+    /* reduced form of the solvers: equality rows eliminated (C = Cpart + N y), the other linear rows
+     * kept as general constraints next to the nonlinear ones */
     struct {
         bool ready = false;
         int nr = 0, n_li = 0, m = 0;
-        double *N = nullptr, *Cpart = nullptr;
+        double *N = nullptr, *Cpart = nullptr; /* N [nr][nC] (basis vector k contiguous), Cpart [nC] */
         double *M = nullptr, *Ae = nullptr; /* Cpart = M be, M [nC][me]; eliminated rows Ae [me][nC] */
         int *li_idx = nullptr;      /* [n_li] linear row of general constraint i */
         double *hl = nullptr, *hu = nullptr; /* [m] bounds: linear inequality rows, then the nonlinear rows */
@@ -152,9 +148,6 @@ struct ntgb_problem {
         std::vector<double> hN;     /* host copy of N */
         std::vector<int> eq, li;    /* linear rows: eliminated equalities / kept as general constraints */
         uint64_t digest = 0;        /* ntg_warm.h warm_digest of this reduced form: SQP warm-start rows match it */
-        size_t cap = 0, capt = 0;
-        double *blob = nullptr, *tblob = nullptr;
-        int *iblob = nullptr;
     } alm;
     /* ntgb_solve_sqp: on top of alm's reduced form */
     struct {
@@ -163,14 +156,10 @@ struct ntgb_problem {
         double *W = nullptr;   /* [me][nC] (Ae Ae')^-1 Ae */
         int *eq_idx = nullptr; /* [me] */
         int me = 0;
-        size_t cap = 0;
-        double *blob = nullptr, *tblob = nullptr;
-        int *iblob = nullptr;
     } sqp;
-    /* scratch of ntgb_linesearch: trial coefficients, result table, linear violation */
-    struct { size_t n = 0; double *Ct = nullptr, *res = nullptr, *lv = nullptr; } ls;
-    /* per-problem bounds of ntgb_solve_*_bounds (k_bounds_prep): Cpart [P][nC], hl / hu [P][m], be [P][me] */
-    struct { size_t n = 0; double *blob = nullptr; } bnd;
+    /* per-call device arrays, kept between calls: one scratch per driver, so that no call's arrays alias
+     * another solver's (ntgb_solve_eq, ntgb_solve_nlp, ntgb_solve_sqp, ntgb_linesearch, per-problem bounds) */
+    struct { Scratch eq, nlp, sqp, ls, bnd; } scratch;
 };
 
 namespace {
@@ -204,6 +193,66 @@ int dev_upload(ntgb_problem *pb, T **ptr, const T *src, size_t n)
     int rc = dev_alloc(pb, ptr, n);
     if (rc) return rc;
     if (n) CUDA_TRY(cudaMemcpy(*ptr, src, n * sizeof(T), cudaMemcpyHostToDevice));
+    return 0;
+}
+
+/* one pass over a scratch layout: take(n, p...) hands each p the next n elements, every array starting on a
+ * 256-byte boundary as if it had been allocated alone; with a null base the pass only counts bytes */
+struct Carve {
+    char *base;
+    size_t off = 0;
+    template <class... T>
+    void take(size_t n, T *&...p)
+    {
+        (one(p, n), ...);
+    }
+    template <class T>
+    void one(T *&p, size_t n)
+    {
+        off = (off + 255) & ~(size_t)255;
+        p = base ? reinterpret_cast<T *>(base + off) : nullptr;
+        off += n * sizeof(T);
+    }
+};
+
+/* layout(Carve &) takes every array of a call once, in order: it runs once to size s and once to hand out the
+ * pointers.  s grows when the call needs more and never shrinks; the old buffer may still be in use by work
+ * queued on st, so st is synchronized before it is freed. */
+template <class Layout>
+int scratch_carve(Scratch &s, cudaStream_t st, Layout layout)
+{
+    Carve size{nullptr};
+    layout(size);
+    if (size.off > s.bytes) {
+        CUDA_TRY(cudaStreamSynchronize(st));
+        cudaFree(s.p);
+        s.p = nullptr;
+        s.bytes = 0;
+        CUDA_TRY(cudaMalloc(&s.p, size.off));
+        s.bytes = size.off;
+    }
+    Carve c{static_cast<char *>(s.p)};
+    layout(c);
+    if (c.off != size.off)
+        return fail(NTGB_EINVAL, "internal error: a scratch layout of %zu bytes carved %zu", size.off, c.off);
+    return 0;
+}
+
+/* 1 when all P problems have counted themselves finished in *count, 0 when not, < 0 on a CUDA error */
+int all_finished(const int *count, int P, cudaStream_t st)
+{
+    int done = 0;
+    CUDA_TRY(cudaMemcpyAsync(&done, count, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return done >= P ? 1 : 0;
+}
+
+/* step table of the solvers' line searches: alpha[a] = 2^-a, n <= 16 */
+int upload_halving(double *alpha, int n, cudaStream_t st)
+{
+    double ha[16];
+    for (int a = 0; a < n; a++) ha[a] = std::ldexp(1.0, -a);
+    CUDA_TRY(cudaMemcpyAsync(alpha, ha, sizeof(double) * n, cudaMemcpyHostToDevice, st));
     return 0;
 }
 
@@ -725,8 +774,9 @@ __global__ void k_alm_prep(int P, int m, double rho0, double *lam, double *rho, 
     fin[p] = 0;
 }
 
-/* two-stage line search of ntgb_solve_nlp: the coarse steps are tried for every problem, the fine
- * ones only for the problems (listed in idx) that found no Armijo step among them */
+/* k_ls_trial for the second stage of two_stage_search: the trial points of the n problems listed in idx.  Kept
+ * apart from k_ls_trial: an optional index list there made ntgb_linesearch slower (65 536 problems x 12 steps:
+ * 749.7 against 741.6 us on a B200 at 1000 W) and ntgb_solve_nlp 0.7 % slower. */
 __global__ void k_ls_trial_idx(const double *C, const double *dC, const double *alpha, const int *idx, int n, int nalpha,
                                int nC, double *Ct)
 {
@@ -740,7 +790,7 @@ __global__ void k_ls_trial_idx(const double *C, const double *dC, const double *
     Ct[q] = C[p * nC + e] + alpha[a] * dC[p * nC + e];
 }
 
-/* stage 1: first coarse alpha with Armijo decrease, else the best one seen; problems without an
+/* stage 1 of two_stage_search: first coarse alpha with Armijo decrease, else the best one seen; problems without an
  * Armijo step (and still running) are appended to idx */
 __global__ void k_alm_pick1(const double *res, const double *alpha, int P, int nalpha, double c1, const double *phi0,
                             const double *dphi0, const int *state, double *alpha_best, double *phi_best, int *idx,
@@ -839,7 +889,7 @@ void host_band_row(const ntgb_problem *pb, const double *dz, int bp, double *ban
     }
 }
 
-/* reduced form shared by ntgb_solve_nlp and ntgb_solve_sqp: linear equality rows eliminated
+/* reduced form shared by ntgb_solve_eq, ntgb_solve_nlp and ntgb_solve_sqp: linear equality rows eliminated
  * (C = Cpart + N y), the other linear rows and the nonlinear rows kept as general constraints */
 int alm_prepare(ntgb_problem *pb)
 {
@@ -894,6 +944,73 @@ int alm_prepare(ntgb_problem *pb)
         if ((rc = dev_upload(pb, &al.A, Ad.data(), Ad.size()))) return rc;
     }
     al.ready = true;
+    return 0;
+}
+
+/* the SQP entry points (`who`): alm's reduced form, which must leave a free direction, and once per problem
+ * the reduced gradients ArN of the linear inequality rows and W = (Ae Ae')^-1 Ae for the multipliers of the
+ * eliminated equality rows */
+int sqp_prepare(ntgb_problem *pb, const char *who)
+{
+    int rc;
+    if ((rc = alm_prepare(pb))) return rc;
+    const auto &al = pb->alm;
+    if (al.nr < 1) return fail(NTGB_EINVAL, "%s: the linear equalities leave no free direction", who);
+    auto &sq = pb->sqp;
+    if (sq.ready) return 0;
+    const int nC = pb->dims.nC, nclin = pb->dims.nclin, nr = al.nr, n_li = al.n_li;
+    std::vector<double> ArN((size_t)std::max(n_li, 1) * nr, 0.0);
+    for (int i = 0; i < n_li; i++)
+        for (int k = 0; k < nr; k++) {
+            double a = 0.0;
+            for (int e = 0; e < nC; e++) a += pb->A[al.li[i] + (size_t)e * nclin] * al.hN[(size_t)k * nC + e];
+            ArN[(size_t)i * nr + k] = a;
+        }
+    if ((rc = dev_upload(pb, &sq.ArN, ArN.data(), ArN.size()))) return rc;
+    const int me = (int)al.eq.size();
+    std::vector<double> W((size_t)std::max(me, 1) * nC, 0.0), G((size_t)std::max(me, 1) * std::max(me, 1), 0.0);
+    for (int r = 0; r < me; r++)
+        for (int s = 0; s < me; s++) {
+            double a = 0.0;
+            for (int e = 0; e < nC; e++) a += pb->A[al.eq[r] + (size_t)e * nclin] * pb->A[al.eq[s] + (size_t)e * nclin];
+            G[(size_t)r * me + s] = a;
+        }
+    /* Gauss-Jordan with partial pivoting on [G | Ae]; dependent rows get zero multipliers */
+    for (int r = 0; r < me; r++)
+        for (int e = 0; e < nC; e++) W[(size_t)r * nC + e] = pb->A[al.eq[r] + (size_t)e * nclin];
+    double gmax = 0.0;
+    for (int r = 0; r < me; r++) gmax = std::max(gmax, std::fabs(G[(size_t)r * me + r]));
+    std::vector<char> dead(std::max(me, 1), 0);
+    for (int k = 0; k < me; k++) {
+        int piv = -1;
+        double best = 1e-12 * std::max(gmax, 1e-300);
+        for (int r = k; r < me; r++)
+            if (std::fabs(G[(size_t)r * me + k]) > best) { best = std::fabs(G[(size_t)r * me + k]); piv = r; }
+        if (piv < 0) { dead[k] = 1; continue; }
+        if (piv != k) {
+            for (int s = 0; s < me; s++) std::swap(G[(size_t)k * me + s], G[(size_t)piv * me + s]);
+            for (int e = 0; e < nC; e++) std::swap(W[(size_t)k * nC + e], W[(size_t)piv * nC + e]);
+        }
+        const double d = G[(size_t)k * me + k];
+        for (int s = 0; s < me; s++) G[(size_t)k * me + s] /= d;
+        for (int e = 0; e < nC; e++) W[(size_t)k * nC + e] /= d;
+        for (int r = 0; r < me; r++) {
+            if (r == k) continue;
+            const double t = G[(size_t)r * me + k];
+            if (t == 0.0) continue;
+            for (int s = 0; s < me; s++) G[(size_t)r * me + s] -= t * G[(size_t)k * me + s];
+            for (int e = 0; e < nC; e++) W[(size_t)r * nC + e] -= t * W[(size_t)k * nC + e];
+        }
+    }
+    for (int k = 0; k < me; k++)
+        if (dead[k])
+            for (int e = 0; e < nC; e++) W[(size_t)k * nC + e] = 0.0;
+    if ((rc = dev_upload(pb, &sq.W, W.data(), W.size()))) return rc;
+    std::vector<int> eqi = al.eq;
+    if (eqi.empty()) eqi.push_back(0);
+    if ((rc = dev_upload(pb, &sq.eq_idx, eqi.data(), eqi.size()))) return rc;
+    sq.me = me;
+    sq.ready = true;
     return 0;
 }
 
@@ -1243,20 +1360,15 @@ __global__ void k_bounds_prep(int P, BoundsDesc B, const double *lowerb, const d
 int bounds_prepare(ntgb_problem *pb, int P, const double *lowerb, const double *upperb, const BoundsDesc &B,
                    cudaStream_t st, int *state, int *iters, int *count, double **Cpart, double **hl, double **hu)
 {
-    const size_t n = (size_t)P * ((size_t)B.nC + 2 * (size_t)B.m + (size_t)B.me);
-    if (n > pb->bnd.n) {
-        CUDA_TRY(cudaStreamSynchronize(st));
-        if (pb->bnd.blob) cudaFree(pb->bnd.blob);
-        pb->bnd.blob = nullptr;
-        pb->bnd.n = 0;
-        CUDA_TRY(cudaMalloc((void **)&pb->bnd.blob, n * sizeof(double)));
-        pb->bnd.n = n;
-    }
-    double *q = pb->bnd.blob;
-    *Cpart = q; q += (size_t)P * B.nC;
-    *hl = q;    q += (size_t)P * B.m;
-    *hu = q;    q += (size_t)P * B.m;
-    double *be = q;
+    const size_t Pz = (size_t)P;
+    double *be;
+    int rc;
+    if ((rc = scratch_carve(pb->scratch.bnd, st, [&](Carve &c) {
+             c.take(Pz * B.nC, *Cpart);
+             c.take(Pz * B.m, *hl, *hu);
+             c.take(Pz * B.me, be);
+         })))
+        return rc;
     const long long threads = (long long)P * 32;
     CUDA_TRY(launch(k_bounds_prep, (unsigned)((threads + 127) / 128), 128, st, P, B, lowerb, upperb, *hl, *hu, be, *Cpart,
                     state, iters, count));
@@ -1266,6 +1378,83 @@ int bounds_prepare(ntgb_problem *pb, int P, const double *lowerb, const double *
 ntgb::BoundsLayout bounds_layout(const ntgb_problem *pb)
 {
     return ntgb::BoundsLayout{pb->nlic, pb->nltc, pb->nlfc, pb->nnlic, pb->nnltc, pb->nnlfc, pb->dims.nbps};
+}
+
+/* ---- two-stage Armijo search of ntgb_solve_nlp and ntgb_solve_sqp ------------------------------------------
+ * the steps 1 .. 1/8 for every problem in one evaluation; the steps 2^-4 .. 2^-15 only for the problems that
+ * found no Armijo step among them (compacted by index), in a second one */
+constexpr int kN1 = 4, kN2 = 12, kNalpha = kN1 + kN2;
+
+struct TwoStage {
+    double *alphas;                 /* [kNalpha] 2^-a */
+    double *Ct, *ft, *ct, *lint;    /* trial points and what is evaluated there, up to Q = P*kNalpha of them */
+    double *res;                    /* [Q][2]: the merit at trial q in res[2q] */
+    int *idx, *nidx;                /* [P] problems of the second stage, and their number */
+    double *ab, *pbest;             /* [P] chosen step and its merit */
+
+    /* the evaluator counts trial points in int */
+    static int check_size(int P)
+    {
+        return (size_t)P * kNalpha > 0x7fffffffull ? fail(NTGB_EINVAL, "P*nalpha too large") : 0;
+    }
+    void take(Carve &c, size_t P, const ntgb_dims &dm)
+    {
+        const size_t Q = P * kNalpha;
+        c.take(kNalpha, alphas);
+        c.take(Q * dm.nC, Ct);
+        c.take(Q, ft);
+        c.take(Q * std::max(dm.ncnln, 1), ct);
+        c.take(Q * std::max(dm.nclin, 1), lint);
+        c.take(2 * Q, res);
+        c.take(P, idx, ab, pbest);
+        c.take(1, nidx);
+    }
+    /* once per call */
+    int start(int P, cudaStream_t st) const
+    {
+        int rc;
+        if ((rc = upload_halving(alphas, kNalpha, st))) return rc;
+        CUDA_TRY(cudaMemsetAsync(res, 0, sizeof(double) * 2 * kNalpha * (size_t)P, st));
+        return 0;
+    }
+};
+
+/* the search from C along dC for P problems; merit(n, nalpha, pidx) launches the merit kernel on the n trial
+ * points just evaluated, trial q belonging to problem pidx[q / nalpha] (pidx == nullptr: q / nalpha) */
+template <class Merit>
+int two_stage_search(ntgb_problem *pb, int P, const double *C, const double *dC, double c1, const double *phi0,
+                     const double *dphi0, const int *state, const TwoStage &ts, cudaStream_t st, Merit merit)
+{
+    const int nC = pb->dims.nC;
+    ntgb_eval_args et;
+    memset(&et, 0, sizeof et);
+    et.C = ts.Ct; et.mode_obj = 0; et.mode_con = pb->dims.ncnln > 0 ? 0 : -1; et.f = ts.ft; et.c = ts.ct;
+    et.jac_layout = NTGB_JAC_NONE; et.stream = st;
+    auto trials = [&](int n, int nalpha, const double *alpha, const int *pidx) -> int {
+        const unsigned grid = (unsigned)(((long long)n * nalpha * nC + 255) / 256);
+        if (pidx == nullptr)
+            CUDA_TRY(launch(k_ls_trial, grid, 256, st, C, dC, alpha, n, nalpha, nC, ts.Ct));
+        else
+            CUDA_TRY(launch(k_ls_trial_idx, grid, 256, st, C, dC, alpha, pidx, n, nalpha, nC, ts.Ct));
+        et.P = n * nalpha;
+        int rc;
+        if ((rc = ntgb_eval(pb, &et))) return rc;
+        if (pb->alm.n_li > 0 && (rc = ntgb_eval_linear(pb, et.P, ts.Ct, ts.lint, nullptr, st))) return rc;
+        return merit(et.P, nalpha, pidx);
+    };
+    int rc;
+    if ((rc = trials(P, kN1, ts.alphas, nullptr))) return rc;
+    CUDA_TRY(cudaMemsetAsync(ts.nidx, 0, sizeof(int), st));
+    CUDA_TRY(launch(k_alm_pick1, (unsigned)((P + 127) / 128), 128, st, ts.res, ts.alphas, P, kN1, c1, phi0, dphi0, state,
+                    ts.ab, ts.pbest, ts.idx, ts.nidx));
+    int n2 = 0;
+    CUDA_TRY(cudaMemcpyAsync(&n2, ts.nidx, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if (n2 <= 0) return 0;
+    if ((rc = trials(n2, kN2, ts.alphas + kN1, ts.idx))) return rc;
+    CUDA_TRY(launch(k_alm_pick2, (unsigned)((n2 + 127) / 128), 128, st, ts.res, ts.alphas + kN1, ts.idx, n2, kN2, c1, phi0,
+                    dphi0, ts.ab, ts.pbest));
+    return 0;
 }
 
 int solve_eq_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f, int *iters,
@@ -1320,19 +1509,9 @@ void ntgb_destroy(ntgb_problem *pb)
     if (!pb) return;
     DeviceGuard dg(pb->device);
     for (void *p : pb->allocs) cudaFree(p);
-    if (pb->ls.Ct) cudaFree(pb->ls.Ct);
-    if (pb->ls.res) cudaFree(pb->ls.res);
-    if (pb->ls.lv) cudaFree(pb->ls.lv);
     if (pb->zc.buf) cudaFreeHost(pb->zc.buf);
-    if (pb->alm.blob) cudaFree(pb->alm.blob);
-    if (pb->alm.tblob) cudaFree(pb->alm.tblob);
-    if (pb->alm.iblob) cudaFree(pb->alm.iblob);
-    if (pb->sqp.blob) cudaFree(pb->sqp.blob);
-    if (pb->sqp.tblob) cudaFree(pb->sqp.tblob);
-    if (pb->sqp.iblob) cudaFree(pb->sqp.iblob);
-    if (pb->red.blob) cudaFree(pb->red.blob);
-    if (pb->red.iblob) cudaFree(pb->red.iblob);
-    if (pb->bnd.blob) cudaFree(pb->bnd.blob);
+    auto &s = pb->scratch;
+    for (Scratch *sc : {&s.eq, &s.nlp, &s.sqp, &s.ls, &s.bnd}) cudaFree(sc->p);
     for (auto &h : pb->hs) {
         double *hsp[] = {h.C, h.f, h.g, h.c, h.J, h.Z, h.result};
         for (double *p : hsp)
@@ -2161,32 +2340,24 @@ int ntgb_linesearch(ntgb_problem *pb, int P, const double *C, const double *dC, 
     const size_t n = (size_t)P * nalpha;
     if (n > 0x7fffffffull) return fail(NTGB_EINVAL, "P*nalpha too large");
     cudaStream_t st = (cudaStream_t)stream;
-    if (n > pb->ls.n) {
-        CUDA_TRY(cudaStreamSynchronize(st));
-        if (pb->ls.Ct) cudaFree(pb->ls.Ct);
-        if (pb->ls.res) cudaFree(pb->ls.res);
-        if (pb->ls.lv) cudaFree(pb->ls.lv);
-        pb->ls.Ct = pb->ls.res = pb->ls.lv = nullptr;
-        pb->ls.n = 0;
-        CUDA_TRY(cudaMalloc((void **)&pb->ls.Ct, n * d.nC * sizeof(double)));
-        CUDA_TRY(cudaMalloc((void **)&pb->ls.res, n * 2 * sizeof(double)));
-        CUDA_TRY(cudaMalloc((void **)&pb->ls.lv, n * sizeof(double)));
-        pb->ls.n = n;
-    }
+    double *Ct, *res, *lv; /* trial coefficients, result table, linear violation */
+    int rc;
+    if ((rc = scratch_carve(pb->scratch.ls, st, [&](Carve &c) {
+             c.take(n * d.nC, Ct);
+             c.take(n * 2, res);
+             c.take(n, lv);
+         })))
+        return rc;
     const long long total = (long long)n * d.nC;
-    CUDA_TRY(launch(k_ls_trial, (unsigned)((total + 255) / 256), 256, st, C, dC, alpha, P, nalpha, d.nC, pb->ls.Ct));
+    CUDA_TRY(launch(k_ls_trial, (unsigned)((total + 255) / 256), 256, st, C, dC, alpha, P, nalpha, d.nC, Ct));
     ntgb_eval_args a;
     memset(&a, 0, sizeof a);
-    a.P = (int)n; a.C = pb->ls.Ct; a.mode_obj = 0; a.mode_con = d.ncnln > 0 ? 0 : -1;
-    a.result = pb->ls.res; a.jac_layout = NTGB_JAC_NONE; a.stream = st;
-    int rc = ntgb_eval(pb, &a);
-    if (rc) return rc;
+    a.P = (int)n; a.C = Ct; a.mode_obj = 0; a.mode_con = d.ncnln > 0 ? 0 : -1;
+    a.result = res; a.jac_layout = NTGB_JAC_NONE; a.stream = st;
+    if ((rc = ntgb_eval(pb, &a))) return rc;
     const bool lin = d.nclin > 0;
-    if (lin) {
-        rc = ntgb_eval_linear(pb, (int)n, pb->ls.Ct, nullptr, pb->ls.lv, st);
-        if (rc) return rc;
-    }
-    CUDA_TRY(launch(k_ls_pick, (unsigned)((P + 127) / 128), 128, st, pb->ls.res, lin ? pb->ls.lv : nullptr, alpha, P,
+    if (lin && (rc = ntgb_eval_linear(pb, (int)n, Ct, nullptr, lv, st))) return rc;
+    CUDA_TRY(launch(k_ls_pick, (unsigned)((P + 127) / 128), 128, st, res, lin ? lv : nullptr, alpha, P,
                     nalpha, mu, c1, phi0, dphi0, C, dC, d.nC, alpha_best, phi_best, C_new));
     return 0;
 }
@@ -2233,85 +2404,54 @@ int solve_eq_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, cons
     cudaStream_t st = (cudaStream_t)stream;
     const int nC = dm.nC;
     int rc;
-    if (!pb->red.ready) {
-        std::vector<double> N, Cpart, Mop;
-        int nr = 0;
-        if ((rc = reduce_linear(pb->A, dm.nclin, nC, pb->lin_lb, N, Cpart, nr, &Mop))) return rc;
-        if (nr > kSolveMaxNr)
-            return fail(NTGB_ELIMIT, "ntgb_solve_eq: %d free directions after eliminating the linear constraints (limit %d)",
-                        nr, kSolveMaxNr);
-        pb->red.nr = nr;
-        if (N.empty()) N.push_back(0.0);
-        if ((rc = dev_upload(pb, &pb->red.N, N.data(), N.size()))) return rc;
-        if ((rc = dev_upload(pb, &pb->red.Cpart, Cpart.data(), Cpart.size()))) return rc;
-        std::vector<double> Ar((size_t)std::max(dm.nclin, 1) * nC, 0.0);
-        for (int r = 0; r < dm.nclin; r++)
-            for (int c = 0; c < nC; c++) Ar[(size_t)r * nC + c] = pb->A[r + (size_t)c * dm.nclin];
-        if (Mop.empty()) Mop.push_back(0.0);
-        if ((rc = dev_upload(pb, &pb->red.M, Mop.data(), Mop.size()))) return rc;
-        if ((rc = dev_upload(pb, &pb->red.Ae, Ar.data(), Ar.size()))) return rc;
-        pb->red.ready = true;
-    }
-    const int nr = pb->red.nr;
+    /* every linear row is an equality (the refusals above), so alm's reduced form eliminates all of them */
+    if ((rc = alm_prepare(pb))) return rc;
+    const auto &al = pb->alm;
+    if (al.nr > kSolveMaxNr)
+        return fail(NTGB_ELIMIT, "ntgb_solve_eq: %d free directions after eliminating the linear constraints (limit %d)",
+                    al.nr, kSolveMaxNr);
+    const int nr = al.nr;
     constexpr int kNalpha = 12;
-    if (P > pb->red.cap) {
-        CUDA_TRY(cudaStreamSynchronize(st));
-        if (pb->red.blob) cudaFree(pb->red.blob);
-        if (pb->red.iblob) cudaFree(pb->red.iblob);
-        pb->red.blob = nullptr; pb->red.iblob = nullptr; pb->red.cap = 0;
-        const size_t nd = (size_t)P * ((size_t)4 * nr + (size_t)nr * nr + 2 * (size_t)nC + 5) + kNalpha;
-        CUDA_TRY(cudaMalloc((void **)&pb->red.blob, nd * sizeof(double)));
-        CUDA_TRY(cudaMalloc((void **)&pb->red.iblob, ((size_t)3 * P + 1) * sizeof(int)));
-        pb->red.cap = P;
-    }
-    const size_t cap = (size_t)pb->red.cap;
-    double *q = pb->red.blob;
-    double *y = q;      q += cap * nr;
-    double *yp = q;     q += cap * nr;
-    double *grp = q;    q += cap * nr;
-    double *d = q;      q += cap * nr;
-    double *H = q;      q += cap * nr * nr;
-    double *dC = q;     q += cap * nC;
-    double *g = q;      q += cap * nC;
-    double *fv = q;     q += cap;
-    double *phi0 = q;   q += cap;
-    double *dphi0 = q;  q += cap;
-    double *ab = q;     q += cap;
-    double *pbest = q;  q += cap;
-    double *alphas = q;
-    int *state = pb->red.iblob, *its = state + cap, *fails = its + cap, *count = fails + cap;
-    double ha[kNalpha];
-    for (int a = 0; a < kNalpha; a++) ha[a] = std::ldexp(1.0, -a);
-    CUDA_TRY(cudaMemcpyAsync(alphas, ha, sizeof ha, cudaMemcpyHostToDevice, st));
+    const size_t Pz = (size_t)P;
+    double *y, *yp, *grp, *d, *H, *dC, *g, *fv, *phi0, *dphi0, *ab, *pbest, *alphas;
+    int *state, *its, *fails, *count;
+    if ((rc = scratch_carve(pb->scratch.eq, st, [&](Carve &c) {
+             c.take(Pz * nr, y, yp, grp, d);
+             c.take(Pz * nr * nr, H);
+             c.take(Pz * nC, dC, g);
+             c.take(Pz, fv, phi0, dphi0, ab, pbest, state, its, fails);
+             c.take(kNalpha, alphas);
+             c.take(1, count);
+         })))
+        return rc;
+    if ((rc = upload_halving(alphas, kNalpha, st))) return rc;
     CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
-    const double *Cpart = pb->red.Cpart;
+    const double *Cpart = al.Cpart;
     int Cstride = 0;
     if (lowerb) {
-        /* every linear row is eliminated (the refusals above): be = the expanded linear bounds */
-        BoundsDesc B{bounds_layout(pb), nC, 0, 0, dm.nclin, nullptr, nullptr, pb->red.M, pb->red.Ae};
+        /* be = the expanded linear bounds, row r of be is linear row r */
+        BoundsDesc B{bounds_layout(pb), nC, 0, 0, dm.nclin, nullptr, nullptr, al.M, al.Ae};
         double *Cp = nullptr, *hl = nullptr, *hu = nullptr;
         if ((rc = bounds_prepare(pb, P, lowerb, upperb, B, st, state, its, count, &Cp, &hl, &hu))) return rc;
         Cpart = Cp;
         Cstride = nC;
     }
     const unsigned grid = (unsigned)((P + 127) / 128);
-    CUDA_TRY(launch(k_solve_init, grid, 128, st, P, nC, nr, pb->red.N, Cpart, Cstride, C, y, H, state, its, fails));
+    CUDA_TRY(launch(k_solve_init, grid, 128, st, P, nC, nr, al.N, Cpart, Cstride, C, y, H, state, its, fails));
     ntgb_eval_args a;
     memset(&a, 0, sizeof a);
     a.P = P; a.C = C; a.mode_obj = 2; a.mode_con = -1; a.f = fv; a.g = g; a.jac_layout = NTGB_JAC_NONE; a.stream = st;
     for (int it = 0; it < o.max_iter; it++) {
         if ((rc = ntgb_eval(pb, &a))) return rc;
-        CUDA_TRY(launch(k_solve_dir, grid, 128, st, P, nC, nr, pb->red.N, fv, g, o.gtol, y, yp, grp, H, d, dC, phi0,
+        CUDA_TRY(launch(k_solve_dir, grid, 128, st, P, nC, nr, al.N, fv, g, o.gtol, y, yp, grp, H, d, dC, phi0,
                         dphi0, state, fails, count));
-        if ((it + 1) % o.check_every == 0) {
-            int done = 0;
-            CUDA_TRY(cudaMemcpyAsync(&done, count, sizeof(int), cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(cudaStreamSynchronize(st));
-            if (done >= P) break;
+        if ((it + 1) % o.check_every == 0 && (rc = all_finished(count, P, st)) != 0) {
+            if (rc < 0) return rc;
+            break;
         }
         if ((rc = ntgb_linesearch(pb, P, C, dC, kNalpha, alphas, 0.0, o.c1, phi0, dphi0, ab, pbest, nullptr, st)))
             return rc;
-        CUDA_TRY(launch(k_solve_update, grid, 128, st, P, nC, nr, pb->red.N, Cpart, Cstride, phi0, ab, pbest, d, y, H,
+        CUDA_TRY(launch(k_solve_update, grid, 128, st, P, nC, nr, al.N, Cpart, Cstride, phi0, ab, pbest, d, y, H,
                         C, state, its, fails, count));
     }
     if (f) {
@@ -2357,61 +2497,27 @@ int ntgb_solve_nlp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
         return fail(NTGB_ELIMIT, "ntgb_solve_nlp: %d free directions after eliminating the linear equalities (limit %d)",
                     al.nr, kSolveMaxNr);
     const int nr = al.nr, m = al.m, n_li = al.n_li;
-    constexpr int kN1 = 4, kN2 = 12, kNalpha = kN1 + kN2;
-    const size_t Pz = (size_t)P, Q = Pz * kNalpha;
+    if ((rc = TwoStage::check_size(P))) return rc;
+    const size_t Pz = (size_t)P;
     const size_t mz = (size_t)std::max(m, 1), ncz = (size_t)std::max(ncnln, 1), nlz = (size_t)std::max(nclin, 1);
-    if (Pz > al.cap) {
-        CUDA_TRY(cudaStreamSynchronize(st));
-        if (al.blob) cudaFree(al.blob);
-        if (al.tblob) cudaFree(al.tblob);
-        if (al.iblob) cudaFree(al.iblob);
-        al.blob = al.tblob = nullptr; al.iblob = nullptr; al.cap = 0;
-        const size_t nd = Pz * ((size_t)4 * nr + (size_t)nr * nr + 3 * (size_t)nC + 2 * mz + ncz + ncz * dm.sorder + nlz + 10) + kNalpha;
-        const size_t nt = Q * ((size_t)nC + ncz + nlz + 4);
-        CUDA_TRY(cudaMalloc((void **)&al.blob, nd * sizeof(double)));
-        CUDA_TRY(cudaMalloc((void **)&al.tblob, nt * sizeof(double)));
-        CUDA_TRY(cudaMalloc((void **)&al.iblob, ((size_t)5 * P + 2) * sizeof(int)));
-        al.cap = Pz;
-    }
-    const size_t cap = al.cap;
-    double *q = al.blob;
-    double *y = q;      q += cap * nr;
-    double *yp = q;     q += cap * nr;
-    double *grp = q;    q += cap * nr;
-    double *d = q;      q += cap * nr;
-    double *H = q;      q += cap * nr * nr;
-    double *dC = q;     q += cap * nC;
-    double *g = q;      q += cap * nC;
-    double *gA = q;     q += cap * nC;
-    double *lam = q;    q += cap * mz;
-    double *mu = q;     q += cap * mz;
-    double *cc = q;     q += cap * ncz;
-    double *J = q;      q += cap * ncz * dm.sorder;
-    double *lin = q;    q += cap * nlz;
-    double *fv = q;     q += cap;
-    double *LA = q;     q += cap;
-    double *viol = q;   q += cap;
-    double *violp = q;  q += cap;
-    double *rho = q;    q += cap;
-    double *phi0 = q;   q += cap;
-    double *dphi0 = q;  q += cap;
-    double *ab = q;     q += cap;
-    double *pbest = q;  q += cap;
-    double *alphas = q;
-    const size_t capq = cap * kNalpha;
-    double *t = al.tblob;
-    double *Ct = t;     t += capq * nC;
-    double *ct = t;     t += capq * ncz;
-    double *lint = t;   t += capq * nlz;
-    double *ft = t;     t += capq;
-    double *res = t;    /* [Q][2] */
-    int *state = al.iblob, *its = state + cap, *fails = its + cap, *fin = fails + cap, *idx = fin + cap, *count = idx + cap,
-        *nidx = count + 1;
+    double *y, *yp, *grp, *d, *H, *dC, *g, *gA, *lam, *mu, *cc, *J, *lin, *fv, *LA, *viol, *violp, *rho, *phi0, *dphi0;
+    int *state, *its, *fails, *fin, *count;
+    TwoStage ts;
+    if ((rc = scratch_carve(pb->scratch.nlp, st, [&](Carve &c) {
+             c.take(Pz * nr, y, yp, grp, d);
+             c.take(Pz * nr * nr, H);
+             c.take(Pz * nC, dC, g, gA);
+             c.take(Pz * mz, lam, mu);
+             c.take(Pz * ncz, cc);
+             c.take(Pz * ncz * dm.sorder, J);
+             c.take(Pz * nlz, lin);
+             c.take(Pz, fv, LA, viol, violp, rho, phi0, dphi0, state, its, fails, fin);
+             c.take(1, count);
+             ts.take(c, Pz, dm);
+         })))
+        return rc;
 
-    double ha[kNalpha];
-    for (int a = 0; a < kNalpha; a++) ha[a] = std::ldexp(1.0, -a);
-    CUDA_TRY(cudaMemcpyAsync(alphas, ha, sizeof ha, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemsetAsync(res, 0, sizeof(double) * 2 * Q, st));
+    if ((rc = ts.start(P, st))) return rc;
     const unsigned grid = (unsigned)((P + 127) / 128);
     CUDA_TRY(launch(k_solve_init, grid, 128, st, P, nC, nr, al.N, al.Cpart, 0, C, y, H, state, its, fails));
     CUDA_TRY(launch(k_alm_prep, grid, 128, st, P, m, o.rho0, lam, rho, violp, fin));
@@ -2421,11 +2527,13 @@ int ntgb_solve_nlp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
     memset(&ea, 0, sizeof ea);
     ea.P = P; ea.C = C; ea.mode_obj = 2; ea.mode_con = ncnln > 0 ? 2 : -1; ea.f = fv; ea.g = g; ea.c = cc; ea.J = J;
     ea.jac_layout = ncnln > 0 ? NTGB_JAC_BAND : NTGB_JAC_NONE; ea.stream = st;
-    ntgb_eval_args et;
-    memset(&et, 0, sizeof et);
-    et.P = (int)Q; et.C = Ct; et.mode_obj = 0; et.mode_con = ncnln > 0 ? 0 : -1; et.f = ft; et.c = ct;
-    et.jac_layout = NTGB_JAC_NONE; et.stream = st;
-    if (Q > 0x7fffffffull) return fail(NTGB_EINVAL, "P*nalpha too large");
+    /* the search's merit: the augmented Lagrangian at the trial points */
+    auto merit = [&](int n, int nalpha, const int *pidx) -> int {
+        CUDA_TRY(launch(k_alm_mu, (unsigned)(((long long)n * 32 + 127) / 128), 128, st, n, nalpha, ncnln, nclin, n_li,
+                        al.li_idx, al.hl, al.hu, lam, rho, ts.ft, ts.ct, ts.lint, (double *)nullptr, ts.res,
+                        (double *)nullptr, 2, pidx));
+        return 0;
+    };
 
     auto assemble = [&]() -> int { /* f, g, c, J, lin at C -> mu, L_A, violation, grad L_A */
         int r2;
@@ -2445,54 +2553,23 @@ int ntgb_solve_nlp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
             if ((rc = assemble())) return rc;
             CUDA_TRY(launch(k_solve_dir, grid, 128, st, P, nC, nr, al.N, LA, gA, o.gtol, y, yp, grp, H, d, dC, phi0, dphi0,
                             state, fails, count));
-            if ((it + 1) % o.check_every == 0) {
-                int done = 0;
-                CUDA_TRY(cudaMemcpyAsync(&done, count, sizeof(int), cudaMemcpyDeviceToHost, st));
-                CUDA_TRY(cudaStreamSynchronize(st));
-                if (done >= P) break;
+            if ((it + 1) % o.check_every == 0 && (rc = all_finished(count, P, st)) != 0) {
+                if (rc < 0) return rc;
+                break;
             }
-            /* Armijo line search on the augmented Lagrangian, two stages: the steps 1 .. 1/8 for every
-             * problem in one evaluation; the steps 2^-4 .. 2^-15 only for the problems that found
-             * no Armijo step among them (compacted by index), in a second one */
-            {
-                const long long totc = (long long)P * kN1 * nC;
-                CUDA_TRY(launch(k_ls_trial, (unsigned)((totc + 255) / 256), 256, st, C, dC, alphas, P, kN1, nC, Ct));
-                et.P = P * kN1;
-                if ((rc = ntgb_eval(pb, &et))) return rc;
-                if (n_li > 0 && (rc = ntgb_eval_linear(pb, et.P, Ct, lint, nullptr, st))) return rc;
-                const unsigned gq = (unsigned)(((long long)et.P * 32 + 127) / 128);
-                CUDA_TRY(launch(k_alm_mu, gq, 128, st, et.P, kN1, ncnln, nclin, n_li, al.li_idx, al.hl, al.hu, lam, rho, ft, ct,
-                                lint, (double *)nullptr, res, (double *)nullptr, 2, (const int *)nullptr));
-                CUDA_TRY(cudaMemsetAsync(nidx, 0, sizeof(int), st));
-                CUDA_TRY(launch(k_alm_pick1, grid, 128, st, res, alphas, P, kN1, o.c1, phi0, dphi0, state, ab, pbest, idx, nidx));
-                int n2 = 0;
-                CUDA_TRY(cudaMemcpyAsync(&n2, nidx, sizeof(int), cudaMemcpyDeviceToHost, st));
-                CUDA_TRY(cudaStreamSynchronize(st));
-                if (n2 > 0) {
-                    const long long tot2 = (long long)n2 * kN2 * nC;
-                    CUDA_TRY(launch(k_ls_trial_idx, (unsigned)((tot2 + 255) / 256), 256, st, C, dC, alphas + kN1, idx, n2, kN2, nC, Ct));
-                    et.P = n2 * kN2;
-                    if ((rc = ntgb_eval(pb, &et))) return rc;
-                    if (n_li > 0 && (rc = ntgb_eval_linear(pb, et.P, Ct, lint, nullptr, st))) return rc;
-                    const unsigned g2 = (unsigned)(((long long)et.P * 32 + 127) / 128);
-                    CUDA_TRY(launch(k_alm_mu, g2, 128, st, et.P, kN2, ncnln, nclin, n_li, al.li_idx, al.hl, al.hu, lam, rho, ft,
-                                    ct, lint, (double *)nullptr, res, (double *)nullptr, 2, idx));
-                    CUDA_TRY(launch(k_alm_pick2, (unsigned)((n2 + 127) / 128), 128, st, res, alphas + kN1, idx, n2, kN2, o.c1, phi0,
-                                    dphi0, ab, pbest));
-                }
-            }
-            CUDA_TRY(launch(k_solve_update, grid, 128, st, P, nC, nr, al.N, al.Cpart, 0, phi0, ab, pbest, d, y, H, C, state, its,
-                            fails, count));
+            if ((rc = two_stage_search(pb, P, C, dC, o.c1, phi0, dphi0, state, ts, st, merit))) return rc;
+            CUDA_TRY(launch(k_solve_update, grid, 128, st, P, nC, nr, al.N, al.Cpart, 0, phi0, ts.ab, ts.pbest, d, y, H, C,
+                            state, its, fails, count));
         }
         /* round finished: fresh multipliers at the point reached, then the outer update */
         if ((rc = assemble())) return rc;
         CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
         CUDA_TRY(launch(k_alm_outer, grid, 128, st, P, m, nr, mu, lam, rho, viol, violp, o.ctol, o.rho_mul, o.rho_max,
                         outer + 1 == o.max_outer ? 1 : 0, H, state, fails, fin, count));
-        int done = 0;
-        CUDA_TRY(cudaMemcpyAsync(&done, count, sizeof(int), cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        if (done >= P) break;
+        if ((rc = all_finished(count, P, st)) != 0) {
+            if (rc < 0) return rc;
+            break;
+        }
     }
     if (f) CUDA_TRY(cudaMemcpyAsync(f, fv, sizeof(double) * Pz, cudaMemcpyDeviceToDevice, st));
     if (viol_out) CUDA_TRY(cudaMemcpyAsync(viol_out, viol, sizeof(double) * Pz, cudaMemcpyDeviceToDevice, st));
@@ -2525,8 +2602,7 @@ int ntgb_sqp_warm_doubles(ntgb_problem *pb, size_t *n)
     DeviceGuard dg(pb->device);
     if (!dg.ok) return fail(NTGB_ECUDA, "cannot select device %d", pb->device);
     int rc;
-    if ((rc = alm_prepare(pb))) return rc;
-    if (pb->alm.nr < 1) return fail(NTGB_EINVAL, "ntgb_sqp_warm_doubles: the linear equalities leave no free direction");
+    if ((rc = sqp_prepare(pb, "ntgb_sqp_warm_doubles"))) return rc;
     *n = ntgb::warm_doubles(pb->alm.nr);
     return 0;
 }
@@ -2567,11 +2643,10 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
     cudaStream_t st = (cudaStream_t)stream;
     const int nC = dm.nC, nclin = dm.nclin, ncnln = dm.ncnln;
     int rc;
-    if ((rc = alm_prepare(pb))) return rc;
-    auto &al = pb->alm;
-    auto &sq = pb->sqp;
+    if ((rc = sqp_prepare(pb, "ntgb_solve_sqp"))) return rc;
+    const auto &al = pb->alm;
+    const auto &sq = pb->sqp;
     const int nr = al.nr, m = al.m, n_li = al.n_li;
-    if (nr < 1) return fail(NTGB_EINVAL, "ntgb_solve_sqp: the linear equalities leave no free direction");
     /* one CTA per problem: 32 threads up to 31 reduced variables, 64 beyond */
     const int nt = nr < 32 ? 32 : 64;
     const size_t smem = sqp::sqp_smem_doubles(nr, m, nt) * sizeof(double) + sqp::sqp_smem_ints(nr, m, nt) * sizeof(int);
@@ -2580,113 +2655,27 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
                     "ntgb_solve_sqp: %d reduced variables x %d rows need %zu bytes of shared memory per problem (limit %d): "
                     "the dense reduced-space QP is meant for short horizons",
                     nr, m, smem, pb->max_smem_optin);
-    if (!sq.ready) {
-        /* reduced gradients of the linear inequality rows, and W = (Ae Ae')^-1 Ae for the multipliers
-         * of the eliminated equality rows */
-        std::vector<double> ArN((size_t)std::max(n_li, 1) * nr, 0.0);
-        for (int i = 0; i < n_li; i++)
-            for (int k = 0; k < nr; k++) {
-                double a = 0.0;
-                for (int e = 0; e < nC; e++) a += pb->A[al.li[i] + (size_t)e * nclin] * al.hN[(size_t)k * nC + e];
-                ArN[(size_t)i * nr + k] = a;
-            }
-        if ((rc = dev_upload(pb, &sq.ArN, ArN.data(), ArN.size()))) return rc;
-        const int me = (int)al.eq.size();
-        std::vector<double> W((size_t)std::max(me, 1) * nC, 0.0), G((size_t)std::max(me, 1) * std::max(me, 1), 0.0);
-        for (int r = 0; r < me; r++)
-            for (int s = 0; s < me; s++) {
-                double a = 0.0;
-                for (int e = 0; e < nC; e++) a += pb->A[al.eq[r] + (size_t)e * nclin] * pb->A[al.eq[s] + (size_t)e * nclin];
-                G[(size_t)r * me + s] = a;
-            }
-        /* Gauss-Jordan with partial pivoting on [G | Ae]; dependent rows get zero multipliers */
-        for (int r = 0; r < me; r++)
-            for (int e = 0; e < nC; e++) W[(size_t)r * nC + e] = pb->A[al.eq[r] + (size_t)e * nclin];
-        double gmax = 0.0;
-        for (int r = 0; r < me; r++) gmax = std::max(gmax, std::fabs(G[(size_t)r * me + r]));
-        std::vector<char> dead(std::max(me, 1), 0);
-        for (int k = 0; k < me; k++) {
-            int piv = -1;
-            double best = 1e-12 * std::max(gmax, 1e-300);
-            for (int r = k; r < me; r++)
-                if (std::fabs(G[(size_t)r * me + k]) > best) { best = std::fabs(G[(size_t)r * me + k]); piv = r; }
-            if (piv < 0) { dead[k] = 1; continue; }
-            if (piv != k) {
-                for (int s = 0; s < me; s++) std::swap(G[(size_t)k * me + s], G[(size_t)piv * me + s]);
-                for (int e = 0; e < nC; e++) std::swap(W[(size_t)k * nC + e], W[(size_t)piv * nC + e]);
-            }
-            const double d = G[(size_t)k * me + k];
-            for (int s = 0; s < me; s++) G[(size_t)k * me + s] /= d;
-            for (int e = 0; e < nC; e++) W[(size_t)k * nC + e] /= d;
-            for (int r = 0; r < me; r++) {
-                if (r == k) continue;
-                const double t = G[(size_t)r * me + k];
-                if (t == 0.0) continue;
-                for (int s = 0; s < me; s++) G[(size_t)r * me + s] -= t * G[(size_t)k * me + s];
-                for (int e = 0; e < nC; e++) W[(size_t)r * nC + e] -= t * W[(size_t)k * nC + e];
-            }
-        }
-        for (int k = 0; k < me; k++)
-            if (dead[k])
-                for (int e = 0; e < nC; e++) W[(size_t)k * nC + e] = 0.0;
-        if ((rc = dev_upload(pb, &sq.W, W.data(), W.size()))) return rc;
-        std::vector<int> eqi = al.eq;
-        if (eqi.empty()) eqi.push_back(0);
-        if ((rc = dev_upload(pb, &sq.eq_idx, eqi.data(), eqi.size()))) return rc;
-        sq.me = me;
-        sq.ready = true;
-    }
-    constexpr int kN1 = 4, kN2 = 12, kNalpha = kN1 + kN2;
-    const size_t Pz = (size_t)P, Q = Pz * kNalpha;
-    if (Q > 0x7fffffffull) return fail(NTGB_EINVAL, "P*nalpha too large");
+    if ((rc = TwoStage::check_size(P))) return rc;
+    const size_t Pz = (size_t)P;
     const size_t mz = (size_t)std::max(m, 1), ncz = (size_t)std::max(ncnln, 1), nlz = (size_t)std::max(nclin, 1);
-    if (Pz > sq.cap) {
-        CUDA_TRY(cudaStreamSynchronize(st));
-        if (sq.blob) cudaFree(sq.blob);
-        if (sq.tblob) cudaFree(sq.tblob);
-        if (sq.iblob) cudaFree(sq.iblob);
-        sq.blob = sq.tblob = nullptr; sq.iblob = nullptr; sq.cap = 0;
-        const size_t nd = Pz * ((size_t)5 * nr + (size_t)nr * nr + 3 * (size_t)nC + 2 * mz + ncz + ncz * dm.sorder + nlz + 8 + 8) + kNalpha;
-        const size_t nt2 = Q * ((size_t)nC + ncz + nlz + 4);
-        CUDA_TRY(cudaMalloc((void **)&sq.blob, nd * sizeof(double)));
-        CUDA_TRY(cudaMalloc((void **)&sq.tblob, nt2 * sizeof(double)));
-        CUDA_TRY(cudaMalloc((void **)&sq.iblob, (Pz * (12 + mz) + 2) * sizeof(int)));
-        sq.cap = Pz;
-    }
-    const size_t cap = sq.cap;
-    double *q = sq.blob;
     SqpArrays S;
-    S.y = q;      q += cap * nr;
-    S.sprev = q;  q += cap * nr;
-    S.grLold = q; q += cap * nr;
-    S.grold = q;  q += cap * nr;
-    S.d = q;      q += cap * nr;
-    S.B = q;      q += cap * nr * nr;
-    double *dC = q;    q += cap * nC;
-    double *g = q;     q += cap * nC;
-    double *gL = q;    q += cap * nC;
-    S.lam = q;    q += cap * mz;
-    double *mu = q;    q += cap * mz;
-    double *cc = q;    q += cap * ncz;
-    double *J = q;     q += cap * ncz * dm.sorder;
-    double *lin = q;   q += cap * nlz;
-    S.scal = q;   q += cap * 8;
-    double *fv = q;    q += cap;
-    double *phi0 = q;  q += cap;
-    double *dphi0 = q; q += cap;
-    double *ab = q;    q += cap;
-    double *pbest = q; q += cap;
-    double *alphas = q;
-    const size_t capq = cap * kNalpha;
-    double *t = sq.tblob;
-    double *Ct = t;    t += capq * nC;
-    double *ct = t;    t += capq * ncz;
-    double *lint = t;  t += capq * nlz;
-    double *ft = t;    t += capq;
-    double *res = t;
-    int *state = sq.iblob, *its = state + cap, *idx = its + cap, *count = idx + cap, *nidx = count + 1;
-    S.flag = nidx + 1;
-    S.istate = S.flag + cap * 8;
+    double *dC, *g, *gL, *mu, *cc, *J, *lin, *fv, *phi0, *dphi0;
+    int *state, *its, *count;
+    TwoStage ts;
+    if ((rc = scratch_carve(pb->scratch.sqp, st, [&](Carve &c) {
+             c.take(Pz * nr, S.y, S.sprev, S.grLold, S.grold, S.d);
+             c.take(Pz * nr * nr, S.B);
+             c.take(Pz * nC, dC, g, gL);
+             c.take(Pz * mz, S.lam, mu, S.istate);
+             c.take(Pz * ncz, cc);
+             c.take(Pz * ncz * dm.sorder, J);
+             c.take(Pz * nlz, lin);
+             c.take(Pz * 8, S.scal, S.flag);
+             c.take(Pz, fv, phi0, dphi0, state, its);
+             c.take(1, count);
+             ts.take(c, Pz, dm);
+         })))
+        return rc;
 
     SqpDesc D;
     D.nC = nC; D.nr = nr; D.m = m; D.n_li = n_li; D.nclin = nclin; D.ncnln = ncnln;
@@ -2695,10 +2684,7 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
     D.gtol = o.gtol; D.ctol = o.ctol; D.rho_pen = o.rho_pen;
     const double *Cpart = al.Cpart;
 
-    double ha[kNalpha];
-    for (int a = 0; a < kNalpha; a++) ha[a] = std::ldexp(1.0, -a);
-    CUDA_TRY(cudaMemcpyAsync(alphas, ha, sizeof ha, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(cudaMemsetAsync(res, 0, sizeof(double) * 2 * Q, st));
+    if ((rc = ts.start(P, st))) return rc;
     CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
     if (lowerb) {
         BoundsDesc B{bounds_layout(pb), nC, n_li, m, sq.me, al.li_idx, sq.eq_idx, al.M, al.Ae};
@@ -2717,10 +2703,12 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
     memset(&ea, 0, sizeof ea);
     ea.P = P; ea.C = C; ea.mode_obj = 2; ea.mode_con = ncnln > 0 ? 2 : -1; ea.f = fv; ea.g = g; ea.c = cc; ea.J = J;
     ea.jac_layout = ncnln > 0 ? NTGB_JAC_BAND : NTGB_JAC_NONE; ea.stream = st;
-    ntgb_eval_args et;
-    memset(&et, 0, sizeof et);
-    et.P = (int)Q; et.C = Ct; et.mode_obj = 0; et.mode_con = ncnln > 0 ? 0 : -1; et.f = ft; et.c = ct;
-    et.jac_layout = NTGB_JAC_NONE; et.stream = st;
+    /* the search's merit: the L1 merit at the trial points */
+    auto merit = [&](int n, int nalpha, const int *pidx) -> int {
+        CUDA_TRY(launch(k_sqp_merit, (unsigned)(((long long)n * 32 + 127) / 128), 128, st, n, nalpha, D, S.scal, ts.ft,
+                        ts.ct, ts.lint, ts.res, pidx));
+        return 0;
+    };
 
     auto direction = [&]() -> int { /* f, g, c, J, lin at C -> QP -> d, dC, merit and slope; finished problems counted */
         int r2;
@@ -2739,38 +2727,12 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
     for (int it = 0; it <= o.max_iter; it++) {
         if ((rc = direction())) return rc;
         if (it == o.max_iter) break; /* the last pass only evaluates and tests convergence at the final point */
-        if ((it + 1) % o.check_every == 0) {
-            int done = 0;
-            CUDA_TRY(cudaMemcpyAsync(&done, count, sizeof(int), cudaMemcpyDeviceToHost, st));
-            CUDA_TRY(cudaStreamSynchronize(st));
-            if (done >= P) break;
+        if ((it + 1) % o.check_every == 0 && (rc = all_finished(count, P, st)) != 0) {
+            if (rc < 0) return rc;
+            break;
         }
-        /* Armijo search on the L1 merit, two stages like ntgb_solve_nlp: steps 1 .. 1/8 for every
-         * problem, 2^-4 .. 2^-15 only for the compacted list that found none */
-        const long long totc = (long long)P * kN1 * nC;
-        CUDA_TRY(launch(k_ls_trial, (unsigned)((totc + 255) / 256), 256, st, C, dC, alphas, P, kN1, nC, Ct));
-        et.P = P * kN1;
-        if ((rc = ntgb_eval(pb, &et))) return rc;
-        if (n_li > 0 && (rc = ntgb_eval_linear(pb, et.P, Ct, lint, nullptr, st))) return rc;
-        CUDA_TRY(launch(k_sqp_merit, (unsigned)(((long long)et.P * 32 + 127) / 128), 128, st, et.P, kN1, D, S.scal, ft, ct, lint, res,
-                        (const int *)nullptr));
-        CUDA_TRY(cudaMemsetAsync(nidx, 0, sizeof(int), st));
-        CUDA_TRY(launch(k_alm_pick1, grid, 128, st, res, alphas, P, kN1, o.c1, phi0, dphi0, state, ab, pbest, idx, nidx));
-        int n2 = 0;
-        CUDA_TRY(cudaMemcpyAsync(&n2, nidx, sizeof(int), cudaMemcpyDeviceToHost, st));
-        CUDA_TRY(cudaStreamSynchronize(st));
-        if (n2 > 0) {
-            const long long tot2 = (long long)n2 * kN2 * nC;
-            CUDA_TRY(launch(k_ls_trial_idx, (unsigned)((tot2 + 255) / 256), 256, st, C, dC, alphas + kN1, idx, n2, kN2, nC, Ct));
-            et.P = n2 * kN2;
-            if ((rc = ntgb_eval(pb, &et))) return rc;
-            if (n_li > 0 && (rc = ntgb_eval_linear(pb, et.P, Ct, lint, nullptr, st))) return rc;
-            CUDA_TRY(launch(k_sqp_merit, (unsigned)(((long long)et.P * 32 + 127) / 128), 128, st, et.P, kN2, D, S.scal, ft, ct, lint,
-                            res, (const int *)idx));
-            CUDA_TRY(launch(k_alm_pick2, (unsigned)((n2 + 127) / 128), 128, st, res, alphas + kN1, idx, n2, kN2, o.c1, phi0, dphi0,
-                            ab, pbest));
-        }
-        CUDA_TRY(launch(k_sqp_update, grid, 128, st, P, D, S, Cpart, phi0, ab, pbest, C, state, its, count));
+        if ((rc = two_stage_search(pb, P, C, dC, o.c1, phi0, dphi0, state, ts, st, merit))) return rc;
+        CUDA_TRY(launch(k_sqp_update, grid, 128, st, P, D, S, Cpart, phi0, ts.ab, ts.pbest, C, state, its, count));
     }
     if (warm)
         CUDA_TRY(launch(k_sqp_warm_store, (unsigned)(((long long)P * 32 + 127) / 128), 128, st, P, S, wk, (const int *)state,
