@@ -415,6 +415,50 @@ int  ntgb_solve_sqp_warm(ntgb_problem *pb, int P, double *C, const double *lower
                          double *warm, double *f, double *viol, int *iters, int *status, double *lambda,
                          int *istate, const ntgb_sqp_opts *opts, void *stream);
 
+/*
+ * Stream-ordered solvers, for a fixed small number of iterations per control step (real-time iteration):
+ * the call queues its work on `stream` and returns.  It synchronizes nothing, copies nothing to or from
+ * the host, allocates nothing and sets no kernel attribute, so a whole control step can be recorded in
+ * a CUDA graph (cudaStreamBeginCapture ... cudaStreamEndCapture) and replayed, or queued behind and
+ * beside other GPU work.  Full solves stay with the synchronous entry points.
+ *
+ * ntgb_solve_eq_reserve / ntgb_solve_sqp_reserve: the one-time host work (the reduced form, the step
+ * table and, for SQP, the QP kernel's shared-memory limit) and a work space for up to P_max problems.
+ * They refuse what ntgb_solve_eq / ntgb_solve_sqp refuse, with the same code and message (nonlinear or
+ * inequality rows for eq, too many free directions, QP work space above the shared memory: NTGB_ELIMIT,
+ * no free direction).  They may synchronize the device and allocate.  Reserving again with a larger
+ * P_max replaces the work space: graphs captured before must be captured again.  The work space
+ * belongs to the async entry point alone, apart from what the synchronous calls use, so no synchronous
+ * call on the same ntgb_problem -- one that grows its own scratch included -- invalidates a graph.
+ * A synchronous ntgb_solve_sqp* call sets the QP kernel's shared-memory limit to what its own problem
+ * needs: after one on ANOTHER ntgb_problem, call ntgb_solve_sqp_reserve again before the next async
+ * call or replay.
+ *
+ * ntgb_solve_eq_async / ntgb_solve_sqp_async: arguments and outputs as in the synchronous entry points.
+ * lowerb and upperb are both NULL (the setup's bounds) or both set (per-problem bounds, as in
+ * ntgb_solve_*_bounds); warm is NULL (no state carried) or a [P][ntgb_sqp_warm_doubles] array (as in
+ * ntgb_solve_sqp_warm); lambda, istate and the other outputs may be NULL.  The call runs EXACTLY
+ * opts->max_iter iterations (default 100 for SQP, 200 for eq); check_every is ignored.  A finished
+ * problem is inert in every solver kernel, so each output -- C, f, viol, iters, status, lambda, istate,
+ * the warm rows, and problems with rejected bounds left untouched -- is bit-identical to the synchronous
+ * call with the same arguments.  That call stops once every problem has finished; an async call pays for
+ * all max_iter iterations even then.  The SQP line search evaluates the 16 steps 1 .. 2^-15 of every
+ * problem in one batch (the synchronous one evaluates 4 steps, then 12 more only for the problems that
+ * need them), and picks the same step.
+ *
+ * P above the reserved P_max, or no reserve yet, is NTGB_EINVAL before any CUDA call; so is exactly
+ * one of lowerb / upperb NULL.  P == 0 returns 0.  An ntgb_problem runs one async call per solver at a
+ * time: async calls on different streams must be ordered by the caller (an event), since they share
+ * the work space.
+ */
+int  ntgb_solve_eq_reserve(ntgb_problem *pb, int P_max);
+int  ntgb_solve_eq_async(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb,
+                         double *f, int *iters, int *status, const ntgb_solve_opts *opts, void *stream);
+int  ntgb_solve_sqp_reserve(ntgb_problem *pb, int P_max);
+int  ntgb_solve_sqp_async(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb,
+                          double *warm, double *f, double *viol, int *iters, int *status, double *lambda,
+                          int *istate, const ntgb_sqp_opts *opts, void *stream);
+
 /* Gathered result tables for the fused multi-GPU gather (ntgb_eval_args.peer_result): alloc creates
  * this rank's table (rows x 2 doubles, zeroed) and the 64-byte CUDA IPC handle the other ranks
  * need; open maps another rank's table into this process (peer access over NVLink is enabled on

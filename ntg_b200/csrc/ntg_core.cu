@@ -83,6 +83,13 @@ struct Scratch {
     size_t bytes = 0;
 };
 
+/* work space of one stream-ordered solver entry point (ntgb_solve_*_async), sized by its reserve call for up to
+ * P problems */
+struct AsyncWork {
+    Scratch s;
+    int P = 0;
+};
+
 } /* namespace */
 
 struct ntgb_problem {
@@ -160,6 +167,12 @@ struct ntgb_problem {
     /* per-call device arrays, kept between calls: one scratch per driver, so that no call's arrays alias
      * another solver's (ntgb_solve_eq, ntgb_solve_nlp, ntgb_solve_sqp, ntgb_linesearch, per-problem bounds) */
     struct { Scratch eq, nlp, sqp, ls, bnd; } scratch;
+    /* ntgb_solve_eq_async / ntgb_solve_sqp_async: their own work spaces, apart from `scratch`, so that no
+     * synchronous call moves an array that a captured graph uses; halving = the step table 2^-a, a < 16 */
+    struct {
+        AsyncWork eq, sqp;
+        double *halving = nullptr;
+    } async;
 };
 
 namespace {
@@ -217,13 +230,16 @@ struct Carve {
 
 /* layout(Carve &) takes every array of a call once, in order: it runs once to size s and once to hand out the
  * pointers.  s grows when the call needs more and never shrinks; the old buffer may still be in use by work
- * queued on st, so st is synchronized before it is freed. */
+ * queued on st, so st is synchronized before it is freed.  grow == false (a reserved work space): a layout
+ * larger than s is an error. */
 template <class Layout>
-int scratch_carve(Scratch &s, cudaStream_t st, Layout layout)
+int scratch_carve(Scratch &s, cudaStream_t st, Layout layout, bool grow = true)
 {
     Carve size{nullptr};
     layout(size);
     if (size.off > s.bytes) {
+        if (!grow)
+            return fail(NTGB_EINVAL, "internal error: a reserved work space of %zu bytes cannot hold %zu", s.bytes, size.off);
         CUDA_TRY(cudaStreamSynchronize(st));
         cudaFree(s.p);
         s.p = nullptr;
@@ -1355,23 +1371,25 @@ __global__ void k_bounds_prep(int P, BoundsDesc B, const double *lowerb, const d
     }
 }
 
-/* per-problem bounds: size the scratch (grows with P, never per iteration) and run k_bounds_prep;
- * returns problem p's Cpart / hl / hu at Cpart + p*nC, hl + p*m, hu + p*m */
-int bounds_prepare(ntgb_problem *pb, int P, const double *lowerb, const double *upperb, const BoundsDesc &B,
-                   cudaStream_t st, int *state, int *iters, int *count, double **Cpart, double **hl, double **hu)
+/* what k_bounds_prep writes: problem p's Cpart / hl / hu at Cpart + p*nC, hl + p*m, hu + p*m */
+struct BoundsArrays {
+    double *Cpart, *hl, *hu, *be;
+
+    void take(Carve &c, size_t P, const BoundsDesc &B)
+    {
+        c.take(P * B.nC, Cpart);
+        c.take(P * B.m, hl, hu);
+        c.take(P * B.me, be);
+    }
+};
+
+/* per-problem bounds, once per call: k_bounds_prep into the caller's arrays */
+int bounds_prepare(int P, const double *lowerb, const double *upperb, const BoundsDesc &B, const BoundsArrays &ba,
+                   cudaStream_t st, int *state, int *iters, int *count)
 {
-    const size_t Pz = (size_t)P;
-    double *be;
-    int rc;
-    if ((rc = scratch_carve(pb->scratch.bnd, st, [&](Carve &c) {
-             c.take(Pz * B.nC, *Cpart);
-             c.take(Pz * B.m, *hl, *hu);
-             c.take(Pz * B.me, be);
-         })))
-        return rc;
     const long long threads = (long long)P * 32;
-    CUDA_TRY(launch(k_bounds_prep, (unsigned)((threads + 127) / 128), 128, st, P, B, lowerb, upperb, *hl, *hu, be, *Cpart,
-                    state, iters, count));
+    CUDA_TRY(launch(k_bounds_prep, (unsigned)((threads + 127) / 128), 128, st, P, B, lowerb, upperb, ba.hl, ba.hu, ba.be,
+                    ba.Cpart, state, iters, count));
     return 0;
 }
 
@@ -1409,21 +1427,25 @@ struct TwoStage {
         c.take(P, idx, ab, pbest);
         c.take(1, nidx);
     }
-    /* once per call */
-    int start(int P, cudaStream_t st) const
+    /* once per call; upload == false: alphas already holds the step table */
+    int start(int P, cudaStream_t st, bool upload = true) const
     {
         int rc;
-        if ((rc = upload_halving(alphas, kNalpha, st))) return rc;
+        if (upload && (rc = upload_halving(alphas, kNalpha, st))) return rc;
         CUDA_TRY(cudaMemsetAsync(res, 0, sizeof(double) * 2 * kNalpha * (size_t)P, st));
         return 0;
     }
 };
 
 /* the search from C along dC for P problems; merit(n, nalpha, pidx) launches the merit kernel on the n trial
- * points just evaluated, trial q belonging to problem pidx[q / nalpha] (pidx == nullptr: q / nalpha) */
+ * points just evaluated, trial q belonging to problem pidx[q / nalpha] (pidx == nullptr: q / nalpha).
+ * single: all kNalpha steps of every problem in one evaluation and one pick, so that the host never waits for
+ * the size of the second stage.  For a running problem k_alm_pick1 over the 16 steps chooses what the two
+ * stages choose: the first Armijo step in order, else the smallest merit, ties to the earlier step. */
 template <class Merit>
 int two_stage_search(ntgb_problem *pb, int P, const double *C, const double *dC, double c1, const double *phi0,
-                     const double *dphi0, const int *state, const TwoStage &ts, cudaStream_t st, Merit merit)
+                     const double *dphi0, const int *state, const TwoStage &ts, cudaStream_t st, Merit merit,
+                     bool single = false)
 {
     const int nC = pb->dims.nC;
     ntgb_eval_args et;
@@ -1443,10 +1465,12 @@ int two_stage_search(ntgb_problem *pb, int P, const double *C, const double *dC,
         return merit(et.P, nalpha, pidx);
     };
     int rc;
-    if ((rc = trials(P, kN1, ts.alphas, nullptr))) return rc;
+    const int n1 = single ? kNalpha : kN1;
+    if ((rc = trials(P, n1, ts.alphas, nullptr))) return rc;
     CUDA_TRY(cudaMemsetAsync(ts.nidx, 0, sizeof(int), st));
-    CUDA_TRY(launch(k_alm_pick1, (unsigned)((P + 127) / 128), 128, st, ts.res, ts.alphas, P, kN1, c1, phi0, dphi0, state,
+    CUDA_TRY(launch(k_alm_pick1, (unsigned)((P + 127) / 128), 128, st, ts.res, ts.alphas, P, n1, c1, phi0, dphi0, state,
                     ts.ab, ts.pbest, ts.idx, ts.nidx));
+    if (single) return 0;
     int n2 = 0;
     CUDA_TRY(cudaMemcpyAsync(&n2, ts.nidx, sizeof(int), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
@@ -1457,9 +1481,64 @@ int two_stage_search(ntgb_problem *pb, int P, const double *C, const double *dC,
     return 0;
 }
 
-int solve_eq_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f, int *iters,
-                  int *status, const ntgb_solve_opts *opts, void *stream);
-int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *warm,
+/* arrays of ntgb_linesearch for n = P*nalpha trial points */
+struct LsArrays {
+    double *Ct, *res, *lv; /* trial coefficients, result table, linear violation */
+
+    void take(Carve &c, size_t n, int nC)
+    {
+        c.take(n * nC, Ct);
+        c.take(n * 2, res);
+        c.take(n, lv);
+    }
+};
+
+/* body of ntgb_linesearch, on the caller's arrays */
+int linesearch_run(ntgb_problem *pb, int P, const double *C, const double *dC, int nalpha, const double *alpha, double mu,
+                   double c1, const double *phi0, const double *dphi0, double *alpha_best, double *phi_best, double *C_new,
+                   cudaStream_t st, const LsArrays &la)
+{
+    const ntgb_dims &d = pb->dims;
+    const size_t n = (size_t)P * nalpha;
+    const long long total = (long long)n * d.nC;
+    CUDA_TRY(launch(k_ls_trial, (unsigned)((total + 255) / 256), 256, st, C, dC, alpha, P, nalpha, d.nC, la.Ct));
+    ntgb_eval_args a;
+    memset(&a, 0, sizeof a);
+    a.P = (int)n; a.C = la.Ct; a.mode_obj = 0; a.mode_con = d.ncnln > 0 ? 0 : -1;
+    a.result = la.res; a.jac_layout = NTGB_JAC_NONE; a.stream = st;
+    int rc;
+    if ((rc = ntgb_eval(pb, &a))) return rc;
+    const bool lin = d.nclin > 0;
+    if (lin && (rc = ntgb_eval_linear(pb, (int)n, la.Ct, nullptr, la.lv, st))) return rc;
+    CUDA_TRY(launch(k_ls_pick, (unsigned)((P + 127) / 128), 128, st, la.res, lin ? la.lv : nullptr, alpha, P,
+                    nalpha, mu, c1, phi0, dphi0, C, dC, d.nC, alpha_best, phi_best, C_new));
+    return 0;
+}
+
+/* how a solver driver runs: Sync (ntgb_solve_eq*, ntgb_solve_sqp*), Reserve (ntgb_solve_*_reserve: the refusals,
+ * the one-time host work and the work space for P problems; nothing is queued) or Async (ntgb_solve_*_async:
+ * from the reserved work space, exactly max_iter iterations, no synchronization, no host copy, no allocation) */
+enum class Run { Sync, Reserve, Async };
+
+/* the Reserve step of a driver whose Async arrays are carved by layout: the step table once per problem, then
+ * the work space grows to the layout of P problems (never shrinks).  Work queued on any stream may still use
+ * the old work space, so the device is synchronized first. */
+template <class Layout>
+int reserve_work(ntgb_problem *pb, AsyncWork &w, int P, Layout layout)
+{
+    int rc;
+    if (!pb->async.halving && ((rc = dev_alloc(pb, &pb->async.halving, kNalpha)) ||
+                               (rc = upload_halving(pb->async.halving, kNalpha, nullptr))))
+        return rc;
+    CUDA_TRY(cudaDeviceSynchronize());
+    if ((rc = scratch_carve(w.s, nullptr, layout))) return rc;
+    w.P = std::max(w.P, P);
+    return 0;
+}
+
+int solve_eq_impl(ntgb_problem *pb, Run run, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                  int *iters, int *status, const ntgb_solve_opts *opts, void *stream);
+int solve_sqp_impl(ntgb_problem *pb, Run run, int P, double *C, const double *lowerb, const double *upperb, double *warm,
                    double *f, double *viol_out, int *iters, int *status, double *lambda, int *istate,
                    const ntgb_sqp_opts *opts, void *stream);
 
@@ -1511,7 +1590,7 @@ void ntgb_destroy(ntgb_problem *pb)
     for (void *p : pb->allocs) cudaFree(p);
     if (pb->zc.buf) cudaFreeHost(pb->zc.buf);
     auto &s = pb->scratch;
-    for (Scratch *sc : {&s.eq, &s.nlp, &s.sqp, &s.ls, &s.bnd}) cudaFree(sc->p);
+    for (Scratch *sc : {&s.eq, &s.nlp, &s.sqp, &s.ls, &s.bnd, &pb->async.eq.s, &pb->async.sqp.s}) cudaFree(sc->p);
     for (auto &h : pb->hs) {
         double *hsp[] = {h.C, h.f, h.g, h.c, h.J, h.Z, h.result};
         for (double *p : hsp)
@@ -2336,37 +2415,20 @@ int ntgb_linesearch(ntgb_problem *pb, int P, const double *C, const double *dC, 
     if (nalpha < 1 || nalpha > 64) return fail(NTGB_EINVAL, "nalpha = %d outside [1,64]", nalpha);
     DeviceGuard dg(pb->device);
     if (!dg.ok) return fail(NTGB_ECUDA, "cannot select device %d", pb->device);
-    const ntgb_dims &d = pb->dims;
     const size_t n = (size_t)P * nalpha;
     if (n > 0x7fffffffull) return fail(NTGB_EINVAL, "P*nalpha too large");
     cudaStream_t st = (cudaStream_t)stream;
-    double *Ct, *res, *lv; /* trial coefficients, result table, linear violation */
+    LsArrays la;
     int rc;
-    if ((rc = scratch_carve(pb->scratch.ls, st, [&](Carve &c) {
-             c.take(n * d.nC, Ct);
-             c.take(n * 2, res);
-             c.take(n, lv);
-         })))
-        return rc;
-    const long long total = (long long)n * d.nC;
-    CUDA_TRY(launch(k_ls_trial, (unsigned)((total + 255) / 256), 256, st, C, dC, alpha, P, nalpha, d.nC, Ct));
-    ntgb_eval_args a;
-    memset(&a, 0, sizeof a);
-    a.P = (int)n; a.C = Ct; a.mode_obj = 0; a.mode_con = d.ncnln > 0 ? 0 : -1;
-    a.result = res; a.jac_layout = NTGB_JAC_NONE; a.stream = st;
-    if ((rc = ntgb_eval(pb, &a))) return rc;
-    const bool lin = d.nclin > 0;
-    if (lin && (rc = ntgb_eval_linear(pb, (int)n, Ct, nullptr, lv, st))) return rc;
-    CUDA_TRY(launch(k_ls_pick, (unsigned)((P + 127) / 128), 128, st, res, lin ? lv : nullptr, alpha, P,
-                    nalpha, mu, c1, phi0, dphi0, C, dC, d.nC, alpha_best, phi_best, C_new));
-    return 0;
+    if ((rc = scratch_carve(pb->scratch.ls, st, [&](Carve &c) { la.take(c, n, pb->dims.nC); }))) return rc;
+    return linesearch_run(pb, P, C, dC, nalpha, alpha, mu, c1, phi0, dphi0, alpha_best, phi_best, C_new, st, la);
 }
 
 int ntgb_solve_eq(ntgb_problem *pb, int P, double *C, double *f, int *iters, int *status,
                   const ntgb_solve_opts *opts, void *stream)
 {
     if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_eq: null argument");
-    return solve_eq_impl(pb, P, C, nullptr, nullptr, f, iters, status, opts, stream);
+    return solve_eq_impl(pb, Run::Sync, P, C, nullptr, nullptr, f, iters, status, opts, stream);
 }
 
 int ntgb_solve_eq_bounds(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
@@ -2375,18 +2437,39 @@ int ntgb_solve_eq_bounds(ntgb_problem *pb, int P, double *C, const double *lower
     if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_eq_bounds: null argument");
     if (bounds_layout(pb).nb() > 0 && (!lowerb || !upperb))
         return fail(NTGB_EINVAL, "ntgb_solve_eq_bounds: lowerb / upperb is NULL");
-    return solve_eq_impl(pb, P, C, lowerb, upperb, f, iters, status, opts, stream);
+    return solve_eq_impl(pb, Run::Sync, P, C, lowerb, upperb, f, iters, status, opts, stream);
+}
+
+int ntgb_solve_eq_reserve(ntgb_problem *pb, int P_max)
+{
+    if (!pb) return fail(NTGB_EINVAL, "ntgb_solve_eq_reserve: null argument");
+    if (P_max < 1) return fail(NTGB_EINVAL, "ntgb_solve_eq_reserve: P_max = %d", P_max);
+    return solve_eq_impl(pb, Run::Reserve, P_max, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr);
+}
+
+int ntgb_solve_eq_async(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                        int *iters, int *status, const ntgb_solve_opts *opts, void *stream)
+{
+    if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_eq_async: null argument");
+    if ((lowerb == nullptr) != (upperb == nullptr))
+        return fail(NTGB_EINVAL, "ntgb_solve_eq_async: exactly one of lowerb / upperb is NULL");
+    return solve_eq_impl(pb, Run::Async, P, C, lowerb, upperb, f, iters, status, opts, stream);
 }
 
 } /* extern "C" */
 
 namespace {
 
-/* ntgb_solve_eq and ntgb_solve_eq_bounds: lowerb == nullptr = the setup's bounds for every problem */
-int solve_eq_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f, int *iters,
-                  int *status, const ntgb_solve_opts *opts, void *stream)
+/* ntgb_solve_eq, ntgb_solve_eq_bounds and their reserve / async entry points (Run): lowerb == nullptr = the
+ * setup's bounds for every problem */
+int solve_eq_impl(ntgb_problem *pb, Run run, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                  int *iters, int *status, const ntgb_solve_opts *opts, void *stream)
 {
     if (P <= 0) return 0;
+    AsyncWork &aw = pb->async.eq;
+    if (run == Run::Async && P > aw.P)
+        return fail(NTGB_EINVAL, "ntgb_solve_eq_async: P = %d above the %d problems reserved by ntgb_solve_eq_reserve", P,
+                    aw.P);
     const ntgb_dims &dm = pb->dims;
     if (dm.ncnln > 0) return fail(NTGB_EINVAL, "ntgb_solve_eq: problem has %d nonlinear constraints", dm.ncnln);
     for (int i = 0; i < dm.nclin; i++)
@@ -2415,25 +2498,39 @@ int solve_eq_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, cons
     const size_t Pz = (size_t)P;
     double *y, *yp, *grp, *d, *H, *dC, *g, *fv, *phi0, *dphi0, *ab, *pbest, *alphas;
     int *state, *its, *fails, *count;
-    if ((rc = scratch_carve(pb->scratch.eq, st, [&](Carve &c) {
-             c.take(Pz * nr, y, yp, grp, d);
-             c.take(Pz * nr * nr, H);
-             c.take(Pz * nC, dC, g);
-             c.take(Pz, fv, phi0, dphi0, ab, pbest, state, its, fails);
-             c.take(kNalpha, alphas);
-             c.take(1, count);
-         })))
-        return rc;
-    if ((rc = upload_halving(alphas, kNalpha, st))) return rc;
+    /* be = the expanded linear bounds, row r of be is linear row r */
+    const BoundsDesc B{bounds_layout(pb), nC, 0, 0, dm.nclin, nullptr, nullptr, al.M, al.Ae};
+    BoundsArrays ba;
+    LsArrays la;
+    auto layout = [&](Carve &c) {
+        c.take(Pz * nr, y, yp, grp, d);
+        c.take(Pz * nr * nr, H);
+        c.take(Pz * nC, dC, g);
+        c.take(Pz, fv, phi0, dphi0, ab, pbest, state, its, fails);
+        c.take(kNalpha, alphas);
+        c.take(1, count);
+        if (run != Run::Sync) { /* what the synchronous path takes from the bounds' and the line search's scratch */
+            ba.take(c, Pz, B);
+            la.take(c, Pz * kNalpha, nC);
+        }
+    };
+    if (run == Run::Reserve) {
+        if (Pz * kNalpha > 0x7fffffffull) return fail(NTGB_EINVAL, "P*nalpha too large"); /* ntgb_linesearch's check */
+        return reserve_work(pb, aw, P, layout);
+    }
+    if ((rc = scratch_carve(run == Run::Sync ? pb->scratch.eq : aw.s, st, layout, run == Run::Sync))) return rc;
+    if (run == Run::Sync) {
+        if ((rc = upload_halving(alphas, kNalpha, st))) return rc;
+    } else {
+        alphas = pb->async.halving;
+    }
     CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
     const double *Cpart = al.Cpart;
     int Cstride = 0;
     if (lowerb) {
-        /* be = the expanded linear bounds, row r of be is linear row r */
-        BoundsDesc B{bounds_layout(pb), nC, 0, 0, dm.nclin, nullptr, nullptr, al.M, al.Ae};
-        double *Cp = nullptr, *hl = nullptr, *hu = nullptr;
-        if ((rc = bounds_prepare(pb, P, lowerb, upperb, B, st, state, its, count, &Cp, &hl, &hu))) return rc;
-        Cpart = Cp;
+        if (run == Run::Sync && (rc = scratch_carve(pb->scratch.bnd, st, [&](Carve &c) { ba.take(c, Pz, B); }))) return rc;
+        if ((rc = bounds_prepare(P, lowerb, upperb, B, ba, st, state, its, count))) return rc;
+        Cpart = ba.Cpart;
         Cstride = nC;
     }
     const unsigned grid = (unsigned)((P + 127) / 128);
@@ -2445,12 +2542,15 @@ int solve_eq_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, cons
         if ((rc = ntgb_eval(pb, &a))) return rc;
         CUDA_TRY(launch(k_solve_dir, grid, 128, st, P, nC, nr, al.N, fv, g, o.gtol, y, yp, grp, H, d, dC, phi0,
                         dphi0, state, fails, count));
-        if ((it + 1) % o.check_every == 0 && (rc = all_finished(count, P, st)) != 0) {
+        if (run == Run::Sync && (it + 1) % o.check_every == 0 && (rc = all_finished(count, P, st)) != 0) {
             if (rc < 0) return rc;
             break;
         }
-        if ((rc = ntgb_linesearch(pb, P, C, dC, kNalpha, alphas, 0.0, o.c1, phi0, dphi0, ab, pbest, nullptr, st)))
-            return rc;
+        if (run == Run::Sync)
+            rc = ntgb_linesearch(pb, P, C, dC, kNalpha, alphas, 0.0, o.c1, phi0, dphi0, ab, pbest, nullptr, st);
+        else
+            rc = linesearch_run(pb, P, C, dC, kNalpha, alphas, 0.0, o.c1, phi0, dphi0, ab, pbest, nullptr, st, la);
+        if (rc) return rc;
         CUDA_TRY(launch(k_solve_update, grid, 128, st, P, nC, nr, al.N, Cpart, Cstride, phi0, ab, pbest, d, y, H,
                         C, state, its, fails, count));
     }
@@ -2460,7 +2560,7 @@ int solve_eq_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, cons
     }
     if (iters) CUDA_TRY(cudaMemcpyAsync(iters, its, sizeof(int) * (size_t)P, cudaMemcpyDeviceToDevice, st));
     if (status) CUDA_TRY(cudaMemcpyAsync(status, state, sizeof(int) * (size_t)P, cudaMemcpyDeviceToDevice, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
+    if (run == Run::Sync) CUDA_TRY(cudaStreamSynchronize(st));
     return 0;
 }
 
@@ -2583,7 +2683,8 @@ int ntgb_solve_sqp(ntgb_problem *pb, int P, double *C, double *f, double *viol_o
                    double *lambda, int *istate, const ntgb_sqp_opts *opts, void *stream)
 {
     if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_sqp: null argument");
-    return solve_sqp_impl(pb, P, C, nullptr, nullptr, nullptr, f, viol_out, iters, status, lambda, istate, opts, stream);
+    return solve_sqp_impl(pb, Run::Sync, P, C, nullptr, nullptr, nullptr, f, viol_out, iters, status, lambda, istate, opts,
+                          stream);
 }
 
 int ntgb_solve_sqp_bounds(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
@@ -2593,7 +2694,8 @@ int ntgb_solve_sqp_bounds(ntgb_problem *pb, int P, double *C, const double *lowe
     if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_sqp_bounds: null argument");
     if (bounds_layout(pb).nb() > 0 && (!lowerb || !upperb))
         return fail(NTGB_EINVAL, "ntgb_solve_sqp_bounds: lowerb / upperb is NULL");
-    return solve_sqp_impl(pb, P, C, lowerb, upperb, nullptr, f, viol_out, iters, status, lambda, istate, opts, stream);
+    return solve_sqp_impl(pb, Run::Sync, P, C, lowerb, upperb, nullptr, f, viol_out, iters, status, lambda, istate, opts,
+                          stream);
 }
 
 int ntgb_sqp_warm_doubles(ntgb_problem *pb, size_t *n)
@@ -2614,20 +2716,44 @@ int ntgb_solve_sqp_warm(ntgb_problem *pb, int P, double *C, const double *lowerb
     if (!pb || !C || !warm) return fail(NTGB_EINVAL, "ntgb_solve_sqp_warm: null argument");
     if ((lowerb == nullptr) != (upperb == nullptr))
         return fail(NTGB_EINVAL, "ntgb_solve_sqp_warm: exactly one of lowerb / upperb is NULL");
-    return solve_sqp_impl(pb, P, C, lowerb, upperb, warm, f, viol_out, iters, status, lambda, istate, opts, stream);
+    return solve_sqp_impl(pb, Run::Sync, P, C, lowerb, upperb, warm, f, viol_out, iters, status, lambda, istate, opts,
+                          stream);
+}
+
+int ntgb_solve_sqp_reserve(ntgb_problem *pb, int P_max)
+{
+    if (!pb) return fail(NTGB_EINVAL, "ntgb_solve_sqp_reserve: null argument");
+    if (P_max < 1) return fail(NTGB_EINVAL, "ntgb_solve_sqp_reserve: P_max = %d", P_max);
+    return solve_sqp_impl(pb, Run::Reserve, P_max, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
+                          nullptr, nullptr, nullptr, nullptr);
+}
+
+int ntgb_solve_sqp_async(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *warm,
+                         double *f, double *viol_out, int *iters, int *status, double *lambda, int *istate,
+                         const ntgb_sqp_opts *opts, void *stream)
+{
+    if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_sqp_async: null argument");
+    if ((lowerb == nullptr) != (upperb == nullptr))
+        return fail(NTGB_EINVAL, "ntgb_solve_sqp_async: exactly one of lowerb / upperb is NULL");
+    return solve_sqp_impl(pb, Run::Async, P, C, lowerb, upperb, warm, f, viol_out, iters, status, lambda, istate, opts,
+                          stream);
 }
 
 } /* extern "C" */
 
 namespace {
 
-/* ntgb_solve_sqp, ntgb_solve_sqp_bounds and ntgb_solve_sqp_warm: lowerb == nullptr = the setup's bounds for
- * every problem; warm == nullptr = cold start, no state written back */
-int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *warm,
+/* ntgb_solve_sqp, ntgb_solve_sqp_bounds, ntgb_solve_sqp_warm and the reserve / async entry points (Run):
+ * lowerb == nullptr = the setup's bounds for every problem; warm == nullptr = cold start, no state written back */
+int solve_sqp_impl(ntgb_problem *pb, Run run, int P, double *C, const double *lowerb, const double *upperb, double *warm,
                    double *f, double *viol_out, int *iters, int *status, double *lambda, int *istate,
                    const ntgb_sqp_opts *opts, void *stream)
 {
     if (P <= 0) return 0;
+    AsyncWork &aw = pb->async.sqp;
+    if (run == Run::Async && P > aw.P)
+        return fail(NTGB_EINVAL, "ntgb_solve_sqp_async: P = %d above the %d problems reserved by ntgb_solve_sqp_reserve", P,
+                    aw.P);
     const ntgb_dims &dm = pb->dims;
     ntgb_sqp_opts o{100, 1e-6, 1e-8, 1e4, 1e-4, 4};
     if (opts) {
@@ -2662,20 +2788,35 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
     double *dC, *g, *gL, *mu, *cc, *J, *lin, *fv, *phi0, *dphi0;
     int *state, *its, *count;
     TwoStage ts;
-    if ((rc = scratch_carve(pb->scratch.sqp, st, [&](Carve &c) {
-             c.take(Pz * nr, S.y, S.sprev, S.grLold, S.grold, S.d);
-             c.take(Pz * nr * nr, S.B);
-             c.take(Pz * nC, dC, g, gL);
-             c.take(Pz * mz, S.lam, mu, S.istate);
-             c.take(Pz * ncz, cc);
-             c.take(Pz * ncz * dm.sorder, J);
-             c.take(Pz * nlz, lin);
-             c.take(Pz * 8, S.scal, S.flag);
-             c.take(Pz, fv, phi0, dphi0, state, its);
-             c.take(1, count);
-             ts.take(c, Pz, dm);
-         })))
-        return rc;
+    const BoundsDesc B{bounds_layout(pb), nC, n_li, m, sq.me, al.li_idx, sq.eq_idx, al.M, al.Ae};
+    BoundsArrays ba;
+    auto layout = [&](Carve &c) {
+        c.take(Pz * nr, S.y, S.sprev, S.grLold, S.grold, S.d);
+        c.take(Pz * nr * nr, S.B);
+        c.take(Pz * nC, dC, g, gL);
+        c.take(Pz * mz, S.lam, mu, S.istate);
+        c.take(Pz * ncz, cc);
+        c.take(Pz * ncz * dm.sorder, J);
+        c.take(Pz * nlz, lin);
+        c.take(Pz * 8, S.scal, S.flag);
+        c.take(Pz, fv, phi0, dphi0, state, its);
+        c.take(1, count);
+        ts.take(c, Pz, dm);
+        if (run != Run::Sync) ba.take(c, Pz, B); /* the synchronous path takes these from the bounds' scratch */
+    };
+    if (run == Run::Reserve) {
+        /* the limit every launch of k_sqp_step needs, raised to what the device offers: a reserve for a smaller
+         * QP on another ntgb_problem cannot lower it below this one's */
+        if (smem > 48 * 1024) {
+            cudaFuncAttributes fa;
+            CUDA_TRY(cudaFuncGetAttributes(&fa, k_sqp_step));
+            CUDA_TRY(cudaFuncSetAttribute(k_sqp_step, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          pb->max_smem_optin - (int)fa.sharedSizeBytes));
+        }
+        return reserve_work(pb, aw, P, layout);
+    }
+    if ((rc = scratch_carve(run == Run::Sync ? pb->scratch.sqp : aw.s, st, layout, run == Run::Sync))) return rc;
+    if (run == Run::Async) ts.alphas = pb->async.halving;
 
     SqpDesc D;
     D.nC = nC; D.nr = nr; D.m = m; D.n_li = n_li; D.nclin = nclin; D.ncnln = ncnln;
@@ -2684,20 +2825,20 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
     D.gtol = o.gtol; D.ctol = o.ctol; D.rho_pen = o.rho_pen;
     const double *Cpart = al.Cpart;
 
-    if ((rc = ts.start(P, st))) return rc;
+    if ((rc = ts.start(P, st, run == Run::Sync))) return rc;
     CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
     if (lowerb) {
-        BoundsDesc B{bounds_layout(pb), nC, n_li, m, sq.me, al.li_idx, sq.eq_idx, al.M, al.Ae};
-        double *Cp = nullptr, *hl = nullptr, *hu = nullptr;
-        if ((rc = bounds_prepare(pb, P, lowerb, upperb, B, st, state, its, count, &Cp, &hl, &hu))) return rc;
-        Cpart = Cp;
-        D.hl = hl; D.hu = hu;
+        if (run == Run::Sync && (rc = scratch_carve(pb->scratch.bnd, st, [&](Carve &c) { ba.take(c, Pz, B); }))) return rc;
+        if ((rc = bounds_prepare(P, lowerb, upperb, B, ba, st, state, its, count))) return rc;
+        Cpart = ba.Cpart;
+        D.hl = ba.hl; D.hu = ba.hu;
         D.Cstride = nC; D.hstride = m;
     }
     const unsigned grid = (unsigned)((P + 127) / 128);
     const ntgb::WarmKey wk{nr, m, al.digest};
     CUDA_TRY(launch(k_sqp_init, grid, 128, st, P, D, S, Cpart, C, state, its, (const double *)warm, wk));
-    if (smem > 48 * 1024) CUDA_TRY(cudaFuncSetAttribute(k_sqp_step, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (run == Run::Sync && smem > 48 * 1024)
+        CUDA_TRY(cudaFuncSetAttribute(k_sqp_step, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 
     ntgb_eval_args ea;
     memset(&ea, 0, sizeof ea);
@@ -2727,11 +2868,11 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
     for (int it = 0; it <= o.max_iter; it++) {
         if ((rc = direction())) return rc;
         if (it == o.max_iter) break; /* the last pass only evaluates and tests convergence at the final point */
-        if ((it + 1) % o.check_every == 0 && (rc = all_finished(count, P, st)) != 0) {
+        if (run == Run::Sync && (it + 1) % o.check_every == 0 && (rc = all_finished(count, P, st)) != 0) {
             if (rc < 0) return rc;
             break;
         }
-        if ((rc = two_stage_search(pb, P, C, dC, o.c1, phi0, dphi0, state, ts, st, merit))) return rc;
+        if ((rc = two_stage_search(pb, P, C, dC, o.c1, phi0, dphi0, state, ts, st, merit, run == Run::Async))) return rc;
         CUDA_TRY(launch(k_sqp_update, grid, 128, st, P, D, S, Cpart, phi0, ts.ab, ts.pbest, C, state, its, count));
     }
     if (warm)
@@ -2750,7 +2891,7 @@ int solve_sqp_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, con
                                              cudaMemcpyDeviceToDevice, st));
     if (iters) CUDA_TRY(cudaMemcpyAsync(iters, its, sizeof(int) * Pz, cudaMemcpyDeviceToDevice, st));
     if (status) CUDA_TRY(cudaMemcpyAsync(status, state, sizeof(int) * Pz, cudaMemcpyDeviceToDevice, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
+    if (run == Run::Sync) CUDA_TRY(cudaStreamSynchronize(st));
     return 0;
 }
 

@@ -64,6 +64,13 @@ def core() -> C.CDLL:
         lib.ntgb_sqp_warm_doubles.restype = C.c_int
         lib.ntgb_solve_sqp_warm.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 12
         lib.ntgb_solve_sqp_warm.restype = C.c_int
+        for name in ("ntgb_solve_eq_reserve", "ntgb_solve_sqp_reserve"):
+            getattr(lib, name).argtypes = [C.c_void_p, C.c_int]
+            getattr(lib, name).restype = C.c_int
+        lib.ntgb_solve_eq_async.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 8
+        lib.ntgb_solve_eq_async.restype = C.c_int
+        lib.ntgb_solve_sqp_async.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 12
+        lib.ntgb_solve_sqp_async.restype = C.c_int
         lib.ntgb_peer_table_alloc.argtypes = [C.c_void_p, C.c_size_t, C.POINTER(C.c_void_p), C.c_char_p]
         lib.ntgb_peer_table_open.argtypes = [C.c_void_p, C.c_char_p, C.POINTER(C.c_void_p)]
         lib.ntgb_peer_table_close.argtypes = [C.c_void_p, C.c_void_p]
@@ -318,11 +325,23 @@ class Problem:
                 raise ValueError(f"{name} must be a contiguous float64 tensor of shape {shape} on {Cdev.device}")
         return True
 
-    def solve_eq(self, Cdev, max_iter=0, gtol=0.0, c1=0.0, check_every=0, lowerb=None, upperb=None):
+    def solver_reserve(self, solver: str, P_max: int):
+        """one-time work and the work space of the stream-ordered solver ("eq" or "sqp") for up to P_max
+        problems (ntgb_solve_eq_reserve / ntgb_solve_sqp_reserve); needed before solve_eq / solve_sqp with
+        sync=False.  Synchronizes the device.  Reserving more replaces the work space: capture graphs again."""
+        fn = {"eq": core().ntgb_solve_eq_reserve, "sqp": core().ntgb_solve_sqp_reserve}.get(solver)
+        if fn is None:
+            raise ValueError(f"solver must be 'eq' or 'sqp', not {solver!r}")
+        _check(fn(self._h, int(P_max)))
+
+    def solve_eq(self, Cdev, max_iter=0, gtol=0.0, c1=0.0, check_every=0, lowerb=None, upperb=None, sync=True):
         """batched reduced-space BFGS (ntgb_solve_eq); Cdev [P][nC] is overwritten with the solutions.
         Returns f [P], iters [P], status [P] (1 converged, 2 no further decrease, 0 iteration limit).
         lowerb / upperb [P][spec.nbounds] (device): each problem's own bounds, in the layout of
-        spec.lowerb / upperb (ntgb_solve_eq_bounds; status 5 = that problem's bounds were rejected)."""
+        spec.lowerb / upperb (ntgb_solve_eq_bounds; status 5 = that problem's bounds were rejected).
+        sync=False: ntgb_solve_eq_async on torch's current stream (after solver_reserve("eq", P)): exactly
+        max_iter iterations, the same outputs bit for bit, returned without waiting; capturable in a
+        torch.cuda.graph."""
         import torch
         P = Cdev.shape[0]
         per_problem = self._check_bounds(Cdev, lowerb, upperb)
@@ -331,7 +350,11 @@ class Problem:
         stt = torch.zeros(P, dtype=torch.int32, device=Cdev.device)
         opts = SolveOpts(int(max_iter), float(gtol), float(c1), int(check_every))
         st = torch.cuda.current_stream(Cdev.device).cuda_stream
-        if per_problem:
+        if not sync:
+            lo_p, up_p = (lowerb.data_ptr(), upperb.data_ptr()) if per_problem else (None, None)
+            _check(core().ntgb_solve_eq_async(self._h, P, Cdev.data_ptr(), lo_p, up_p, f.data_ptr(), it.data_ptr(),
+                                              stt.data_ptr(), C.addressof(opts), st))
+        elif per_problem:
             _check(core().ntgb_solve_eq_bounds(self._h, P, Cdev.data_ptr(), lowerb.data_ptr(), upperb.data_ptr(),
                                                f.data_ptr(), it.data_ptr(), stt.data_ptr(), C.addressof(opts), st))
         else:
@@ -369,12 +392,15 @@ class Problem:
         return torch.zeros((P, self.sqp_warm_doubles()), dtype=torch.float64, device=torch.device("cuda", self.device))
 
     def solve_sqp(self, Cdev, max_iter=0, gtol=0.0, ctol=0.0, rho_pen=0.0, c1=0.0, check_every=0, multipliers=False,
-                  lowerb=None, upperb=None, warm=None):
+                  lowerb=None, upperb=None, warm=None, sync=True):
         """batched SQP solve (ntgb_solve_sqp); Cdev [P][nC] is overwritten.  Returns f [P], violation [P],
         iters [P], status [P] and, with multipliers=True, lambda and istate [P][nclin + ncnln] (NPSOL's order).
         lowerb / upperb [P][spec.nbounds] (device): each problem's own bounds (ntgb_solve_sqp_bounds).
         warm [P][sqp_warm_doubles()] (device, from sqp_warm_state): solver state carried from the previous
-        call and updated in place (ntgb_solve_sqp_warm)."""
+        call and updated in place (ntgb_solve_sqp_warm).
+        sync=False: ntgb_solve_sqp_async on torch's current stream (after solver_reserve("sqp", P)): exactly
+        max_iter iterations, the same outputs bit for bit, returned without waiting; capturable in a
+        torch.cuda.graph."""
         import torch
         P, d = Cdev.shape[0], self.dims
         per_problem = self._check_bounds(Cdev, lowerb, upperb)
@@ -394,7 +420,12 @@ class Problem:
         opts = SqpOpts(int(max_iter), float(gtol), float(ctol), float(rho_pen), float(c1), int(check_every))
         st = torch.cuda.current_stream(Cdev.device).cuda_stream
         lam_p, ist_p = (lam.data_ptr(), ist.data_ptr()) if multipliers else (None, None)
-        if warm is not None:
+        if not sync:
+            lo_p, up_p = (lowerb.data_ptr(), upperb.data_ptr()) if per_problem else (None, None)
+            _check(core().ntgb_solve_sqp_async(self._h, P, Cdev.data_ptr(), lo_p, up_p, _ptr(warm), f.data_ptr(),
+                                               v.data_ptr(), it.data_ptr(), stt.data_ptr(), lam_p, ist_p,
+                                               C.addressof(opts), st))
+        elif warm is not None:
             lo_p, up_p = (lowerb.data_ptr(), upperb.data_ptr()) if per_problem else (None, None)
             _check(core().ntgb_solve_sqp_warm(self._h, P, Cdev.data_ptr(), lo_p, up_p, warm.data_ptr(), f.data_ptr(),
                                               v.data_ptr(), it.data_ptr(), stt.data_ptr(), lam_p, ist_p,
