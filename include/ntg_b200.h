@@ -459,6 +459,44 @@ int  ntgb_solve_sqp_async(ntgb_problem *pb, int P, double *C, const double *lowe
                           double *warm, double *f, double *viol, int *iters, int *status, double *lambda,
                           int *istate, const ntgb_sqp_opts *opts, void *stream);
 
+/*
+ * Long horizons: the problem class of ntgb_solve_eq (a smooth cost, only EQUALITY linear constraints, no
+ * nonlinear ones) with any number of free directions.  Projected L-BFGS: no null-space basis is formed.
+ * The projector onto null(A) is P v = v - Q1 (Q1' v), Q1 the nC x r orthonormal basis of the equality
+ * rows' span from the same pivoted QR that ntgb_solve_eq uses.  C is projected onto each problem's affine
+ * set at entry and after every accepted step, so A C = b holds to rounding throughout.  Per iteration:
+ * one batched evaluation (cost + gradient), one CTA per problem for the projected gradient, the curvature
+ * pair (s = the step taken, u = the change of P g; skipped when s'u <= 1e-10 |s| |u|), the two-loop
+ * recursion with H0 = (s'u / u'u) I of the newest pair, and d = -P (H P g) (the history is dropped and
+ * d = -P g when d'g >= 0), then the two-stage Armijo search of ntgb_solve_sqp on the cost (steps 1 .. 1/8
+ * for every problem, 2^-4 .. 2^-15 for the rest).  Each reduction has a fixed order that depends on nC
+ * alone: results do not depend on the batch size or order.
+ *
+ * Arguments and outputs as in ntgb_solve_eq_bounds: lowerb / upperb both NULL (the setup's bounds) or both
+ * set (DEVICE [P][nb] per-problem bounds); exactly one NULL is NTGB_EINVAL before any CUDA call, and so is
+ * opts->memory outside 1..32.  opts may be NULL (every default); in a non-NULL opts, a max_iter, gtol, c1
+ * or check_every <= 0 takes its default.  status: 1 |P g|_inf <= gtol max(1, |f|), 2 no further decrease
+ * (also from steepest descent) or a NaN gradient, 0 iteration limit, NTGB_STATUS_BAD_BOUNDS rejected bounds
+ * (C left untouched bit for bit, iters 0).  Refusals as in ntgb_solve_eq (nonlinear or inequality rows:
+ * NTGB_EINVAL).  Linear equalities that leave no free direction give C = C_part, status 1 and iters 0, as
+ * ntgb_solve_eq does.  There is no limit on free directions.  Synchronous.
+ *
+ * Work space (device, kept between calls, freed by ntgb_destroy): about
+ *     P (2 memory + 16 + 4) nC + r nC  doubles
+ * (the curvature pairs, the 16 trial points of the search, the gradient, direction, last step and last
+ * projected gradient; Q1), plus nC per problem with per-problem bounds.  Nothing of size nC x nC or
+ * nC x (nC - r) is on the device.  The host builds the dense nC x nC Q of the QR once per setup.
+ */
+typedef struct ntgb_lbfgs_opts {
+    int max_iter;     /* default 500 */
+    double gtol;      /* |P g|_inf <= gtol * max(1, |f|), default 1e-9 */
+    double c1;        /* Armijo constant, default 1e-4 */
+    int memory;       /* curvature pairs kept per problem, 1..32, default 8 */
+    int check_every;  /* host reads the done counter every this many iterations, default 4 */
+} ntgb_lbfgs_opts;
+int  ntgb_solve_eq_lbfgs(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb,
+                         double *f, int *iters, int *status, const ntgb_lbfgs_opts *opts, void *stream);
+
 /* Gathered result tables for the fused multi-GPU gather (ntgb_eval_args.peer_result): alloc creates
  * this rank's table (rows x 2 doubles, zeroed) and the 64-byte CUDA IPC handle the other ranks
  * need; open maps another rank's table into this process (peer access over NVLink is enabled on

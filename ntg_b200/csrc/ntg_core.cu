@@ -33,6 +33,7 @@
 #include "ntg_sqp.cuh"
 #include "ntg_bounds.h"
 #include "ntg_warm.h"
+#include "ntg_lbfgs.h"
 
 namespace {
 
@@ -148,6 +149,8 @@ struct ntgb_problem {
         bool ready = false;
         int nr = 0, n_li = 0, m = 0;
         double *N = nullptr, *Cpart = nullptr; /* N [nr][nC] (basis vector k contiguous), Cpart [nC] */
+        int r = 0;                  /* rank of the eliminated rows, nC - nr */
+        double *Q1 = nullptr;       /* [r][nC] orthonormal rows spanning the eliminated rows (ntgb_solve_eq_lbfgs) */
         double *M = nullptr, *Ae = nullptr; /* Cpart = M be, M [nC][me]; eliminated rows Ae [me][nC] */
         int *li_idx = nullptr;      /* [n_li] linear row of general constraint i */
         double *hl = nullptr, *hu = nullptr; /* [m] bounds: linear inequality rows, then the nonlinear rows */
@@ -166,7 +169,7 @@ struct ntgb_problem {
     } sqp;
     /* per-call device arrays, kept between calls: one scratch per driver, so that no call's arrays alias
      * another solver's (ntgb_solve_eq, ntgb_solve_nlp, ntgb_solve_sqp, ntgb_linesearch, per-problem bounds) */
-    struct { Scratch eq, nlp, sqp, ls, bnd; } scratch;
+    struct { Scratch eq, nlp, sqp, ls, bnd, lbfgs; } scratch;
     /* ntgb_solve_eq_async / ntgb_solve_sqp_async: their own work spaces, apart from `scratch`, so that no
      * synchronous call moves an array that a captured graph uses; halving = the step table 2^-a, a < 16 */
     struct {
@@ -570,12 +573,13 @@ __global__ void k_solve_update(int P, int nC, int nr, const double *N, const dou
     }
 }
 
-/* Host: orthonormal null-space basis N of A (m x n, column-major) and the minimum-norm solution of
- * A*C = b, by Householder QR with column pivoting of A^T.  Mop (optional) receives the linear operator
- * of that solution, Cpart = Mop b for any right-hand side b ([n][m] row-major; zero columns for the
- * rows the pivoting found dependent), which the per-problem-bounds solvers apply on the device. */
-int reduce_linear(const std::vector<double> &A, int m, int n, const std::vector<double> &b, std::vector<double> &N,
-                  std::vector<double> &Cpart, int &nr, std::vector<double> *Mop = nullptr)
+/* Host: the minimum-norm solution of A*C = b (A m x n, column-major) and nr = n - rank(A), by Householder QR
+ * with column pivoting of A^T.  Optional outputs: N, the orthonormal null-space basis of A ([nr][n], the last
+ * nr columns of Q); Q1, the orthonormal basis of its row space ([r][n], the first r columns of Q, r = n - nr);
+ * Mop, the linear operator of that solution, Cpart = Mop b for any right-hand side b ([n][m] row-major; zero
+ * columns for the rows the pivoting found dependent), which the per-problem-bounds solvers apply on the device. */
+int reduce_linear(const std::vector<double> &A, int m, int n, const std::vector<double> &b, std::vector<double> *N,
+                  std::vector<double> &Cpart, int &nr, std::vector<double> *Mop = nullptr, std::vector<double> *Q1 = nullptr)
 {
     std::vector<double> M((size_t)n * std::max(m, 1)), Q((size_t)n * n, 0.0), v(n);
     std::vector<int> perm(m);
@@ -656,9 +660,16 @@ int reduce_linear(const std::vector<double> &A, int m, int n, const std::vector<
     }
     if (res > 1e-8 * (1.0 + bmax)) return fail(NTGB_EINVAL, "linear equality constraints are inconsistent (residual %g)", res);
     nr = n - r;
-    N.resize((size_t)nr * n);
-    for (int k = 0; k < nr; k++)
-        for (int i = 0; i < n; i++) N[(size_t)k * n + i] = Q[i + (size_t)(r + k) * n];
+    if (N) {
+        N->resize((size_t)nr * n);
+        for (int k = 0; k < nr; k++)
+            for (int i = 0; i < n; i++) (*N)[(size_t)k * n + i] = Q[i + (size_t)(r + k) * n];
+    }
+    if (Q1) {
+        Q1->resize((size_t)r * n);
+        for (int k = 0; k < r; k++)
+            for (int i = 0; i < n; i++) (*Q1)[(size_t)k * n + i] = Q[i + (size_t)k * n];
+    }
     return 0;
 }
 
@@ -905,37 +916,41 @@ void host_band_row(const ntgb_problem *pb, const double *dz, int bp, double *ban
     }
 }
 
-/* reduced form shared by ntgb_solve_eq, ntgb_solve_nlp and ntgb_solve_sqp: linear equality rows eliminated
- * (C = Cpart + N y), the other linear rows and the nonlinear rows kept as general constraints */
-int alm_prepare(ntgb_problem *pb)
+/* reduced form shared by the batched solvers: linear equality rows eliminated (C = Cpart + N y), the other
+ * linear rows and the nonlinear rows kept as general constraints.  The part every solver uses (the row split,
+ * Cpart, M, Ae, the general rows' bounds) is built on the first call; the basis each solver needs on top of it
+ * on the first call that asks for it: want_N, the null-space basis N and the warm digest (ntgb_solve_eq,
+ * ntgb_solve_nlp, ntgb_solve_sqp); want_Q1, the row-space basis Q1 (ntgb_solve_eq_lbfgs, which puts nothing
+ * of size nC x nr on the device).  A later call that needs the other basis repeats the host QR, which
+ * gives the same bits. */
+int reduced_form(ntgb_problem *pb, bool want_N, bool want_Q1)
 {
     auto &al = pb->alm;
-    if (al.ready) return 0;
+    const bool need_N = want_N && !al.N, need_Q1 = want_Q1 && !al.Q1;
+    if (al.ready && !need_N && !need_Q1) return 0;
     const ntgb_dims &dm = pb->dims;
     const int nC = dm.nC, nclin = dm.nclin, ncnln = dm.ncnln;
     int rc;
-    {
-        /* split the linear rows: equalities are eliminated, the rest become general constraints */
-        std::vector<int> eq, li;
-        for (int i = 0; i < nclin; i++) (pb->lin_lb[i] == pb->lin_ub[i] ? eq : li).push_back(i);
-        const int me = (int)eq.size();
-        std::vector<double> Ae((size_t)std::max(me, 1) * nC, 0.0), be((size_t)me);
-        for (int r = 0; r < me; r++) {
-            be[r] = pb->lin_lb[eq[r]];
-            for (int c = 0; c < nC; c++) Ae[r + (size_t)c * me] = pb->A[eq[r] + (size_t)c * nclin];
-        }
-        std::vector<double> N, Cpart, Mop;
-        int nr = 0;
-        if ((rc = reduce_linear(Ae, me, nC, be, N, Cpart, nr, &Mop))) return rc;
+    /* split the linear rows: equalities are eliminated, the rest become general constraints */
+    std::vector<int> eq, li;
+    for (int i = 0; i < nclin; i++) (pb->lin_lb[i] == pb->lin_ub[i] ? eq : li).push_back(i);
+    const int me = (int)eq.size();
+    std::vector<double> Ae((size_t)std::max(me, 1) * nC, 0.0), be((size_t)me);
+    for (int r = 0; r < me; r++) {
+        be[r] = pb->lin_lb[eq[r]];
+        for (int c = 0; c < nC; c++) Ae[r + (size_t)c * me] = pb->A[eq[r] + (size_t)c * nclin];
+    }
+    std::vector<double> N, Cpart, Mop, Q1;
+    int nr = 0;
+    if ((rc = reduce_linear(Ae, me, nC, be, need_N ? &N : nullptr, Cpart, nr, al.ready ? nullptr : &Mop,
+                            need_Q1 ? &Q1 : nullptr)))
+        return rc;
+    if (!al.ready) {
         al.nr = nr;
-        al.hN = N;
         al.eq = eq;
         al.li = li;
         al.n_li = (int)li.size();
         al.m = al.n_li + ncnln;
-        al.digest = ntgb::warm_digest(nC, nr, al.m, al.n_li, li.data(), N.data());
-        if (N.empty()) N.push_back(0.0);
-        if ((rc = dev_upload(pb, &al.N, N.data(), N.size()))) return rc;
         if ((rc = dev_upload(pb, &al.Cpart, Cpart.data(), Cpart.size()))) return rc;
         /* for per-problem right-hand sides: Cpart = M be and the rows to check the residual against */
         std::vector<double> Aer((size_t)std::max(me, 1) * nC, 0.0);
@@ -951,17 +966,31 @@ int alm_prepare(ntgb_problem *pb)
         std::vector<double> bl((size_t)nC + nclin + ncnln), bu(bl.size());
         if ((rc = ntgb_get_bounds(pb, bl.data(), bu.data()))) return rc;
         std::vector<double> hl((size_t)std::max(al.m, 1), 0.0), hu((size_t)std::max(al.m, 1), 0.0);
-        for (int i = 0; i < al.n_li; i++) { hl[i] = pb->lin_lb[li[i]]; hu[i] = pb->lin_ub[li[i]]; }
+        for (int i = 0; i < al.n_li; i++) { hl[i] = pb->lin_lb[al.li[i]]; hu[i] = pb->lin_ub[al.li[i]]; }
         for (int i = 0; i < ncnln; i++) { hl[al.n_li + i] = bl[(size_t)nC + nclin + i]; hu[al.n_li + i] = bu[(size_t)nC + nclin + i]; }
         if ((rc = dev_upload(pb, &al.hl, hl.data(), hl.size()))) return rc;
         if ((rc = dev_upload(pb, &al.hu, hu.data(), hu.size()))) return rc;
         std::vector<double> Ad = pb->A;
         if (Ad.empty()) Ad.push_back(0.0);
         if ((rc = dev_upload(pb, &al.A, Ad.data(), Ad.size()))) return rc;
+        al.ready = true;
     }
-    al.ready = true;
+    if (need_N) {
+        al.hN = N;
+        al.digest = ntgb::warm_digest(nC, nr, al.m, al.n_li, al.li.data(), N.data());
+        if (N.empty()) N.push_back(0.0);
+        if ((rc = dev_upload(pb, &al.N, N.data(), N.size()))) return rc;
+    }
+    if (need_Q1) {
+        al.r = nC - nr;
+        if (Q1.empty()) Q1.push_back(0.0);
+        if ((rc = dev_upload(pb, &al.Q1, Q1.data(), Q1.size()))) return rc;
+    }
     return 0;
 }
+
+/* the reduced form of the solvers that work on y (C = Cpart + N y) */
+int alm_prepare(ntgb_problem *pb) { return reduced_form(pb, true, false); }
 
 /* the SQP entry points (`who`): alm's reduced form, which must leave a free direction, and once per problem
  * the reduced gradients ArN of the linear inequality rows and W = (Ae Ae')^-1 Ae for the multipliers of the
@@ -1536,8 +1565,21 @@ int reserve_work(ntgb_problem *pb, AsyncWork &w, int P, Layout layout)
     return 0;
 }
 
+/* the problem class of ntgb_solve_eq and ntgb_solve_eq_lbfgs (`who`): no nonlinear row, every linear row an
+ * equality */
+int check_eq_only(const ntgb_problem *pb, const char *who)
+{
+    const ntgb_dims &dm = pb->dims;
+    if (dm.ncnln > 0) return fail(NTGB_EINVAL, "%s: problem has %d nonlinear constraints", who, dm.ncnln);
+    for (int i = 0; i < dm.nclin; i++)
+        if (pb->lin_lb[i] != pb->lin_ub[i]) return fail(NTGB_EINVAL, "%s: linear constraint %d is not an equality", who, i);
+    return 0;
+}
+
 int solve_eq_impl(ntgb_problem *pb, Run run, int P, double *C, const double *lowerb, const double *upperb, double *f,
                   int *iters, int *status, const ntgb_solve_opts *opts, void *stream);
+int solve_lbfgs_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                     int *iters, int *status, const ntgb_lbfgs_opts &o, void *stream);
 int solve_sqp_impl(ntgb_problem *pb, Run run, int P, double *C, const double *lowerb, const double *upperb, double *warm,
                    double *f, double *viol_out, int *iters, int *status, double *lambda, int *istate,
                    const ntgb_sqp_opts *opts, void *stream);
@@ -1590,7 +1632,7 @@ void ntgb_destroy(ntgb_problem *pb)
     for (void *p : pb->allocs) cudaFree(p);
     if (pb->zc.buf) cudaFreeHost(pb->zc.buf);
     auto &s = pb->scratch;
-    for (Scratch *sc : {&s.eq, &s.nlp, &s.sqp, &s.ls, &s.bnd, &pb->async.eq.s, &pb->async.sqp.s}) cudaFree(sc->p);
+    for (Scratch *sc : {&s.eq, &s.nlp, &s.sqp, &s.ls, &s.bnd, &s.lbfgs, &pb->async.eq.s, &pb->async.sqp.s}) cudaFree(sc->p);
     for (auto &h : pb->hs) {
         double *hsp[] = {h.C, h.f, h.g, h.c, h.J, h.Z, h.result};
         for (double *p : hsp)
@@ -2456,6 +2498,28 @@ int ntgb_solve_eq_async(ntgb_problem *pb, int P, double *C, const double *lowerb
     return solve_eq_impl(pb, Run::Async, P, C, lowerb, upperb, f, iters, status, opts, stream);
 }
 
+int ntgb_solve_eq_lbfgs(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                        int *iters, int *status, const ntgb_lbfgs_opts *opts, void *stream)
+{
+    /* the argument checks read nothing behind pb */
+    if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_eq_lbfgs: null argument");
+    if ((lowerb == nullptr) != (upperb == nullptr))
+        return fail(NTGB_EINVAL, "ntgb_solve_eq_lbfgs: exactly one of lowerb / upperb is NULL");
+    ntgb_lbfgs_opts o{500, 1e-9, 1e-4, 8, 4};
+    if (opts) {
+        if (opts->memory < 1 || opts->memory > ntgb::lbfgs::kMaxMemory)
+            return fail(NTGB_EINVAL, "ntgb_solve_eq_lbfgs: memory = %d outside [1,%d]", opts->memory,
+                        ntgb::lbfgs::kMaxMemory);
+        o.memory = opts->memory;
+        if (opts->max_iter > 0) o.max_iter = opts->max_iter;
+        if (opts->gtol > 0.0) o.gtol = opts->gtol;
+        if (opts->c1 > 0.0) o.c1 = opts->c1;
+        if (opts->check_every > 0) o.check_every = opts->check_every;
+    }
+    if (P <= 0) return 0;
+    return solve_lbfgs_impl(pb, P, C, lowerb, upperb, f, iters, status, o, stream);
+}
+
 } /* extern "C" */
 
 namespace {
@@ -2471,10 +2535,8 @@ int solve_eq_impl(ntgb_problem *pb, Run run, int P, double *C, const double *low
         return fail(NTGB_EINVAL, "ntgb_solve_eq_async: P = %d above the %d problems reserved by ntgb_solve_eq_reserve", P,
                     aw.P);
     const ntgb_dims &dm = pb->dims;
-    if (dm.ncnln > 0) return fail(NTGB_EINVAL, "ntgb_solve_eq: problem has %d nonlinear constraints", dm.ncnln);
-    for (int i = 0; i < dm.nclin; i++)
-        if (pb->lin_lb[i] != pb->lin_ub[i])
-            return fail(NTGB_EINVAL, "ntgb_solve_eq: linear constraint %d is not an equality", i);
+    int rc;
+    if ((rc = check_eq_only(pb, "ntgb_solve_eq"))) return rc;
     ntgb_solve_opts o{200, 1e-9, 1e-4, 4};
     if (opts) {
         if (opts->max_iter > 0) o.max_iter = opts->max_iter;
@@ -2486,7 +2548,6 @@ int solve_eq_impl(ntgb_problem *pb, Run run, int P, double *C, const double *low
     if (!dg.ok) return fail(NTGB_ECUDA, "cannot select device %d", pb->device);
     cudaStream_t st = (cudaStream_t)stream;
     const int nC = dm.nC;
-    int rc;
     /* every linear row is an equality (the refusals above), so alm's reduced form eliminates all of them */
     if ((rc = alm_prepare(pb))) return rc;
     const auto &al = pb->alm;
@@ -2561,6 +2622,213 @@ int solve_eq_impl(ntgb_problem *pb, Run run, int P, double *C, const double *low
     if (iters) CUDA_TRY(cudaMemcpyAsync(iters, its, sizeof(int) * (size_t)P, cudaMemcpyDeviceToDevice, st));
     if (status) CUDA_TRY(cudaMemcpyAsync(status, state, sizeof(int) * (size_t)P, cudaMemcpyDeviceToDevice, st));
     if (run == Run::Sync) CUDA_TRY(cudaStreamSynchronize(st));
+    return 0;
+}
+
+
+/* ---- ntgb_solve_eq_lbfgs: projected L-BFGS, one CTA per problem running ntg_lbfgs.h --------------------- */
+struct LbfgsDesc {
+    const double *Q1; /* [r][nC] */
+    int r, nC, mem;
+};
+
+/* per-problem state: the ring [P][mem][2][nC] of curvature pairs and what ntg_lbfgs.h keeps next to it */
+struct LbfgsArrays {
+    double *ring, *sv, *gp; /* [P][mem][2][nC], [P][nC], [P][nC] */
+    double *rho;            /* [P][mem] */
+    double *gamma;          /* [P] */
+    int *state, *its, *head, *npair, *pend; /* [P] */
+
+    void take(Carve &c, size_t P, int nC, int mem)
+    {
+        c.take(P * mem * 2 * nC, ring);
+        c.take(P * nC, sv, gp);
+        c.take(P * mem, rho);
+        c.take(P, gamma);
+        c.take(P, state, its, head, npair, pend);
+    }
+    __device__ ntgb::lbfgs::View view(const LbfgsDesc &D, int p) const
+    {
+        const size_t n = D.nC;
+        return ntgb::lbfgs::View{D.Q1, D.r, D.nC, D.mem, ring + (size_t)p * D.mem * 2 * n, rho + (size_t)p * D.mem,
+                                 sv + p * n, gp + p * n};
+    }
+    __device__ ntgb::lbfgs::State load(int p) const { return ntgb::lbfgs::State{head[p], npair[p], pend[p], gamma[p]}; }
+    __device__ void store(int p, const ntgb::lbfgs::State &s) const
+    {
+        head[p] = s.head;
+        npair[p] = s.npair;
+        pend[p] = s.pend;
+        gamma[p] = s.gamma;
+    }
+};
+
+/* threads per problem: every step streams a handful of nC-vectors through a chain of block reductions.  Up to
+ * a few thousand coefficients, 128 threads keep each reduction short and leave room for more resident CTAs;
+ * at CFG-5 sizes (nC = 4824) 256 threads halve the elements each thread walks between two reductions, and
+ * such batches are small, so the larger CTA costs no occupancy.  It depends on nC alone, so the reduction
+ * order, and every result, does not depend on the batch. */
+int lbfgs_threads(int nC) { return nC >= 2048 ? 256 : 128; }
+
+/* the CTA as ntg_lbfgs.h's group; its reductions take one double of shared memory per warp */
+__device__ __forceinline__ sqp::Coop lbfgs_group()
+{
+    return sqp::Coop{(int)threadIdx.x, (int)blockDim.x, (int)(threadIdx.x & 31), 32};
+}
+
+/* at entry: C onto problem p's affine set, fresh history.  Per-problem bounds (Cstride = nC): k_bounds_prep has
+ * set state / iters, a rejected problem keeps its C.  No free direction (r == nC): C = Cpart and status 1, as
+ * ntgb_solve_eq gives */
+__global__ void k_lbfgs_init(int P, LbfgsDesc D, LbfgsArrays S, const double *Cpart, int Cstride, double *C)
+{
+    __shared__ double red[8];
+    const int p = blockIdx.x;
+    if (Cstride != 0 && S.state[p] == NTGB_STATUS_BAD_BOUNDS) return;
+    Cpart += (size_t)p * Cstride;
+    double *Cp = C + (size_t)p * D.nC;
+    if (D.r == D.nC) {
+        for (int e = threadIdx.x; e < D.nC; e += blockDim.x) Cp[e] = Cpart[e];
+    } else {
+        ntgb::lbfgs::affine_step(lbfgs_group(), red, S.view(D, p), Cpart, Cp, nullptr, 0.0);
+    }
+    if (threadIdx.x == 0) {
+        S.state[p] = D.r == D.nC ? 1 : 0;
+        S.its[p] = 0;
+        S.store(p, ntgb::lbfgs::State{0, 0, 0, 1.0});
+    }
+}
+
+/* projected gradient, convergence test, pair update, two-loop direction dC and its slope; a finished problem
+ * gets dC = 0 and slope 0, which keeps it where it is through the search */
+__global__ void k_lbfgs_dir(int P, LbfgsDesc D, LbfgsArrays S, const double *f, const double *g, double gtol, double *dC,
+                            double *phi0, double *dphi0, int *count)
+{
+    __shared__ double red[8];
+    const int p = blockIdx.x;
+    const size_t n = D.nC;
+    double *d = dC + p * n;
+    int st = S.state[p];
+    double dg = 0.0;
+    if (st == 0) {
+        ntgb::lbfgs::State s = S.load(p);
+        st = ntgb::lbfgs::direction(lbfgs_group(), red, S.view(D, p), s, f[p], g + p * n, gtol, d, dg);
+        if (threadIdx.x == 0) {
+            S.store(p, s);
+            if (st != 0) {
+                S.state[p] = st;
+                atomicAdd(count, 1);
+            }
+        }
+    }
+    if (st != 0) {
+        for (size_t e = threadIdx.x; e < n; e += blockDim.x) d[e] = 0.0;
+        dg = 0.0;
+    }
+    if (threadIdx.x == 0) {
+        phi0[p] = f[p];
+        dphi0[p] = dg;
+    }
+}
+
+/* the step the search chose, or what a failed search means (ntg_lbfgs.h accept) */
+__global__ void k_lbfgs_update(int P, LbfgsDesc D, LbfgsArrays S, const double *Cpart, int Cstride, const double *phi0,
+                               const double *alpha_best, const double *phi_best, const double *dC, double *C, int *count)
+{
+    __shared__ double red[8];
+    const int p = blockIdx.x;
+    if (S.state[p] != 0) return;
+    const size_t n = D.nC;
+    ntgb::lbfgs::State s = S.load(p);
+    const int st = ntgb::lbfgs::accept(lbfgs_group(), red, S.view(D, p), s, Cpart + (size_t)p * Cstride, C + p * n,
+                                       dC + p * n, alpha_best[p], phi0[p], phi_best[p]);
+    if (threadIdx.x == 0) {
+        S.its[p] += 1;
+        S.store(p, s);
+        if (st != 0) {
+            S.state[p] = st;
+            atomicAdd(count, 1);
+        }
+    }
+}
+
+/* merit of the L-BFGS search: the plain cost, where two_stage_search's pick kernels read it */
+__global__ void k_cost_merit(int Q, const double *f, double *res)
+{
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q < Q) res[2 * (size_t)q] = f[q];
+}
+
+/* ntgb_solve_eq_lbfgs.  The search is two_stage_search on the plain cost: L-BFGS accepts the unit step most of
+ * the time, so the 4 coarse steps evaluated for every problem usually decide, and the 12 fine ones are
+ * evaluated only for the few problems that need them (ntgb_linesearch would evaluate 12 for every problem). */
+int solve_lbfgs_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                     int *iters, int *status, const ntgb_lbfgs_opts &o, void *stream)
+{
+    const ntgb_dims &dm = pb->dims;
+    const int nC = dm.nC;
+    int rc;
+    if ((rc = check_eq_only(pb, "ntgb_solve_eq_lbfgs"))) return rc;
+    if ((rc = TwoStage::check_size(P))) return rc;
+    DeviceGuard dg(pb->device);
+    if (!dg.ok) return fail(NTGB_ECUDA, "cannot select device %d", pb->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    if ((rc = reduced_form(pb, false, true))) return rc;
+    const auto &al = pb->alm;
+    const size_t Pz = (size_t)P;
+    const LbfgsDesc D{al.Q1, al.r, nC, o.memory};
+    /* be = the expanded linear bounds, row r of be is linear row r (every linear row is eliminated) */
+    const BoundsDesc B{bounds_layout(pb), nC, 0, 0, dm.nclin, nullptr, nullptr, al.M, al.Ae};
+    LbfgsArrays S;
+    TwoStage ts;
+    BoundsArrays ba;
+    double *g, *dC, *fv, *phi0, *dphi0;
+    int *count;
+    if ((rc = scratch_carve(pb->scratch.lbfgs, st, [&](Carve &c) {
+             S.take(c, Pz, nC, o.memory);
+             c.take(Pz * nC, g, dC);
+             c.take(Pz, fv, phi0, dphi0);
+             c.take(1, count);
+             ts.take(c, Pz, dm);
+             if (lowerb) ba.take(c, Pz, B);
+         })))
+        return rc;
+    if ((rc = ts.start(P, st))) return rc;
+    CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
+    const double *Cpart = al.Cpart;
+    int Cstride = 0;
+    if (lowerb) {
+        if ((rc = bounds_prepare(P, lowerb, upperb, B, ba, st, S.state, S.its, count))) return rc;
+        Cpart = ba.Cpart;
+        Cstride = nC;
+    }
+    const int nt = lbfgs_threads(nC);
+    CUDA_TRY(launch(k_lbfgs_init, (unsigned)P, nt, st, P, D, S, Cpart, Cstride, C));
+    ntgb_eval_args a;
+    memset(&a, 0, sizeof a);
+    a.P = P; a.C = C; a.mode_obj = 2; a.mode_con = -1; a.f = fv; a.g = g; a.jac_layout = NTGB_JAC_NONE; a.stream = st;
+    auto merit = [&](int n, int, const int *) -> int {
+        CUDA_TRY(launch(k_cost_merit, (unsigned)((n + 255) / 256), 256, st, n, (const double *)ts.ft, ts.res));
+        return 0;
+    };
+    const int max_iter = al.nr > 0 ? o.max_iter : 0; /* no free direction: k_lbfgs_init has finished every problem */
+    for (int it = 0; it < max_iter; it++) {
+        if ((rc = ntgb_eval(pb, &a))) return rc;
+        CUDA_TRY(launch(k_lbfgs_dir, (unsigned)P, nt, st, P, D, S, (const double *)fv, (const double *)g, o.gtol, dC, phi0,
+                        dphi0, count));
+        if ((it + 1) % o.check_every == 0 && (rc = all_finished(count, P, st)) != 0) {
+            if (rc < 0) return rc;
+            break;
+        }
+        if ((rc = two_stage_search(pb, P, C, dC, o.c1, phi0, dphi0, S.state, ts, st, merit))) return rc;
+        CUDA_TRY(launch(k_lbfgs_update, (unsigned)P, nt, st, P, D, S, Cpart, Cstride, phi0, ts.ab, ts.pbest, dC, C, count));
+    }
+    if (f) {
+        a.mode_obj = 0; a.f = f; a.g = nullptr;
+        if ((rc = ntgb_eval(pb, &a))) return rc;
+    }
+    if (iters) CUDA_TRY(cudaMemcpyAsync(iters, S.its, sizeof(int) * Pz, cudaMemcpyDeviceToDevice, st));
+    if (status) CUDA_TRY(cudaMemcpyAsync(status, S.state, sizeof(int) * Pz, cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
     return 0;
 }
 

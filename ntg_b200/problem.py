@@ -13,7 +13,7 @@ from typing import Dict, Optional
 import numpy as np
 
 from . import abi
-from .abi import (JAC_BAND, JAC_DENSE, JAC_NONE, BuiltSetup, NtgbDims, NtgbEvalArgs, NtgbPack, SolveOpts, NlpOpts, SqpOpts,
+from .abi import (JAC_BAND, JAC_DENSE, JAC_NONE, BuiltSetup, NtgbDims, NtgbEvalArgs, NtgbPack, SolveOpts, LbfgsOpts, NlpOpts, SqpOpts,
                   ProblemSpec, c_double_p, c_int_p)
 
 _LIBDIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib")
@@ -51,6 +51,8 @@ def core() -> C.CDLL:
         lib.ntgb_solve_eq.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.c_void_p, C.c_void_p]
         lib.ntgb_solve_eq.restype = C.c_int
+        lib.ntgb_solve_eq_lbfgs.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 8
+        lib.ntgb_solve_eq_lbfgs.restype = C.c_int
         lib.ntgb_solve_nlp.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p]
         lib.ntgb_solve_nlp.restype = C.c_int
@@ -360,6 +362,25 @@ class Problem:
         else:
             _check(core().ntgb_solve_eq(self._h, P, Cdev.data_ptr(), f.data_ptr(), it.data_ptr(), stt.data_ptr(),
                                         C.addressof(opts), st))
+        return f, it, stt
+
+    def solve_eq_lbfgs(self, Cdev, max_iter=0, gtol=0.0, c1=0.0, memory=0, check_every=0, lowerb=None, upperb=None):
+        """batched projected L-BFGS (ntgb_solve_eq_lbfgs): the problems of solve_eq with any number of free
+        directions.  Cdev [P][nC] is overwritten with the solutions.  Returns f [P], iters [P], status [P]
+        (1 converged, 2 no further decrease, 0 iteration limit, 5 rejected per-problem bounds).  memory: the
+        curvature pairs kept per problem, 1..32 (0: 8); the other options take their defaults at 0.
+        lowerb / upperb [P][spec.nbounds] (device): each problem's own bounds, as in solve_eq."""
+        import torch
+        P = Cdev.shape[0]
+        per_problem = self._check_bounds(Cdev, lowerb, upperb)
+        f = torch.zeros(P, dtype=torch.float64, device=Cdev.device)
+        it = torch.zeros(P, dtype=torch.int32, device=Cdev.device)
+        stt = torch.zeros(P, dtype=torch.int32, device=Cdev.device)
+        opts = LbfgsOpts(int(max_iter), float(gtol), float(c1), int(memory) if memory else 8, int(check_every))
+        st = torch.cuda.current_stream(Cdev.device).cuda_stream
+        lo_p, up_p = (lowerb.data_ptr(), upperb.data_ptr()) if per_problem else (None, None)
+        _check(core().ntgb_solve_eq_lbfgs(self._h, P, Cdev.data_ptr(), lo_p, up_p, f.data_ptr(), it.data_ptr(),
+                                          stt.data_ptr(), C.addressof(opts), st))
         return f, it, stt
 
     def solve_nlp(self, Cdev, max_outer=0, max_inner=0, gtol=0.0, ctol=0.0, rho0=0.0, rho_mul=0.0, rho_max=0.0,
