@@ -497,6 +497,57 @@ typedef struct ntgb_lbfgs_opts {
 int  ntgb_solve_eq_lbfgs(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb,
                          double *f, int *iters, int *status, const ntgb_lbfgs_opts *opts, void *stream);
 
+/*
+ * Long horizons with a Newton method: the problem class of ntgb_solve_eq_lbfgs (a smooth cost, only EQUALITY
+ * linear constraints, no nonlinear ones, any number of free directions), with an iteration count that does not
+ * grow with the horizon.
+ *
+ * Structure (host, once per setup; ntgb_newton_structure reports it).  A breakpoint touches only order_j
+ * coefficients of each output, so the cost's Hessian H couples exactly the coefficients of the outputs in its
+ * active-variable lists that share a breakpoint.  The columns are ordered by the first breakpoint that touches
+ * them (ties by output): then H + A'A is a band of half-bandwidth w, independent of the horizon.  A greedy
+ * distance-2 colouring of H's pattern (no two columns of one colour share a row) gives K colours.
+ *
+ * Per iteration: one batched evaluation (cost + gradient) and the test |P g|_inf <= gtol max(1, |f|), P the
+ * projector onto null(A) (as in ntgb_solve_eq_lbfgs); then ONE batched gradient evaluation of the 2K points
+ * C +- h e_k (central differences on colour k, h_c = eps^(1/3) max(1, |C_c|)), from which each problem's band of
+ * H is recovered; M = H + rho A'A + tau I with rho = max diag H / max diag A'A and tau a per-problem
+ * Levenberg-Marquardt shift; a banded Cholesky of M (O(nC w^2)); the range-space step
+ * d = -M^-1 (g + Q1' lam), S lam = -Q1 M^-1 g, S = Q1 M^-1 Q1' (r x r, Q1 the orthonormal basis of the equality
+ * rows' span, r its dimension); the two-stage Armijo search on the cost with a rounding allowance of
+ * 8 eps |f|; the step projected onto the affine set again.  The shift: tau = tau / 4 after a unit step,
+ * max(4 tau, beta) after a step below 1/4, a failed search or a nonpositive pivot (then refactored, up to 8
+ * times, before the direction falls back to -P g), beta = 1e-3 max diag (H + rho A'A); tau starts at 0.
+ * Stopping: status 1 by the gradient test; status 2 after two consecutive iterations without a strict decrease
+ * of the cost (the cost no longer resolves a decrease: the rounding floor) or at a NaN gradient; status 0 at
+ * max_iter.  Each reduction has a fixed order: results do not depend on the batch size or order.
+ *
+ * Arguments, outputs and refusals as in ntgb_solve_eq_lbfgs: lowerb / upperb both NULL or both DEVICE [P][nb];
+ * exactly one NULL is NTGB_EINVAL before any CUDA call; opts may be NULL (every default), a field <= 0 takes its
+ * default; status 1, 2, 0 or NTGB_STATUS_BAD_BOUNDS (C left untouched bit for bit, iters 0); nonlinear or
+ * inequality rows are NTGB_EINVAL; no free direction gives C = C_part, status 1 and iters 0.  Limits
+ * (NTGB_ELIMIT): r <= 128 (trajectory equality rows at many breakpoints can exceed it) and w <= 64.
+ * Synchronous.
+ *
+ * Work space (device, kept between calls, freed by ntgb_destroy): about
+ *     P (4K + w + r + 24) nC + P r^2  doubles
+ * (the 2K difference points and their gradients, the band, M^-1 [g, Q1'], the 16 trial points of the search and
+ * a handful of vectors; S), plus r nC for Q1 and nC per problem with per-problem bounds.  Nothing of size
+ * nC x nC is on the device.
+ */
+typedef struct ntgb_newton_opts {
+    int max_iter;     /* default 100 */
+    double gtol;      /* |P g|_inf <= gtol * max(1, |f|), default 1e-9 */
+    double c1;        /* Armijo constant, default 1e-4 */
+    int check_every;  /* host reads the done counter every this many iterations, default 4 */
+} ntgb_newton_opts;
+int  ntgb_solve_eq_newton(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb,
+                          double *f, int *iters, int *status, const ntgb_newton_opts *opts, void *stream);
+/* the structure ntgb_solve_eq_newton uses for this setup: K colours (2K gradient evaluations per Hessian), the
+ * half-bandwidth w and perm [nC] (perm[i] = the column at band position i; may be NULL).  NTGB_ELIMIT when
+ * w > 64.  Use K, w and r (nC minus the free directions) to size the work space above. */
+int  ntgb_newton_structure(ntgb_problem *pb, int *ncolors, int *half_bandwidth, int *perm);
+
 /* Gathered result tables for the fused multi-GPU gather (ntgb_eval_args.peer_result): alloc creates
  * this rank's table (rows x 2 doubles, zeroed) and the 64-byte CUDA IPC handle the other ranks
  * need; open maps another rank's table into this process (peer access over NVLink is enabled on

@@ -91,6 +91,11 @@ class LbfgsOpts(C.Structure):
                 ("check_every", C.c_int)]
 
 
+class NewtonOpts(C.Structure):
+    """ntgb_newton_opts (include/ntg_b200.h)"""
+    _fields_ = [("max_iter", C.c_int), ("gtol", C.c_double), ("c1", C.c_double), ("check_every", C.c_int)]
+
+
 class NlpOpts(C.Structure):
     """ntgb_nlp_opts (include/ntg_b200.h)"""
     _fields_ = [("max_outer", C.c_int), ("max_inner", C.c_int), ("gtol", C.c_double), ("ctol", C.c_double),

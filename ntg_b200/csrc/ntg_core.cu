@@ -34,6 +34,7 @@
 #include "ntg_bounds.h"
 #include "ntg_warm.h"
 #include "ntg_lbfgs.h"
+#include "ntg_newton.h"
 
 namespace {
 
@@ -169,7 +170,19 @@ struct ntgb_problem {
     } sqp;
     /* per-call device arrays, kept between calls: one scratch per driver, so that no call's arrays alias
      * another solver's (ntgb_solve_eq, ntgb_solve_nlp, ntgb_solve_sqp, ntgb_linesearch, per-problem bounds) */
-    struct { Scratch eq, nlp, sqp, ls, bnd, lbfgs; } scratch;
+    struct { Scratch eq, nlp, sqp, ls, bnd, lbfgs, newton; } scratch;
+    /* ntgb_solve_eq_newton: bit j of cost_out[0 / 1 / 2] = output j in the initial / trajectory / final cost's
+     * active variables; the structure ntg_newton.h derives from them, built on the first call that needs it */
+    unsigned cost_out[3] = {0, 0, 0};
+    struct {
+        bool ready = false;
+        int K = 0, w = 0;
+        std::vector<int> hperm;
+        int *perm = nullptr, *color = nullptr;
+        unsigned char *hmask = nullptr;
+        double *ata = nullptr;
+        double ata_max = 0.0;
+    } newton;
     /* ntgb_solve_eq_async / ntgb_solve_sqp_async: their own work spaces, apart from `scratch`, so that no
      * synchronous call moves an array that a captured graph uses; halving = the step table 2^-a, a < 16 */
     struct {
@@ -1580,6 +1593,9 @@ int solve_eq_impl(ntgb_problem *pb, Run run, int P, double *C, const double *low
                   int *iters, int *status, const ntgb_solve_opts *opts, void *stream);
 int solve_lbfgs_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
                      int *iters, int *status, const ntgb_lbfgs_opts &o, void *stream);
+int solve_newton_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                      int *iters, int *status, const ntgb_newton_opts &o, void *stream);
+int newton_prepare(ntgb_problem *pb);
 int solve_sqp_impl(ntgb_problem *pb, Run run, int P, double *C, const double *lowerb, const double *upperb, double *warm,
                    double *f, double *viol_out, int *iters, int *status, double *lambda, int *istate,
                    const ntgb_sqp_opts *opts, void *stream);
@@ -1632,7 +1648,8 @@ void ntgb_destroy(ntgb_problem *pb)
     for (void *p : pb->allocs) cudaFree(p);
     if (pb->zc.buf) cudaFreeHost(pb->zc.buf);
     auto &s = pb->scratch;
-    for (Scratch *sc : {&s.eq, &s.nlp, &s.sqp, &s.ls, &s.bnd, &s.lbfgs, &pb->async.eq.s, &pb->async.sqp.s}) cudaFree(sc->p);
+    for (Scratch *sc : {&s.eq, &s.nlp, &s.sqp, &s.ls, &s.bnd, &s.lbfgs, &s.newton, &pb->async.eq.s, &pb->async.sqp.s})
+        cudaFree(sc->p);
     for (auto &h : pb->hs) {
         double *hsp[] = {h.C, h.f, h.g, h.c, h.J, h.Z, h.result};
         for (double *p : hsp)
@@ -1761,6 +1778,13 @@ int ntgb_create(ntgb_problem **out, const ntgb_setup *s, int device)
     if (s->nnlic != 0) add_mask(T.avmask, s->initialconstrav, s->ninitialconstrav, 1);
     if (s->nnltc != 0) add_mask(T.avmask, s->trajectoryconstrav, s->ntrajectoryconstrav, 0);
     if (s->nnlfc != 0) add_mask(T.avmask, s->finalconstrav, s->nfinalconstrav, 2);
+    {
+        const int ncost[3] = {s->nicf, s->nucf, s->nfcf}, nav[3] = {s->ninitialcostav, s->ntrajectorycostav, s->nfinalcostav};
+        const AV *av[3] = {s->initialcostav, s->trajectorycostav, s->finalcostav};
+        for (int k = 0; k < 3; k++)
+            if (ncost[k] != 0)
+                for (int i = 0; i < nav[k]; i++) pb->cost_out[k] |= 1u << av[k][i].output;
+    }
 
     /* ---- K0: tables on the device ---- */
     double *dbps = nullptr;
@@ -2520,6 +2544,38 @@ int ntgb_solve_eq_lbfgs(ntgb_problem *pb, int P, double *C, const double *lowerb
     return solve_lbfgs_impl(pb, P, C, lowerb, upperb, f, iters, status, o, stream);
 }
 
+int ntgb_solve_eq_newton(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                         int *iters, int *status, const ntgb_newton_opts *opts, void *stream)
+{
+    /* the argument checks read nothing behind pb */
+    if (!pb || !C) return fail(NTGB_EINVAL, "ntgb_solve_eq_newton: null argument");
+    if ((lowerb == nullptr) != (upperb == nullptr))
+        return fail(NTGB_EINVAL, "ntgb_solve_eq_newton: exactly one of lowerb / upperb is NULL");
+    ntgb_newton_opts o{100, 1e-9, 1e-4, 4};
+    if (opts) {
+        if (opts->max_iter > 0) o.max_iter = opts->max_iter;
+        if (opts->gtol > 0.0) o.gtol = opts->gtol;
+        if (opts->c1 > 0.0) o.c1 = opts->c1;
+        if (opts->check_every > 0) o.check_every = opts->check_every;
+    }
+    if (P <= 0) return 0;
+    return solve_newton_impl(pb, P, C, lowerb, upperb, f, iters, status, o, stream);
+}
+
+int ntgb_newton_structure(ntgb_problem *pb, int *ncolors, int *half_bandwidth, int *perm)
+{
+    if (!pb) return fail(NTGB_EINVAL, "ntgb_newton_structure: null argument");
+    DeviceGuard dg(pb->device);
+    if (!dg.ok) return fail(NTGB_ECUDA, "cannot select device %d", pb->device);
+    int rc;
+    if ((rc = newton_prepare(pb))) return rc;
+    const auto &nw = pb->newton;
+    if (ncolors) *ncolors = nw.K;
+    if (half_bandwidth) *half_bandwidth = nw.w;
+    if (perm) memcpy(perm, nw.hperm.data(), sizeof(int) * nw.hperm.size());
+    return 0;
+}
+
 } /* extern "C" */
 
 namespace {
@@ -2821,6 +2877,328 @@ int solve_lbfgs_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, c
         }
         if ((rc = two_stage_search(pb, P, C, dC, o.c1, phi0, dphi0, S.state, ts, st, merit))) return rc;
         CUDA_TRY(launch(k_lbfgs_update, (unsigned)P, nt, st, P, D, S, Cpart, Cstride, phi0, ts.ab, ts.pbest, dC, C, count));
+    }
+    if (f) {
+        a.mode_obj = 0; a.f = f; a.g = nullptr;
+        if ((rc = ntgb_eval(pb, &a))) return rc;
+    }
+    if (iters) CUDA_TRY(cudaMemcpyAsync(iters, S.its, sizeof(int) * Pz, cudaMemcpyDeviceToDevice, st));
+    if (status) CUDA_TRY(cudaMemcpyAsync(status, S.state, sizeof(int) * Pz, cudaMemcpyDeviceToDevice, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return 0;
+}
+
+/* ---- ntgb_solve_eq_newton: banded Newton, one CTA per problem running ntg_newton.h ----------------------- */
+
+/* threads of the factor and direction CTAs: fixed, so that no result depends on the batch.  The window update
+ * of the factor has w (w+1) / 2 entries per column (91 at the lane change's w = 13), the direction walks r + 1
+ * right-hand sides, one per thread (r <= kMaxRows). */
+constexpr int kNewtonThreads = 128;
+
+struct NewtonArrays {
+    double *Xp, *Gp, *fp;                  /* [P][2K][nC] difference points and their gradients, [P][2K] costs */
+    double *band;                          /* [P][nC][w+1] H + rho A'A + tau I, then its factor */
+    double *Y, *S, *lam;                   /* [P][r+1][nC], [P][r][r], [P][r] of the range-space step */
+    double *pg, *sv;                       /* [P][nC] projected gradient, the last step */
+    double *tau, *beta;                    /* [P] */
+    int *state, *its, *stall, *factored;   /* [P] */
+
+    void take(Carve &c, size_t P, int nC, int K, int w, int r)
+    {
+        c.take(P * 2 * K * nC, Xp, Gp);
+        c.take(P * 2 * K, fp);
+        c.take(P * nC * (w + 1), band);
+        c.take(P * (r + 1) * nC, Y);
+        c.take(P * std::max(r * r, 1), S);
+        c.take(P * std::max(r, 1), lam);
+        c.take(P * nC, pg, sv);
+        c.take(P, tau, beta);
+        c.take(P, state, its, stall, factored);
+    }
+    __device__ ntgb::lbfgs::View proj(const ntgb::newton::Desc &D, int p) const
+    {
+        return ntgb::lbfgs::View{D.Q1, D.r, D.nC, 0, nullptr, nullptr, sv + (size_t)p * D.nC, nullptr};
+    }
+};
+
+/* at entry: C onto problem p's affine set, no shift.  Per-problem bounds (Cstride = nC): k_bounds_prep has set
+ * state / iters, a rejected problem keeps its C.  No free direction (r == nC): C = Cpart and status 1 */
+__global__ void k_newton_init(int P, ntgb::newton::Desc D, NewtonArrays S, const double *Cpart, int Cstride, double *C)
+{
+    __shared__ double red[kNewtonThreads / 32];
+    const int p = blockIdx.x;
+    if (Cstride != 0 && S.state[p] == NTGB_STATUS_BAD_BOUNDS) return;
+    Cpart += (size_t)p * Cstride;
+    double *Cp = C + (size_t)p * D.nC;
+    if (D.r == D.nC) {
+        for (int e = threadIdx.x; e < D.nC; e += blockDim.x) Cp[e] = Cpart[e];
+    } else {
+        ntgb::lbfgs::affine_step(lbfgs_group(), red, S.proj(D, p), Cpart, Cp, nullptr, 0.0);
+    }
+    if (threadIdx.x == 0) {
+        S.state[p] = D.r == D.nC ? 1 : 0;
+        S.its[p] = 0;
+        S.tau[p] = 0.0;
+        S.beta[p] = 0.0;
+        S.stall[p] = 0;
+    }
+}
+
+/* P g and the convergence test: |P g|_inf <= gtol max(1, |f|) is status 1, a NaN gradient status 2 */
+__global__ void k_newton_check(int P, ntgb::newton::Desc D, NewtonArrays S, const double *f, const double *g, double gtol,
+                               int *count)
+{
+    __shared__ double red[kNewtonThreads / 32];
+    const int p = blockIdx.x;
+    if (S.state[p] != 0) return;
+    const size_t n = D.nC;
+    double *pg = S.pg + p * n;
+    const sqp::Coop cg = lbfgs_group();
+    for (size_t e = threadIdx.x; e < n; e += blockDim.x) pg[e] = g[p * n + e];
+    ntgb::lbfgs::project(cg, red, D.Q1, D.r, D.nC, pg);
+    double gmax = 0.0, gg = 0.0;
+    for (size_t e = threadIdx.x; e < n; e += blockDim.x) {
+        gmax = fmax(gmax, fabs(pg[e]));
+        gg += pg[e] * pg[e];
+    }
+    gmax = cg.reduce<true>(gmax, red);
+    gg = cg.reduce<false>(gg, red);
+    const double fa = fabs(f[p]);
+    const int st = gg != gg ? 2 : (!(gmax > gtol * (fa > 1.0 ? fa : 1.0)) ? 1 : 0);
+    if (threadIdx.x == 0 && st != 0) {
+        S.state[p] = st;
+        atomicAdd(count, 1);
+    }
+}
+
+/* the 2K difference points of every problem: point 2k = C + h on the columns of colour k, 2k + 1 = C - h */
+__global__ void k_newton_points(int P, int nC, int K, const int *color, const double *C, double *Xp)
+{
+    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= (long long)P * 2 * K * nC) return;
+    const int e = (int)(q % nC);
+    const long long pk = q / nC;
+    const int k2 = (int)(pk % (2 * K));
+    const long long p = pk / (2 * K);
+    const double x = C[p * nC + e], h = ntgb::newton::fd_step(x);
+    Xp[q] = color[e] == (k2 >> 1) ? ((k2 & 1) ? x - h : x + h) : x;
+}
+
+/* M = H + rho A'A + tau I from the differences and its banded Cholesky; a nonpositive pivot raises tau to
+ * max(4 tau, beta) and refactors, up to kMaxShift times.  The window is dynamic shared memory. */
+__global__ void k_newton_factor(int P, ntgb::newton::Desc D, NewtonArrays S, const double *C)
+{
+    extern __shared__ double win[];
+    __shared__ double red[kNewtonThreads / 32];
+    const int p = blockIdx.x;
+    if (S.state[p] != 0) return;
+    const size_t n = D.nC;
+    const sqp::Coop cg = lbfgs_group();
+    double *band = S.band + p * n * (D.w + 1);
+    double tau = S.tau[p], beta = 0.0;
+    bool ok = false;
+    for (int a = 0; a <= ntgb::newton::kMaxShift && !ok; a++) {
+        if (a > 0) tau = fmax(4.0 * tau, beta);
+        double dmax = 0.0;
+        ntgb::newton::assemble(cg, red, D, C + p * n, S.Gp + p * 2 * D.K * n, tau, band, dmax);
+        beta = ntgb::newton::kBetaRel * (dmax > 0.0 ? dmax : 1.0);
+        ok = ntgb::newton::band_cholesky(cg, D.nC, D.w, band, win);
+    }
+    if (threadIdx.x == 0) {
+        S.tau[p] = tau;
+        S.beta[p] = beta;
+        S.factored[p] = ok ? 1 : 0;
+    }
+}
+
+/* the range-space Newton step, or d = -P g after a failed factorization, a singular S or a slope d'g >= 0;
+ * phi0 = f + 8 eps |f| (the search's rounding allowance), dphi0 = d'g.  A finished problem gets d = 0. */
+__global__ void k_newton_dir(int P, ntgb::newton::Desc D, NewtonArrays S, const double *f, const double *g, double *dC,
+                             double *phi0, double *dphi0)
+{
+    __shared__ double red[kNewtonThreads / 32];
+    const int p = blockIdx.x;
+    const size_t n = D.nC;
+    double *d = dC + p * n;
+    const sqp::Coop cg = lbfgs_group();
+    double dg = 0.0;
+    if (S.state[p] == 0) {
+        const size_t r = D.r, rr = r > 0 ? r * r : 1, r1 = r > 0 ? r : 1; /* NewtonArrays::take */
+        bool ok = S.factored[p] && ntgb::newton::range_step(cg, D, S.band + p * n * (D.w + 1), g + p * n,
+                                                             S.Y + p * (r + 1) * n, S.S + p * rr, S.lam + p * r1, d);
+        if (ok) {
+            dg = ntgb::lbfgs::dot(cg, red, d, g + p * n, D.nC);
+            ok = dg < 0.0;
+        }
+        if (!ok) {
+            const double *pg = S.pg + p * n;
+            double gg = 0.0;
+            for (size_t e = threadIdx.x; e < n; e += blockDim.x) {
+                d[e] = -pg[e];
+                gg += pg[e] * pg[e];
+            }
+            dg = -cg.reduce<false>(gg, red);
+        }
+    } else {
+        for (size_t e = threadIdx.x; e < n; e += blockDim.x) d[e] = 0.0;
+    }
+    if (threadIdx.x == 0) {
+        const double fa = fabs(f[p]);
+        phi0[p] = S.state[p] == 0 ? f[p] + 8.0 * DBL_EPSILON * fa : f[p];
+        dphi0[p] = dg;
+    }
+}
+
+/* the step the search chose, the shift and the stopping rule (ntg_newton.h after_search) */
+__global__ void k_newton_update(int P, ntgb::newton::Desc D, NewtonArrays S, const double *Cpart, int Cstride, double c1,
+                                const double *f, const double *phi0, const double *dphi0, const double *alpha_best,
+                                const double *phi_best, const double *dC, double *C, int *count)
+{
+    __shared__ double red[kNewtonThreads / 32];
+    const int p = blockIdx.x;
+    if (S.state[p] != 0) return;
+    const size_t n = D.nC;
+    const double a = alpha_best[p];
+    /* the test of k_alm_pick1 / k_alm_pick2, on the same operands */
+    const bool armijo = phi_best[p] <= phi0[p] + c1 * a * dphi0[p];
+    if (armijo) ntgb::lbfgs::affine_step(lbfgs_group(), red, S.proj(D, p), Cpart + (size_t)p * Cstride, C + p * n, dC + p * n, a);
+    if (threadIdx.x == 0) {
+        ntgb::newton::State s{S.tau[p], S.beta[p], S.stall[p]};
+        int done = 0;
+        ntgb::newton::after_search(s, armijo, a, phi_best[p], f[p], &done);
+        S.tau[p] = s.tau;
+        S.stall[p] = s.stall;
+        S.its[p] += 1;
+        if (done != 0) {
+            S.state[p] = done;
+            atomicAdd(count, 1);
+        }
+    }
+}
+
+/* the structure of ntg_newton.h for this setup, once: the pattern of the cost from the K0 offsets and the
+ * cost's active variables, and of A'A from the equality rows */
+int newton_prepare(ntgb_problem *pb)
+{
+    auto &nw = pb->newton;
+    if (nw.ready) return 0;
+    const ntgb_dims &dm = pb->dims;
+    const int nC = dm.nC, nclin = dm.nclin;
+    std::vector<double> A;
+    int m = 0;
+    for (int i = 0; i < nclin; i++)
+        if (pb->lin_lb[i] == pb->lin_ub[i]) {
+            for (int c = 0; c < nC; c++) A.push_back(pb->A[i + (size_t)c * nclin]);
+            m++;
+        }
+    if (A.empty()) A.push_back(0.0);
+    ntgb::newton::Structure S;
+    ntgb::newton::build_structure(dm.nout, dm.nbps, pb->order.data(), pb->ncoef.data(), pb->hoff.data(), pb->cost_out,
+                                  A.data(), m, S);
+    if (S.w > ntgb::newton::kMaxHalfBand)
+        return fail(NTGB_ELIMIT, "ntgb_solve_eq_newton: the Hessian's half-bandwidth %d is above the limit of %d", S.w,
+                    ntgb::newton::kMaxHalfBand);
+    int rc;
+    if ((rc = dev_upload(pb, &nw.perm, S.perm.data(), S.perm.size())) ||
+        (rc = dev_upload(pb, &nw.color, S.color.data(), S.color.size())) ||
+        (rc = dev_upload(pb, &nw.hmask, S.hmask.data(), S.hmask.size())) ||
+        (rc = dev_upload(pb, &nw.ata, S.ata.data(), S.ata.size())))
+        return rc;
+    nw.ata_max = 0.0;
+    for (int i = 0; i < nC; i++) nw.ata_max = std::max(nw.ata_max, S.ata[(size_t)i * (S.w + 1)]);
+    nw.K = S.K;
+    nw.w = S.w;
+    nw.hperm = S.perm;
+    nw.ready = true;
+    return 0;
+}
+
+/* ntgb_solve_eq_newton.  Per iteration: one evaluation at C, the convergence test, one evaluation of the 2K
+ * difference points of every problem, the factor, the direction, two_stage_search on the cost and the update. */
+int solve_newton_impl(ntgb_problem *pb, int P, double *C, const double *lowerb, const double *upperb, double *f,
+                      int *iters, int *status, const ntgb_newton_opts &o, void *stream)
+{
+    const ntgb_dims &dm = pb->dims;
+    const int nC = dm.nC;
+    int rc;
+    if ((rc = check_eq_only(pb, "ntgb_solve_eq_newton"))) return rc;
+    if ((rc = TwoStage::check_size(P))) return rc;
+    DeviceGuard dg(pb->device);
+    if (!dg.ok) return fail(NTGB_ECUDA, "cannot select device %d", pb->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    if ((rc = reduced_form(pb, false, true))) return rc;
+    const auto &al = pb->alm;
+    if (al.nr > 0 && al.r > ntgb::newton::kMaxRows)
+        return fail(NTGB_ELIMIT,
+                    "ntgb_solve_eq_newton: the equality rows span %d dimensions, above the limit of %d of the range-space "
+                    "step (trajectory equality rows at many breakpoints exceed it)",
+                    al.r, ntgb::newton::kMaxRows);
+    if ((rc = newton_prepare(pb))) return rc;
+    const auto &nw = pb->newton;
+    if ((size_t)P * 2 * nw.K > 0x7fffffffull) return fail(NTGB_EINVAL, "P*2*ncolors too large");
+    const size_t Pz = (size_t)P;
+    const ntgb::newton::Desc D{nw.perm, nw.color, nw.hmask, nw.ata, al.Q1, nC, nw.w, nw.K, al.r, nw.ata_max};
+    const BoundsDesc B{bounds_layout(pb), nC, 0, 0, dm.nclin, nullptr, nullptr, al.M, al.Ae};
+    NewtonArrays S;
+    TwoStage ts;
+    BoundsArrays ba;
+    double *g, *dC, *fv, *phi0, *dphi0;
+    int *count;
+    if ((rc = scratch_carve(pb->scratch.newton, st, [&](Carve &c) {
+             S.take(c, Pz, nC, nw.K, nw.w, al.r);
+             c.take(Pz * nC, g, dC);
+             c.take(Pz, fv, phi0, dphi0);
+             c.take(1, count);
+             ts.take(c, Pz, dm);
+             if (lowerb) ba.take(c, Pz, B);
+         })))
+        return rc;
+    if ((rc = ts.start(P, st))) return rc;
+    CUDA_TRY(cudaMemsetAsync(count, 0, sizeof(int), st));
+    const double *Cpart = al.Cpart;
+    int Cstride = 0;
+    if (lowerb) {
+        if ((rc = bounds_prepare(P, lowerb, upperb, B, ba, st, S.state, S.its, count))) return rc;
+        Cpart = ba.Cpart;
+        Cstride = nC;
+    }
+    const int nt = kNewtonThreads;
+    const size_t win = sizeof(double) * (nw.w + 1) * (nw.w + 1);
+    CUDA_TRY(launch(k_newton_init, (unsigned)P, nt, st, P, D, S, Cpart, Cstride, C));
+    ntgb_eval_args a, ad;
+    memset(&a, 0, sizeof a);
+    a.P = P; a.C = C; a.mode_obj = 2; a.mode_con = -1; a.f = fv; a.g = g; a.jac_layout = NTGB_JAC_NONE; a.stream = st;
+    ad = a;
+    ad.P = P * 2 * nw.K; ad.C = S.Xp; ad.f = S.fp; ad.g = S.Gp;
+    const long long npts = (long long)ad.P * nC;
+    auto merit = [&](int n, int, const int *) -> int {
+        CUDA_TRY(launch(k_cost_merit, (unsigned)((n + 255) / 256), 256, st, n, (const double *)ts.ft, ts.res));
+        return 0;
+    };
+    const int max_iter = al.nr > 0 ? o.max_iter : 0; /* no free direction: k_newton_init has finished every problem */
+    for (int it = 0; it < max_iter; it++) {
+        if ((rc = ntgb_eval(pb, &a))) return rc;
+        CUDA_TRY(launch(k_newton_check, (unsigned)P, nt, st, P, D, S, (const double *)fv, (const double *)g, o.gtol, count));
+        if ((it + 1) % o.check_every == 0 && (rc = all_finished(count, P, st)) != 0) {
+            if (rc < 0) return rc;
+            break;
+        }
+        CUDA_TRY(launch(k_newton_points, (unsigned)((npts + 255) / 256), 256, st, P, nC, nw.K, (const int *)nw.color,
+                        (const double *)C, S.Xp));
+        if ((rc = ntgb_eval(pb, &ad))) return rc;
+        {
+            cudaLaunchConfig_t cfg = {};
+            cfg.gridDim = dim3((unsigned)P);
+            cfg.blockDim = dim3(nt);
+            cfg.dynamicSmemBytes = win;
+            cfg.stream = st;
+            CUDA_TRY(cudaLaunchKernelEx(&cfg, k_newton_factor, P, D, S, (const double *)C));
+        }
+        CUDA_TRY(launch(k_newton_dir, (unsigned)P, nt, st, P, D, S, (const double *)fv, (const double *)g, dC, phi0, dphi0));
+        if ((rc = two_stage_search(pb, P, C, dC, o.c1, phi0, dphi0, S.state, ts, st, merit))) return rc;
+        CUDA_TRY(launch(k_newton_update, (unsigned)P, nt, st, P, D, S, Cpart, Cstride, o.c1, (const double *)fv,
+                        (const double *)phi0, (const double *)dphi0, (const double *)ts.ab, (const double *)ts.pbest,
+                        (const double *)dC, C, count));
     }
     if (f) {
         a.mode_obj = 0; a.f = f; a.g = nullptr;

@@ -13,7 +13,7 @@ from typing import Dict, Optional
 import numpy as np
 
 from . import abi
-from .abi import (JAC_BAND, JAC_DENSE, JAC_NONE, BuiltSetup, NtgbDims, NtgbEvalArgs, NtgbPack, SolveOpts, LbfgsOpts, NlpOpts, SqpOpts,
+from .abi import (JAC_BAND, JAC_DENSE, JAC_NONE, BuiltSetup, NtgbDims, NtgbEvalArgs, NtgbPack, SolveOpts, LbfgsOpts, NewtonOpts, NlpOpts, SqpOpts,
                   ProblemSpec, c_double_p, c_int_p)
 
 _LIBDIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib")
@@ -53,6 +53,10 @@ def core() -> C.CDLL:
         lib.ntgb_solve_eq.restype = C.c_int
         lib.ntgb_solve_eq_lbfgs.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 8
         lib.ntgb_solve_eq_lbfgs.restype = C.c_int
+        lib.ntgb_solve_eq_newton.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 8
+        lib.ntgb_solve_eq_newton.restype = C.c_int
+        lib.ntgb_newton_structure.argtypes = [C.c_void_p] * 4
+        lib.ntgb_newton_structure.restype = C.c_int
         lib.ntgb_solve_nlp.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_void_p]
         lib.ntgb_solve_nlp.restype = C.c_int
@@ -382,6 +386,31 @@ class Problem:
         _check(core().ntgb_solve_eq_lbfgs(self._h, P, Cdev.data_ptr(), lo_p, up_p, f.data_ptr(), it.data_ptr(),
                                           stt.data_ptr(), C.addressof(opts), st))
         return f, it, stt
+
+    def solve_eq_newton(self, Cdev, max_iter=0, gtol=0.0, c1=0.0, check_every=0, lowerb=None, upperb=None):
+        """batched banded Newton (ntgb_solve_eq_newton): the problems of solve_eq_lbfgs, with the Hessian from
+        coloured gradient differences.  Cdev [P][nC] is overwritten with the solutions.  Returns f [P], iters [P],
+        status [P] (1 converged, 2 no further decrease, 0 iteration limit, 5 rejected per-problem bounds); the
+        options take their defaults at 0.  lowerb / upperb [P][spec.nbounds] (device): each problem's own bounds."""
+        import torch
+        P = Cdev.shape[0]
+        per_problem = self._check_bounds(Cdev, lowerb, upperb)
+        f = torch.zeros(P, dtype=torch.float64, device=Cdev.device)
+        it = torch.zeros(P, dtype=torch.int32, device=Cdev.device)
+        stt = torch.zeros(P, dtype=torch.int32, device=Cdev.device)
+        opts = NewtonOpts(int(max_iter), float(gtol), float(c1), int(check_every))
+        st = torch.cuda.current_stream(Cdev.device).cuda_stream
+        lo_p, up_p = (lowerb.data_ptr(), upperb.data_ptr()) if per_problem else (None, None)
+        _check(core().ntgb_solve_eq_newton(self._h, P, Cdev.data_ptr(), lo_p, up_p, f.data_ptr(), it.data_ptr(),
+                                           stt.data_ptr(), C.addressof(opts), st))
+        return f, it, stt
+
+    def newton_structure(self):
+        """-> (K colours, half-bandwidth w, perm [nC]) of solve_eq_newton for this setup"""
+        K, w = C.c_int(), C.c_int()
+        perm = np.zeros(self.spec.nC, dtype=np.int32)
+        _check(core().ntgb_newton_structure(self._h, C.byref(K), C.byref(w), perm.ctypes.data))
+        return K.value, w.value, perm
 
     def solve_nlp(self, Cdev, max_outer=0, max_inner=0, gtol=0.0, ctol=0.0, rho0=0.0, rho_mul=0.0, rho_max=0.0,
                   c1=0.0, check_every=0):
