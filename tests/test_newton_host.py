@@ -261,13 +261,16 @@ def test_shift_and_stopping_rule(lib):
     assert lib.newton_host_after_search(_p(st), 0, 1.0, 1.0, 1.0) == 2 and tuple(st) == (2.0, 2.0, 2.0)
 
 
-def newton_restated(lib, port, spec, s, x0, gtol=1e-9, c1=1e-4, max_iter=50):
-    """the device loop restated with the g++ build and the oracle's evaluations: -> (C, status, iters)"""
+def newton_restated(lib, port, spec, s, x0, gtol=1e-9, c1=1e-4, max_iter=50, Q1=None, Cpart=None, proj=None,
+                    dot=np.dot):
+    """the device loop restated with the g++ build and the oracle's evaluations: -> (C, status, iters).  By default
+    Q1 from numpy's QR, Cpart from lstsq, P v = v - Q1' (Q1 v) and BLAS dot products; Q1, Cpart, proj and dot may
+    be given instead (the library's basis and a fixed summation order make the result exact)."""
     nC = spec.nC
     A, b = s.A, s.b
-    Q1 = np.ascontiguousarray(np.linalg.qr(A.T)[0].T)
-    Cpart = np.linalg.lstsq(A, b, rcond=None)[0]
-    proj = lambda v: v - Q1.T @ (Q1 @ v)        # noqa: E731
+    Q1 = np.ascontiguousarray(np.linalg.qr(A.T)[0].T) if Q1 is None else Q1
+    Cpart = np.linalg.lstsq(A, b, rcond=None)[0] if Cpart is None else Cpart
+    proj = (lambda v: v - Q1.T @ (Q1 @ v)) if proj is None else proj
     x = Cpart + proj(x0 - Cpart)
     ata_max = float(s.ata.reshape(nC, -1)[:, 0].max())
     st = np.array([0.0, 0.0, 0.0])
@@ -276,7 +279,8 @@ def newton_restated(lib, port, spec, s, x0, gtol=1e-9, c1=1e-4, max_iter=50):
     for it in range(max_iter):
         r = port.eval(spec, x[None, :], mode_obj=2, mode_con=-1, dense=False, band=False)
         f, g = float(r["f"][0]), r["g"][0]
-        if np.abs(proj(g)).max() <= gtol * max(1.0, abs(f)):
+        pg = proj(g)
+        if np.abs(pg).max() <= gtol * max(1.0, abs(f)):
             return x, 1, it
         G = _colored_gradients(port, spec, s, x)
         ok = False
@@ -288,14 +292,17 @@ def newton_restated(lib, port, spec, s, x0, gtol=1e-9, c1=1e-4, max_iter=50):
                 break
             st[0] = max(4 * st[0], st[1])
         d = np.zeros(nC)
-        if not ok or not lib.newton_host_range_step(nC, s.w, Q1.shape[0], _p(s.perm, ip), _p(Q1), _p(band), _p(g), _p(d)) \
-                or d @ g >= 0:
-            d = -proj(g)
+        dg = 0.0
+        if ok and lib.newton_host_range_step(nC, s.w, Q1.shape[0], _p(s.perm, ip), _p(Q1), _p(band), _p(g), _p(d)):
+            dg = dot(d, g)
+        if not dg < 0:
+            d = -pg
+            dg = -dot(pg, pg)
         phi0 = f + 8 * eps * abs(f)
         alphas = 2.0 ** -np.arange(16)
         ft = port.eval(spec, x[None, :] + alphas[:, None] * d[None, :], mode_obj=0, mode_con=-1, dense=False,
                        band=False)["f"]
-        arm = np.flatnonzero(ft <= phi0 + c1 * alphas * (d @ g))
+        arm = np.flatnonzero(ft <= phi0 + c1 * alphas * dg)
         a = alphas[arm[0]] if arm.size else 1.0
         if arm.size:
             x = Cpart + proj(x + a * d - Cpart)

@@ -41,75 +41,69 @@ def fnv1a(data: bytes) -> int:
     return h
 
 
-def reduce_linear(Ae, b):
+def reduce_linear(Ae, b, q1=False):
     """reduce_linear (ntg_core.cu) for the rows Ae [m][n] and right-hand side b [m]: N [nr][n], Cpart [n],
-    Mop [n][m] (Cpart = Mop b for any b; zero columns for rows found dependent), rank r.  Same operations
-    in the same order as the C++ (no FMA contraction on the host), so the results are bit-identical."""
+    Mop [n][m] (Cpart = Mop b for any b; zero columns for rows found dependent), rank r, and with q1=True
+    also Q1 [r][n] (the first r columns of Q, the row-space basis of ntgb_solve_eq_lbfgs / _newton).  Same
+    operations in the same order as the C++ (no FMA contraction on the host), so the results are
+    bit-identical: every sequential sum of the C++ stays sequential here, numpy only runs the independent
+    sums of different columns side by side, one elementwise IEEE operation at a time."""
     m, n = int(Ae.shape[0]), int(Ae.shape[1])
-    M = [[float(Ae[j, i]) for i in range(n)] for j in range(m)]   # M[j] = column j of A'
-    Q = [[1.0 if i == l else 0.0 for l in range(n)] for i in range(n)]
+    M = np.array(Ae, dtype=np.float64).reshape(m, n).copy()      # M[j] = column j of A'
+    Q = np.eye(n)
     perm = list(range(m))
-    v = [0.0] * n
     r, norm0 = 0, 0.0
     for k in range(min(n, m)):
-        jb, nb = k, -1.0
-        for j in range(k, m):
-            col, a = M[j], 0.0
-            for i in range(k, n):
-                a += col[i] * col[i]
-            if a > nb:
-                nb, jb = a, j
-        norm = math.sqrt(nb)
+        a = np.zeros(m - k)
+        for i in range(k, n):
+            a = a + M[k:, i] * M[k:, i]
+        jb = k + int(np.argmax(a))                               # the first largest, as `if (a > nb)`
+        norm = math.sqrt(a[jb - k])
         if k == 0:
             norm0 = norm
         if not (norm > 1e-11 * max(norm0, 1e-300)):
             break
         if jb != k:
-            M[k], M[jb] = M[jb], M[k]
+            M[[k, jb]] = M[[jb, k]]
             perm[k], perm[jb] = perm[jb], perm[k]
-        col = M[k]
-        alpha = -norm if col[k] > 0.0 else norm
-        for i in range(k, n):
-            v[i] = col[i]
+        alpha = -norm if M[k, k] > 0.0 else norm
+        v = np.zeros(n)
+        v[k:] = M[k, k:]
         v[k] -= alpha
         vv = 0.0
-        for i in range(k, n):
-            vv += v[i] * v[i]
+        for x in v[k:].tolist():
+            vv += x * x
         if vv > 0.0:
-            for j in range(k, m):
-                cj, t = M[j], 0.0
-                for i in range(k, n):
-                    t += v[i] * cj[i]
-                t = 2.0 * t / vv
-                for i in range(k, n):
-                    cj[i] -= t * v[i]
-            for i in range(n):
-                qi, t = Q[i], 0.0
-                for l in range(k, n):
-                    t += qi[l] * v[l]
-                t = 2.0 * t / vv
-                for l in range(k, n):
-                    qi[l] -= t * v[l]
+            t = np.zeros(m - k)
+            for i in range(k, n):
+                t = t + v[i] * M[k:, i]
+            t = 2.0 * t / vv
+            M[k:, k:] = M[k:, k:] - t[:, None] * v[None, k:]
+            t = np.zeros(n)
+            for l in range(k, n):
+                t = t + Q[:, l] * v[l]
+            t = 2.0 * t / vv
+            Q[:, k:] = Q[:, k:] - t[:, None] * v[None, k:]
         r += 1
 
-    def back(rhs):
-        w = [0.0] * r
+    def back(R):
+        """the back substitution for the right-hand sides R [m][q] at once, then Q1 w"""
+        w = np.zeros((r, R.shape[1]))
         for i in range(r):
-            a = rhs(perm[i])
+            a = R[perm[i]].copy()
             for l in range(i):
-                a -= M[i][l] * w[l]
-            w[i] = a / M[i][i]
-        out = [0.0] * n
+                a = a - M[i, l] * w[l]
+            w[i] = a / M[i, i]
+        out = np.zeros((n, R.shape[1]))
         for l in range(r):
-            for i in range(n):
-                out[i] += Q[i][l] * w[l]
+            out = out + Q[:, l:l + 1] * w[l][None, :]
         return out
 
-    Cpart = np.array(back(lambda j: float(b[j])))
-    Mop = np.zeros((n, m))
-    for j in range(m):
-        Mop[:, j] = back(lambda jj: 1.0 if jj == j else 0.0)
-    N = np.array([[Q[i][r + k] for i in range(n)] for k in range(n - r)]).reshape(n - r, n)
+    Cpart = back(np.asarray(b, dtype=np.float64).reshape(m, 1))[:, 0].copy()
+    Mop = back(np.eye(m)) if m else np.zeros((n, 0))
+    N = np.ascontiguousarray(Q[:, r:].T)
+    if q1:
+        return N, Cpart, Mop, r, np.ascontiguousarray(Q[:, :r].T)
     return N, Cpart, Mop, r
 
 
